@@ -4,6 +4,8 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port +
                                                              # the real vendored nanoflann), all host threads
+    python bench.py --gpus 1 ... --dump-outputs DIR          # also writes what the timed path computed in its
+                                                             # last tick as DIR/<name>.npy (see dump_outputs)
 
 Workload (BASELINE.json config 4 = the configuration the metric is quoted on):
   1,048,576 x500 UAVs on a 1024 x 1024 grid, 4 m pitch, spawned at z = 0, heading 0; world of
@@ -39,6 +41,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the bench leaves the source tree as it found it (it may be read-only)
 
 N_UAVS = 1 << 20
 DT = 0.01
@@ -74,6 +77,35 @@ def workload(begin, count, side=1024):
     spawn = np.stack([4.0 * (k % side), 4.0 * (k // side), np.zeros(count)], axis=1).astype(np.float64)
     cmd = np.stack([-2 + 4 * u01(SEED, 1, k), -2 + 4 * u01(SEED, 2, k), 2 * u01(SEED, 3, k), -1 + 2 * u01(SEED, 4, k)], axis=1)
     return spawn, np.ascontiguousarray(cmd)
+
+
+DUMP_ROWS = 65536       # UAVs whose whole state --dump-outputs writes (positions: every UAV)
+DUMP_MAX_PAIRS = 1 << 21
+
+
+def seeded_sample(count, k, stream):
+    """`k` of range(count), sorted: the ones with the smallest counter-RNG draws (the same on every run and numpy version)."""
+    return np.sort(np.argsort(u01(SEED, stream, np.arange(count)), kind="stable")[:k])
+
+
+def dump_outputs(out_dir, batch, x):
+    """Writes what a caller of the timed path (mrsb_run: makeStep for every UAV, then handleCollisions) receives after its last
+    tick, one .npy per array: x = every UAV's position; <field>_sample = the whole state, IMU acceleration and collision force
+    of DUMP_ROWS seeded UAVs (their indices in sample_rows); collision_pairs = the directed (i, j) pairs of the last pass, in
+    float32 (indices < 2^24 are exact), a seeded sample of DUMP_MAX_PAIRS when there are more.  At most 60 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = seeded_sample(len(x), DUMP_ROWS, 100).astype(np.int32)
+    out = {"x": x, "sample_rows": rows.astype(np.float64)}
+    for k, a in batch.get_full_state(rows).items():
+        if k != "x":
+            out[f"{k}_sample"] = a
+    out["force_sample"] = batch.get_force(rows)
+    pairs = batch.get_collision_pairs()
+    if len(pairs) > DUMP_MAX_PAIRS:
+        pairs = pairs[seeded_sample(len(pairs), DUMP_MAX_PAIRS, 101)]
+    out["collision_pairs"] = pairs.astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def x500_world():
@@ -431,6 +463,8 @@ def run_b200(args):
     cs = checksum(x_now)
     if dist is not None:
         cs = combine_checksums(cs, dist, dev)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch, x_now)
 
     # shards that fit into L2: the same blocks again without the flush between ticks (what a running simulation sees: tick t + 1
     # reads what tick t wrote), reported beside the headline
@@ -674,7 +708,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write what the timed path computed in its last tick as DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "b200"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,7 @@ cpu_baseline / ``--impl reference`` legs — never by the product package.
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -112,13 +113,16 @@ _fast = None
 def fast_lib():
     """liboracle_fast.so: the same restatement built -O3 -march=native ON THIS HOST (the flags depend on the CPU it runs on, so it
     is never shipped prebuilt) for the separately reported CPU-throughput figure; results may differ from the parity build in the
-    last bits (FMA contraction).  None if it cannot be built here."""
+    last bits (FMA contraction).  None if it cannot be built here.  It is built in a temporary directory, so that the source
+    tree may be read-only."""
     global _fast
     if _fast is None:
-        path = os.path.join(HERE, "_build", "liboracle_fast.so")
         try:
-            subprocess.run(["make", "-s", "-B", "-C", HERE, "fast"], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
-            L = C.CDLL(path)
+            with tempfile.TemporaryDirectory() as tmp:
+                path = os.path.join(tmp, "liboracle_fast.so")
+                subprocess.run(["make", "-s", "-B", "-C", HERE, "fast", f"FAST_OUT={path}"], check=True, stdout=subprocess.DEVNULL,
+                               stderr=subprocess.DEVNULL, timeout=300)
+                L = C.CDLL(path)  # stays mapped after the directory is removed
         except Exception:
             _fast = False
             return None

@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import rand
+from helpers import digest, rand
 from mrs_multirotor_simulator_b200.airframes import AIRFRAMES, airframe
 from oracle import binding as O
 
@@ -24,6 +24,8 @@ def one(frame="x500", pos=(0, 0, 5), hdg=0.0, **kw):
 
 
 # ---------------------------------------------------------------- golden fixtures
+# The trajectory fixtures are the output of the reference's own UavSystem sources (make_golden.py), which the restatement
+# follows bit for bit: the comparison is exact.
 def test_golden_c1_trajectory():
     g = load("c1_position_x500.json")
     s = one("x500", g["spawn"], g["heading"])
@@ -32,7 +34,7 @@ def test_golden_c1_trajectory():
         s.make_step(g["dt"], 200)
         st = s.get_state()
         for k in ("x", "v", "R", "omega", "motor_rpm", "imu"):
-            assert np.allclose(st[k][0], smp[k], rtol=1e-12, atol=1e-12), (smp["t"], k)
+            assert np.array_equal(st[k][0], np.array(smp[k])), (smp["t"], k)
     # independent numpy restatement made during the survey (SURVEY App. D)
     assert np.allclose(st["x"][0], [4.99966878, -2.99316222, 3.99492282], atol=1e-8)
 
@@ -46,7 +48,7 @@ def test_golden_every_mode_every_motor_count():
         s.make_step(c["dt"], c["steps"])
         st = s.get_state()
         for k in ("x", "v", "R", "omega", "motor_rpm", "imu"):
-            assert np.allclose(st[k][0], c[k], rtol=1e-12, atol=1e-12), (c["frame"], c["mode"], k)
+            assert np.array_equal(st[k][0], np.array(c[k])), (c["frame"], c["mode"], k)
 
 
 def test_reference_generated_collision_fixture_vs_port():
@@ -65,9 +67,11 @@ def test_reference_generated_collision_fixture_vs_port():
     assert np.allclose(forces, np.array(g["forces"]), rtol=1e-12, atol=0)
 
 
-@pytest.mark.skipif(O.ref_lib() is None, reason="oracle/_ref/libref_nanoflann.so not built")
 @pytest.mark.parametrize("n,scale", [(1, 1.0), (2, 0.01), (400, 0.5), (5000, 0.3), (40000, 0.35)])
 def test_port_equals_real_nanoflann(n, scale):
+    """Against the reference's nanoflann where oracle/_ref/libref_nanoflann.so is built; otherwise against the stored digests
+    of the results that comparison accepted (golden/nanoflann_port_digests.json: pairs and crash flags equal to nanoflann's,
+    forces within 1e-11 of them)."""
     side = int(np.ceil(np.sqrt(n)))
     k = np.arange(n)
     xyz = np.stack([scale * (4.0 * (k % side) + rand(3, 0, n, -2, 2)), scale * (4.0 * (k // side) + rand(3, 1, n, -2, 2)), rand(3, 2, n, 2, 4)], axis=1)
@@ -77,10 +81,14 @@ def test_port_equals_real_nanoflann(n, scale):
     prop = np.array([AIRFRAMES[f]["prop_radius"] for f in frames])[tou]
     mass = np.array([AIRFRAMES[f]["mass"] for f in frames])[tou]
     for crash in (False, True):
-        a = O.collide_snapshot(xyz, arm, prop, mass, crash, 100.0, engine="nanoflann", n_threads=4)
         b = O.collide_snapshot(xyz, arm, prop, mass, crash, 100.0, engine="port", n_threads=4)
-        pa = a[0][np.lexsort((a[0][:, 1], a[0][:, 0]))] if len(a[0]) else a[0]
         pb = b[0][np.lexsort((b[0][:, 1], b[0][:, 0]))] if len(b[0]) else b[0]
+        if O.ref_lib() is None:
+            stored = load("nanoflann_port_digests.json")["cases"][f"{n}-{scale}-{int(crash)}"]
+            assert [digest(pb), digest(b[2]), digest(b[1])] == stored, "pairs, crash flags, forces"
+            continue
+        a = O.collide_snapshot(xyz, arm, prop, mass, crash, 100.0, engine="nanoflann", n_threads=4)
+        pa = a[0][np.lexsort((a[0][:, 1], a[0][:, 0]))] if len(a[0]) else a[0]
         assert np.array_equal(pa, pb)
         assert np.array_equal(a[2], b[2])
         assert np.allclose(a[1], b[1], rtol=1e-11, atol=0)

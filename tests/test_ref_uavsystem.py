@@ -1,37 +1,48 @@
 """The restated oracle (oracle/uav_oracle.hpp) against the reference's OWN UavSystem sources.
 
 oracle/_ref/libref_uavsystem.so is uav_system.hpp + multirotor_model.hpp + controllers/*.hpp of the
-reference, compiled unmodified from /root/reference/include; only Eigen and Boost.odeint (absent
+reference, compiled unmodified from the reference tree's include/; only Eigen and Boost.odeint (absent
 from the image) are replaced by the stand-ins under oracle/shim.  Both sides follow the same Eigen
 evaluation rules, so the comparison is BIT-EXACT: any difference in dispatch, gains, clamps,
 patches, NaN guards or scalar formulae between the restatement and the reference's code shows up
 as a non-zero difference.  CPU only; the prebuilt library travels to the GPU box, where
 tests/test_ref_uavsystem_gpu.py compares the CUDA path with it directly.
+
+Without that library (the repository does not contain the reference's sources) every observation the
+tests make of the reference side, PIDController results and default parameters included, is checked
+against its stored digest (tests/golden/ref_uavsystem_digests.json, helpers.StoredResults).
 """
 import os
 
 import numpy as np
 import pytest
 
-from helpers import grid_spawn, rand
+from helpers import StoredResults, grid_spawn, rand
 from mrs_multirotor_simulator_b200.airframes import airframe
 from oracle import binding as O
 from test_step_parity import ALL_MODES, _commands
 
 FIELDS = ("x", "v", "R", "omega", "motor_rpm", "v_prev", "imu")
-
-if O.refsys_lib() is None:
-    if os.path.exists("/root/reference/include/mrs_multirotor_simulator/uav_system/uav_system.hpp"):
-        O.build()  # the reference tree is here: the library must build
-    if O.refsys_lib() is None:
-        pytest.skip("oracle/_ref/libref_uavsystem.so not built and no reference tree to build it from", allow_module_level=True)
+STORED = StoredResults(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_uavsystem_digests.json"))
+Ref = STORED.swarm()
+ref_lib = O.refsys_lib if STORED.mode != "check" else O.lib
 
 
-def pair(types, n, type_of_uav=None, spawn=None, heading=None, flavour="default"):
+@pytest.fixture(scope="module", autouse=True)
+def _stored_results():
+    yield from STORED.module()
+
+
+@pytest.fixture(autouse=True)
+def _observations(request):
+    yield from STORED.run(request.node.name)
+
+
+def pair(types, n, type_of_uav=None, spawn=None, heading=None):
     spawn = grid_spawn(n, z=10.0) if spawn is None else np.asarray(spawn, dtype=np.float64)
     heading = np.zeros(n) if heading is None else heading
     kw = dict(type_of_uav=type_of_uav, spawn_xyz=spawn, spawn_heading=heading, n=n)
-    return O.OracleSwarm(types, **kw), O.RefSwarm(types, flavour=flavour, **kw)
+    return O.OracleSwarm(types, **kw), Ref(types, **kw)
 
 
 def assert_identical(orc, ref, what="", pid=True):
@@ -85,7 +96,7 @@ def test_golden_modes_fixture_is_the_compiled_reference():
     with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "modes_2s.json")) as f:
         g = json.load(f)
     for c in g["cases"]:
-        ref = O.RefSwarm([airframe(c["frame"])], spawn_xyz=[g["spawn"]], spawn_heading=[g["heading"]], n=1)
+        ref = Ref([airframe(c["frame"])], spawn_xyz=[g["spawn"]], spawn_heading=[g["heading"]], n=1)
         ref.set_input(c["mode_id"], [c["cmd"]])
         ref.make_step(c["dt"], c["steps"])
         st = ref.get_state()
@@ -250,15 +261,17 @@ def test_pid_controller_is_the_reference_class():
         for _ in range(20):
             e, dt = rng.uniform(-2, 2), rng.choice([0.001, 0.01, 0.02])
             ra = O.lib().orc_pid_update(O._p(sa), kp, kd, ki, sat, aw, e, dt)
-            rb = O.refsys_lib().orc_pid_update(O._p(sb), kp, kd, ki, sat, aw, e, dt)
+            rb = ref_lib().orc_pid_update(O._p(sb), kp, kd, ki, sat, aw, e, dt)
+            STORED.observe(np.append(rb, sb))
             assert ra == rb and np.array_equal(sa, sb)
 
 
 def test_header_default_model_params():
     a, b = O.OrcModelParams(), O.OrcModelParams()
     O.lib().orc_model_params_default(O.C.byref(a))
-    O.refsys_lib().orc_model_params_default(O.C.byref(b))
+    ref_lib().orc_model_params_default(O.C.byref(b))
     b.ground_z = a.ground_z  # the reference's default constructor leaves ground_z uninitialised (multirotor_model.hpp:84)
+    STORED.observe(b)
     assert bytes(a) == bytes(b)
     assert a.n_motors == 4 and a.mass == 2.0 and a.takeoff_patch_enabled == 1 and a.ground_enabled == 0
 

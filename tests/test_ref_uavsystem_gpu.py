@@ -1,18 +1,33 @@
-"""The CUDA stepping path against the reference's OWN UavSystem sources (oracle/_ref/libref_uavsystem.so:
-uav_system.hpp, multirotor_model.hpp, controllers/*.hpp compiled unmodified against the Eigen/odeint
-stand-ins of oracle/shim — built in the container that has /root/reference, shipped prebuilt to the GPU
-box).  Same tolerances as against the restated oracle (helpers.TOL, DESIGN.md §5)."""
+"""The CUDA stepping path against the reference side of tests/test_ref_uavsystem.py: the reference's OWN
+UavSystem sources (oracle/_ref/libref_uavsystem.so: uav_system.hpp, multirotor_model.hpp,
+controllers/*.hpp compiled unmodified against the Eigen/odeint stand-ins of oracle/shim) where that
+build is present.  Without it the restatement stands in, and every state and crash flag it hands these
+tests must equal its stored digest (tests/golden/ref_uavsystem_gpu_digests.json, helpers.StoredResults),
+so that the GPU is compared with fixed results, not with whatever the restatement computes today.
+Same tolerances as against the restated oracle (helpers.TOL, DESIGN.md §5)."""
+import os
+
 import numpy as np
 import pytest
 
-from helpers import TOL, grid_spawn, rand
+from helpers import TOL, StoredResults, grid_spawn, rand
 from oracle import binding as O
 from test_step_parity import ALL_MODES, _commands, af
 
 pytestmark = pytest.mark.gpu
 
-if O.refsys_lib() is None:
-    pytest.skip("oracle/_ref/libref_uavsystem.so was not shipped", allow_module_level=True)
+STORED = StoredResults(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_uavsystem_gpu_digests.json"))
+Ref = STORED.swarm()
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _stored_results():
+    yield from STORED.module()
+
+
+@pytest.fixture(autouse=True)
+def _observations(request):
+    yield from STORED.run(request.node.name)
 
 
 def make(types, tou, spawn, heading=None):
@@ -20,7 +35,7 @@ def make(types, tou, spawn, heading=None):
 
     n = len(spawn)
     heading = np.zeros(n) if heading is None else heading
-    ref = O.RefSwarm(types, type_of_uav=tou, spawn_xyz=spawn, spawn_heading=heading, n=n)
+    ref = Ref(types, type_of_uav=tou, spawn_xyz=spawn, spawn_heading=heading, n=n)
     gpu = UavBatch(types, type_of_uav=tou, spawn_xyz=spawn, spawn_heading=heading, n=n, device=0)
     return ref, gpu
 
@@ -36,7 +51,7 @@ def check(ref, gpu, what, tol=TOL):
     assert not bad, f"{what}: " + "; ".join(bad)
 
 
-def test_c1_single_x500_position_cmd_10s_vs_compiled_reference():
+def test_c1_single_x500_position_cmd_10s():
     ref, gpu = make([af("x500")], None, np.array([[0.0, 0.0, 1.0]]))
     for s in (ref, gpu):
         s.set_input(O.POSITION_CMD, [[5.0, -3.0, 4.0, 1.0]])
@@ -48,7 +63,7 @@ def test_c1_single_x500_position_cmd_10s_vs_compiled_reference():
 
 @pytest.mark.parametrize("frame", ["x500", "f550", "naki"])
 @pytest.mark.parametrize("mode", [m for m in ALL_MODES if m not in (O.ACTUATOR_CMD, O.CONTROL_GROUP_CMD, O.ATTITUDE_RATE_CMD)])
-def test_10s_closed_loop_modes_vs_compiled_reference(mode, frame):
+def test_10s_closed_loop_modes(mode, frame):
     n = 64
     ref, gpu = make([af(frame)], None, grid_spawn(n, z=10.0), rand(3, 0, n, -3, 3))
     cmd = _commands(mode, n)
@@ -65,7 +80,7 @@ def test_10s_closed_loop_modes_vs_compiled_reference(mode, frame):
 
 
 @pytest.mark.parametrize("mode", [O.ACTUATOR_CMD, O.CONTROL_GROUP_CMD, O.ATTITUDE_RATE_CMD])
-def test_open_loop_modes_vs_compiled_reference(mode):
+def test_open_loop_modes(mode):
     """Open loop in attitude: compare one second tightly, before the tumbling amplifies rounding."""
     n = 64
     ref, gpu = make([af("x500")], None, grid_spawn(n, z=10.0), rand(3, 0, n, -3, 3))
@@ -78,7 +93,7 @@ def test_open_loop_modes_vs_compiled_reference(mode):
     check(ref, gpu, f"mode {mode}")
 
 
-def test_c5_mixed_airframes_and_events_vs_compiled_reference():
+def test_c5_mixed_airframes_and_events():
     """Mixed 4/6/8-motor swarm, ground plane, custom gains, feed-forward, crash, force — 6 s."""
     n = 96
     types = [af(f, ground_enabled=True, ground_z=0.0) for f in ("x500", "f550", "naki")]
@@ -105,10 +120,10 @@ def test_c5_mixed_airframes_and_events_vs_compiled_reference():
 
 
 @pytest.mark.parametrize("seed", range(6))
-def test_random_event_sequences_vs_compiled_reference(seed):
+def test_random_event_sequences(seed):
     """Fuzz with finite, flight-like payloads: random commands of every mode, feed-forwards, forces, moments,
     gains, crashes, unknown input and setParams between steps of varying dt on a mixed 4/6/8-motor swarm.
-    After every event the CUDA state must be within tolerance of the reference's own code; it is then
+    After every event the CUDA state must be within tolerance of the reference side; it is then
     re-synchronised to it (set_state), so that the open-loop modes' instability does not accumulate."""
     rng = np.random.default_rng(2000 + seed)
     n = 16
