@@ -255,6 +255,26 @@ int mrsb_get_imu_acceleration(mrsb_handle h, int64_t n, const int32_t* idx, doub
 int mrsb_set_state(mrsb_handle h, int64_t n, const int32_t* idx, const double* x, const double* v, const double* R, const double* omega, const double* motor_rpm);
 /* MultirotorModel::setStatePos (MM:439-446): x := pos, initial_pos := pos, R := Rz(-heading). */
 int mrsb_set_state_pos(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading);
+/* Episode reset.  UavSystem(params, spawn_pos, spawn_heading) (US:144-153) again for the n UAVs idx[] (NULL: 0..n-1), keeping
+ * their airframe, parameter edits (mrsb_set_params / mrsb_set_mass / mrsb_set_ground_z) and controller gains; xyz[n][3],
+ * heading[n] in host memory.  Afterwards each of them is exactly a freshly created UAV with those parameters and gains:
+ *   x = xyz, spawn z = xyz.z, R = Rz(-heading) (as mrsb_set_state_pos); v = omega = 0, motor RPM = 0, IMU acceleration = 0,
+ *   v_prev = v; all twelve PIDs zero; input mode INPUT_UNKNOWN with no command ever received (with iterate_without_input
+ *   off it stays frozen until its next command, ROSW:265); no feed-forwards; zero external force and moment; not crashed.
+ * The take-off patch flag (MM:87, MM:275) gets the value of the UAV's parameter set, i.e. the one given at mrsb_create or by the
+ * last mrsb_set_params (mrsb_set_mass / mrsb_set_ground_z keep it): a UAV respawned on the ground gets the one-way patch
+ * again, as a newly spawned one would.  (A reference user who rebuilt a UavSystem from getParams() after take-off would pass
+ * the consumed flag instead.)  The ROS wrapper's two warm-up steps (ROSW:223-232) are not part of UavSystem and not done.
+ * Local to this shard (not collective); may be issued anywhere between two collision passes.  n == 0 is a no-op; duplicate
+ * indices are undefined, as with every setter. */
+int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading);
+/* Same for every local UAV i with mask_dev[i] != 0 (uint8, n_local entries: a torch.bool tensor works as is); xyz_dev[n_local][3]
+ * and heading_dev[n_local] are DEVICE arrays, read only where the mask is set.  Enqueued on the handle's stream; no host
+ * synchronisation, no host round trip; the host never learns whether anybody was respawned.  A mask with a bit set makes the
+ * next collision pass rebuild its table (on every rank of a pull-exchange run); an all-zero mask changes nothing.  The batch
+ * counts as mixed-mode afterwards: an RL loop sets its commands for the whole batch next (mrsb_set_input_device with
+ * idx_dev == NULL), which keeps the stepping kernel specialised for that mode. */
+int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const double* xyz_dev, const double* heading_dev);
 /* Current INPUT_MODE of each UAV (US:95). */
 int mrsb_get_input_mode(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* mode);
 

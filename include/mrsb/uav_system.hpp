@@ -122,6 +122,9 @@ public:
 
   std::vector<double> getMixerAllocation(void);  // row-major n_motors x 4
 
+  // episode reset: UavSystem(params, pos, heading) again (uav_system.hpp:144-153), keeping parameters and gains (mrsb_respawn)
+  void respawn(const Vec3& pos, double heading);
+
 private:
   Swarm*  swarm_;
   int32_t i_;
@@ -171,6 +174,8 @@ public:
   // after writing through mrsb_get_device_view: positions / external forces were changed behind the library's back
   void positionsWritten() { check(mrsb_publish_positions(h_)); }
   void forcesWritten() { check(mrsb_forces_written(h_)); }
+  // episode reset of n UAVs (idx == nullptr: 0..n-1) at xyz[n][3], heading[n] (mrsb_respawn)
+  void respawn(int64_t n, const int32_t* idx, const double* xyz, const double* heading) { check(mrsb_respawn(h_, n, idx, xyz, heading)); }
   mrsb_handle handle() { return h_; }
 
 private:
@@ -285,5 +290,6 @@ inline std::vector<double> UavSystem::getMixerAllocation(void) {
   check(mrsb_get_mixer_allocation(swarm_->handle(), i_, m));
   return std::vector<double>(m, m + 4 * getParams().n_motors);
 }
+inline void UavSystem::respawn(const Vec3& pos, double heading) { swarm_->respawn(1, &i_, pos.data(), &heading); }
 
 }  // namespace mrsb

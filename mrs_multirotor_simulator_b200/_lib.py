@@ -93,6 +93,8 @@ SIGNATURES = {
     "mrsb_get_imu_acceleration": (C.c_int, _N_IDX + [C.c_void_p]),
     "mrsb_set_state": (C.c_int, _N_IDX + [C.c_void_p] * 5),
     "mrsb_set_state_pos": (C.c_int, _N_IDX + [C.c_void_p, C.c_void_p]),
+    "mrsb_respawn": (C.c_int, _N_IDX + [C.c_void_p, C.c_void_p]),
+    "mrsb_respawn_masked_device": (C.c_int, [H, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mrsb_get_input_mode": (C.c_int, _N_IDX + [C.c_void_p]),
     "mrsb_crash": (C.c_int, _N_IDX),
     "mrsb_has_crashed": (C.c_int, _N_IDX + [C.c_void_p]),

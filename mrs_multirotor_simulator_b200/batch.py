@@ -207,6 +207,20 @@ class UavBatch:
         heading = np.ascontiguousarray(heading, dtype=np.float64).reshape(n)
         check(self._L.mrsb_set_state_pos(self.h, n, _ptr(idx), _ptr(xyz), _ptr(heading)))
 
+    def respawn(self, xyz, heading, idx=None):
+        """Episode reset: `UavSystem(params, pos, heading)` again for the addressed UAVs (uav_system.hpp:144-153), keeping their
+        airframe, parameter edits and controller gains; see mrsb_respawn for what a fresh UAV holds."""
+        idx = _idx(idx)
+        n = self._n(idx)
+        xyz = np.ascontiguousarray(xyz, dtype=np.float64).reshape(n, 3)
+        heading = np.ascontiguousarray(np.broadcast_to(heading, (n,)), dtype=np.float64)
+        check(self._L.mrsb_respawn(self.h, n, _ptr(idx), _ptr(xyz), _ptr(heading)))
+
+    def respawn_masked_device(self, mask_ptr, xyz_ptr, heading_ptr):
+        """respawn() for every UAV i with mask[i] != 0, all three raw device addresses (e.g. torch tensor .data_ptr()): mask
+        uint8 / bool [n], xyz float64 [n][3], heading float64 [n].  Enqueued on the handle's stream, no host synchronisation."""
+        check(self._L.mrsb_respawn_masked_device(self.h, mask_ptr, xyz_ptr, heading_ptr))
+
     def get_input_mode(self, idx=None):
         idx = _idx(idx)
         out = np.empty(self._n(idx), dtype=np.int32)

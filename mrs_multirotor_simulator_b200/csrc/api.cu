@@ -101,6 +101,7 @@ struct mrsb_sim {
   std::vector<int32_t>       pset_host;  // [n_global]
   DevParams*                 d_params     = nullptr;
   int                        d_params_cap = 0;
+  uint8_t*                   d_takeoff0   = nullptr;  // [d_params_cap] initial take-off flag of every set (what a respawn restores)
   int32_t*                   d_pset       = nullptr;
   bool                       params_dirty = true;
 
@@ -278,15 +279,22 @@ static int flush_params(mrsb_sim* h) {
   if (n_sets > h->d_params_cap) {
     CU(cudaStreamSynchronize(h->stream));
     if (h->d_params) CU(cudaFree(h->d_params));
+    if (h->d_takeoff0) CU(cudaFree(h->d_takeoff0));
     h->d_params_cap = std::max(16, 2 * n_sets);
     CU(cudaMalloc(&h->d_params, sizeof(DevParams) * h->d_params_cap));
+    CU(cudaMalloc(&h->d_takeoff0, size_t(h->d_params_cap)));
     h->ds.params = h->d_params;
     drop_collision_graphs(h);
   }
   std::vector<DevParams> host(n_sets);
-  for (int k = 0; k < n_sets; k++) mrsb_derive(h->sets[k].mp, h->sets[k].cp, &host[k]);
+  std::vector<uint8_t>   takeoff0(size_t(n_sets), 0);
+  for (int k = 0; k < n_sets; k++) {
+    mrsb_derive(h->sets[k].mp, h->sets[k].cp, &host[k]);
+    takeoff0[size_t(k)] = h->sets[k].mp.takeoff_patch_enabled != 0;
+  }
   CU(cudaMemcpyAsync(h->d_params, host.data(), sizeof(DevParams) * n_sets, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaStreamSynchronize(h->stream));  // `host` goes out of scope
+  CU(cudaMemcpyAsync(h->d_takeoff0, takeoff0.data(), size_t(n_sets), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaStreamSynchronize(h->stream));  // `host` and `takeoff0` go out of scope
   h->filt_dt = -1.0;                     // DevParams::filt has to be prepared again (ensure_filt)
   for (mrsb_sim::Bucket& b : h->buckets) {
     int nm = -1, ps = -2;
@@ -667,7 +675,7 @@ int mrsb_destroy(mrsb_handle h) {
   if (h->h_one) cudaFreeHost(h->h_one);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
   void* ptrs[] = {h->ds.st,     h->ds.vprev,  h->ds.rpm,      h->ds.pid,      h->ds.fext,         h->ds.mext,       h->ds.imu,    h->ds.initz,
-                  h->ds.cmd,    h->ds.ff,     h->ds.flags,    h->ds.mode,     h->ds.gpos,         h->d_params,      h->d_pset,    h->d_stage,
+                  h->ds.cmd,    h->ds.ff,     h->ds.flags,    h->ds.mode,     h->ds.gpos,         h->d_params,      h->d_takeoff0, h->d_pset,    h->d_stage,
                   h->d_idx,     h->grid.bucket, h->grid.rank, h->grid.count, h->grid.aabb, h->grid.begin, h->grid.rec, h->grid.pairs,
                   h->grid.counters, h->grid.tl, h->grid.scan_state, h->grid.halo_rec, h->grid.halo_bucket, h->grid.halo_rank, h->grid.halo_n, h->grid.halo_work,
                   h->grid.nl_count, h->grid.nl_items, h->grid.nl_active, h->grid.act_items, h->grid.ctl};
@@ -1565,6 +1573,47 @@ int mrsb_set_state_pos(mrsb_handle h, int64_t n, const int32_t* idx, const doubl
   h->positions_touched = true;
   CU(cudaGetLastError());
   return MRSB_OK;
+}
+
+// after a respawn: the buffer peers read has to show the new positions, and their per-group boxes (pull exchange)
+static int respawned(mrsb_sim* h) {
+  if (h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);
+  h->wrote_since_pass = true;
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
+int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading) {
+  GUARD(h);
+  const int32_t* d_idx = nullptr;
+  int            rc    = stage_idx(h, n, idx, &d_idx);
+  if (rc) return rc;
+  if (n == 0) return MRSB_OK;
+  if (!xyz || !heading) return fail(MRSB_ERR_INVALID, "null payload");
+  rc = flush_params(h);  // the kernel reads the take-off flag of every UAV's parameter set
+  if (rc) return rc;
+  rc = ensure_stage(h, sizeof(double) * 4 * size_t(n));
+  if (rc) return rc;
+  double* d_xyz = reinterpret_cast<double*>(h->d_stage);
+  double* d_hdg = d_xyz + 3 * n;
+  CU(cudaMemcpyAsync(d_xyz, xyz, sizeof(double) * 3 * size_t(n), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(d_hdg, heading, sizeof(double) * size_t(n), cudaMemcpyHostToDevice, h->stream));
+  h->n_launches += launch_respawn(h->ds, h->d_takeoff0, n, d_idx, d_xyz, d_hdg, h->stream);
+  h->positions_touched = true;
+  note_mode(h, MRSB_INPUT_UNKNOWN, n, idx == nullptr);
+  return respawned(h);
+}
+
+int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const double* xyz_dev, const double* heading_dev) {
+  GUARD(h);
+  if (!mask_dev || !xyz_dev || !heading_dev) return fail(MRSB_ERR_INVALID, "null device pointer");
+  int rc = flush_params(h);
+  if (rc) return rc;
+  // the host does not learn who was respawned: the kernel raises the displacement word itself (no forced rebuild from here), and
+  // the batch can no longer be assumed to share one input mode unless it is already INPUT_UNKNOWN
+  h->n_launches += launch_respawn_masked(h->ds, h->d_takeoff0, mask_dev, xyz_dev, heading_dev, h->stream);
+  note_mode(h, MRSB_INPUT_UNKNOWN, 1, false);
+  return respawned(h);
 }
 
 int mrsb_get_input_mode(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* mode) {

@@ -69,6 +69,9 @@ struct DevParams {
   double att_kp, att_kd, att_ki, att_sat_rp, att_sat_yaw;
   double rate_kp[3], rate_kd[3], rate_ki[3];  // already multiplied by J_ii (CTL/rate_controller.hpp:62-64)
 };
+// The staged stepping kernel takes a DevParams (and a DevState) by value: a field added to either moves the kernel's parameter
+// layout, which has been seen to change its register allocation and spills.  What only other kernels need goes beside them:
+// the initial take-off flag of every parameter set (mrsb_sim::d_takeoff0), read by the respawn kernels.
 
 // Device pointers of one shard.  Passed to kernels by value.
 struct DevState {
@@ -215,6 +218,12 @@ int launch_gather_u32(const uint32_t* src, int64_t n, const int32_t* idx_dev, ui
 int launch_gather_u8(const uint8_t* src, int64_t n, const int32_t* idx_dev, int32_t* out_dev, const int32_t* perm, cudaStream_t stream);
 int launch_set_mode(const DevState& s, int64_t n, const int32_t* idx_dev, int mode, cudaStream_t stream);
 int launch_set_state_pos(const DevState& s, int64_t n, const int32_t* idx_dev, const double* xyz_dev, const double* hdg_dev, cudaStream_t stream);
+// UavSystem(params, pos, heading) again for the addressed UAVs (payload rows k) / for every UAV e with mask[e] != 0 (payload rows
+// e; raises the displacement word when it respawned anybody).  takeoff0[set]: initial take-off flag of each parameter set.
+int launch_respawn(const DevState& s, const uint8_t* takeoff0, int64_t n, const int32_t* idx_dev, const double* xyz_dev, const double* hdg_dev,
+                   cudaStream_t stream);
+int launch_respawn_masked(const DevState& s, const uint8_t* takeoff0, const uint8_t* mask_dev, const double* xyz_dev, const double* hdg_dev,
+                          cudaStream_t stream);
 int launch_stash_vprev(const DevState& s, int64_t n, const int32_t* idx_dev, cudaStream_t stream);
 int launch_gather_vprev(const DevState& s, int64_t n, const int32_t* idx_dev, double* out_dev, cudaStream_t stream);
 // zero the state (last error and integral) of PIDs [pid0, pid0 + n_pids)

@@ -86,16 +86,10 @@ __global__ void gather_u8_kernel(const uint8_t* __restrict__ src, int64_t n, con
   out[k] = int32_t(src[at(perm, idx, k)]);
 }
 
-// MultirotorModel::setStatePos (MM:439-446): x, _initial_pos_, R = AngleAxis(-heading, z)
-__global__ void set_state_pos_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ xyz,
-                                     const double* __restrict__ hdg) {
-  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (k >= n) return;
-  const int64_t e  = ext(idx, k);
-  const int64_t i  = s.perm ? int64_t(s.perm[e]) : e;
-  const double  px = xyz ? xyz[3 * k] : 0.0, py = xyz ? xyz[3 * k + 1] : 0.0, pz = xyz ? xyz[3 * k + 2] : 0.0;
-  double        sn, cs;
-  sincos(hdg ? -hdg[k] : -0.0, &sn, &cs);
+// MultirotorModel::setStatePos (MM:439-446) of the UAV in slot i, external index e: x, _initial_pos_, R = AngleAxis(-heading, z)
+DEV void write_pose(const DevState& s, int64_t i, int64_t e, double px, double py, double pz, double neg_hdg) {
+  double sn, cs;
+  sincos(neg_hdg, &sn, &cs);
   s.st[tix(ST_ROWS, 0, i)] = px;
   s.st[tix(ST_ROWS, 1, i)] = py;
   s.st[tix(ST_ROWS, 2, i)] = pz;
@@ -114,6 +108,56 @@ __global__ void set_state_pos_kernel(DevState s, int64_t n, const int32_t* __res
   gp[0]             = px;
   gp[1]             = py;
   gp[2]             = pz;
+}
+
+__global__ void set_state_pos_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ xyz,
+                                     const double* __restrict__ hdg) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int64_t e = ext(idx, k);
+  write_pose(s, s.perm ? int64_t(s.perm[e]) : e, e, xyz ? xyz[3 * k] : 0.0, xyz ? xyz[3 * k + 1] : 0.0, xyz ? xyz[3 * k + 2] : 0.0,
+             hdg ? -hdg[k] : -0.0);
+}
+
+// UavSystem(params, pos, heading) (US:144-153 -> MM:183-198 + MM:439-446) for the UAV in slot i, external index e, keeping its
+// parameter set (airframe, edits, controller gains): everything a fresh handle holds after mrsb_create.  v_prev is not written:
+// with FLAG_VPREV clear it reads as v.
+DEV void respawn_one(const DevState& s, const uint8_t* takeoff0, int64_t i, int64_t e, double px, double py, double pz, double hdg) {
+  write_pose(s, i, e, px, py, pz, -hdg);
+  for (int r = 3; r < 6; r++) s.st[tix(ST_ROWS, r, i)] = 0.0;  // v
+  for (int r = 15; r < ST_ROWS; r++) s.st[tix(ST_ROWS, r, i)] = 0.0;  // omega
+  for (int r = 0; r < MRSB_NM; r++) s.rpm[tix(MRSB_NM, r, i)] = 0.0;
+  for (int r = 0; r < PID_ROWS; r++) s.pid[tix(PID_ROWS, r, i)] = 0.0;  // CTL/*::setParams reset every PID
+  for (int r = 0; r < CMD_ROWS; r++) s.cmd[tix(CMD_ROWS, r, i)] = 0.0;
+  for (int r = 0; r < FF_ROWS; r++) s.ff[tix(FF_ROWS, r, i)] = 0.0;
+  for (int r = 0; r < F3_ROWS; r++) {
+    s.fext[tix(F3_ROWS, r, i)] = 0.0;
+    s.mext[tix(F3_ROWS, r, i)] = 0.0;
+    s.imu[tix(F3_ROWS, r, i)]  = 0.0;
+  }
+  s.mode[i]  = uint8_t(MRSB_INPUT_UNKNOWN);
+  // crashed, v_prev, feed-forwards and "had a command" cleared; the take-off patch as the parameter set carries it (MM:87)
+  s.flags[i] = takeoff0[s.pset[s.shard_begin + e]] ? FLAG_TAKEOFF : 0u;
+}
+
+__global__ void respawn_kernel(DevState s, const uint8_t* __restrict__ takeoff0, int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ xyz, const double* __restrict__ hdg) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int64_t e = ext(idx, k);
+  respawn_one(s, takeoff0, s.perm ? int64_t(s.perm[e]) : e, e, xyz[3 * k], xyz[3 * k + 1], xyz[3 * k + 2], hdg[k]);
+}
+
+// One thread per SLOT (tile order), so that a warp's stores to a row of the tiled arrays are coalesced when many UAVs respawn.
+// A respawned UAV moved behind the stepping kernel's displacement bound: the displacement word is raised to "unbounded" (read as
+// NaN by decide_kernel: the next pass rebuilds, and in pull-exchange runs the word travels to every peer) — one atomic per warp
+// that respawned anybody, none otherwise.
+__global__ void respawn_masked_kernel(DevState s, const uint8_t* __restrict__ takeoff0, const uint8_t* __restrict__ mask, const double* __restrict__ xyz, const double* __restrict__ hdg) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  int64_t       e = -1;
+  if (i < s.ld) e = s.inv ? int64_t(s.inv[i]) : (i < s.n ? i : -1);
+  const bool hit = e >= 0 && mask[e] != 0;
+  if (hit) respawn_one(s, takeoff0, i, e, xyz[3 * e], xyz[3 * e + 1], xyz[3 * e + 2], hdg[e]);
+  if (s.disp_max && __ballot_sync(0xffffffffu, hit) && (threadIdx.x & 31) == 0) atomicMax(s.disp_max, 0xFFFFFFFFu);
 }
 
 // before set_state overwrites v: remember the old v as v_prev (MM:424-433 leaves v_prev alone)
@@ -356,6 +400,16 @@ int launch_gather_u8(const uint8_t* src, int64_t n, const int32_t* idx, int32_t*
 int launch_set_state_pos(const DevState& s, int64_t n, const int32_t* idx, const double* xyz, const double* hdg, cudaStream_t st) {
   if (n <= 0) return 0;
   set_state_pos_kernel<<<nblk(n), 256, 0, st>>>(s, n, idx, xyz, hdg);
+  return 1;
+}
+int launch_respawn(const DevState& s, const uint8_t* takeoff0, int64_t n, const int32_t* idx, const double* xyz, const double* hdg, cudaStream_t st) {
+  if (n <= 0) return 0;
+  respawn_kernel<<<nblk(n), 256, 0, st>>>(s, takeoff0, n, idx, xyz, hdg);
+  return 1;
+}
+int launch_respawn_masked(const DevState& s, const uint8_t* takeoff0, const uint8_t* mask, const double* xyz, const double* hdg, cudaStream_t st) {
+  if (s.n <= 0) return 0;
+  respawn_masked_kernel<<<nblk(s.ld), 256, 0, st>>>(s, takeoff0, mask, xyz, hdg);  // s.ld is a whole number of warps
   return 1;
 }
 int launch_stash_vprev(const DevState& s, int64_t n, const int32_t* idx, cudaStream_t st) {

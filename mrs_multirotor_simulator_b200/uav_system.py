@@ -145,6 +145,11 @@ class UavSystem:
     def _idx(self):
         return [self._i]
 
+    def respawn(self, spawn_pos=(0.0, 0.0, 0.0), spawn_heading=0.0):
+        """Start over as `UavSystem(params, spawn_pos, spawn_heading)` (uav_system.hpp:144-153) with the current parameters and
+        controller gains; the take-off patch flag is the one given at creation or by the last setParams (see mrsb_respawn)."""
+        self._batch.respawn([list(spawn_pos)], [spawn_heading], self._idx)
+
     # uav_system.hpp:38
     def makeStep(self, dt):
         if not self._owns:
