@@ -10,7 +10,9 @@
 #include <cstring>
 #include <functional>
 #include <map>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "internal.h"
@@ -83,6 +85,58 @@ static int load_nccl() {
   } while (0)
 
 // ------------------------------------------------------------------------------------------
+// memory: the one owner of every allocation
+// ------------------------------------------------------------------------------------------
+// A block of cap() elements of device memory, or of pinned host memory mapped into the device's address space when Pinned.
+// Move-only; the destructor frees it.
+template <class T, bool Pinned = false>
+class Mem {
+ public:
+  Mem() = default;
+  Mem(Mem&& o) noexcept { *this = std::move(o); }
+  Mem& operator=(Mem&& o) noexcept {
+    release();
+    p_ = std::exchange(o.p_, nullptr), cap_ = std::exchange(o.cap_, 0);
+    return *this;
+  }
+  ~Mem() { release(); }
+
+  T*     get() const { return p_; }
+  size_t cap() const { return cap_; }
+
+  int alloc(size_t count) {  // in place of the block held so far
+    Mem m;
+    if (Pinned) {
+      CU(cudaHostAlloc(&m.p_, sizeof(T) * count, cudaHostAllocMapped));
+    } else {
+      CU(cudaMalloc(&m.p_, sizeof(T) * count));
+    }
+    m.cap_ = count;
+    *this  = std::move(m);
+    return MRSB_OK;
+  }
+  // At least `need` elements: a smaller block is replaced by one of `count` >= need elements.  The new block is allocated first;
+  // only then is `stream`, where the old block may still be in use, waited for and the old block freed.  A grow that fails
+  // leaves the old block and its capacity.
+  int grow(size_t need, size_t count, cudaStream_t stream) {
+    if (need <= cap_) return MRSB_OK;
+    Mem m;
+    int rc = m.alloc(count);
+    if (rc) return rc;
+    if (p_) CU(cudaStreamSynchronize(stream));
+    *this = std::move(m);
+    return MRSB_OK;
+  }
+
+ private:
+  void release() {
+    if (p_) Pinned ? cudaFreeHost(p_) : cudaFree(p_);
+  }
+  T*     p_   = nullptr;
+  size_t cap_ = 0;
+};
+
+// ------------------------------------------------------------------------------------------
 // the handle
 // ------------------------------------------------------------------------------------------
 struct ParamSet {
@@ -95,20 +149,21 @@ struct mrsb_sim {
   cudaStream_t stream = nullptr;
   DevState     ds{};
   DevGrid      grid{};
+  Mem<int32_t> pairs;  // grid.pairs (mrsb_set_pair_capacity)
 
   std::vector<ParamSet>      sets;
   std::map<std::string, int> set_index;
+  // everything allocated once, at create or by setup_p2p (dalloc), freed by the destructor
+  std::vector<Mem<unsigned char>> mem;
+
   std::vector<int32_t>       pset_host;  // [n_global]
-  DevParams*                 d_params     = nullptr;
-  int                        d_params_cap = 0;
-  uint8_t*                   d_takeoff0   = nullptr;  // [d_params_cap] initial take-off flag of every set (what a respawn restores)
+  Mem<DevParams>             d_params;
+  Mem<uint8_t>               d_takeoff0;  // initial take-off flag of every set (what a respawn restores)
   int32_t*                   d_pset       = nullptr;
   bool                       params_dirty = true;
 
-  char*    d_stage       = nullptr;  // staging for payload transposes
-  size_t   d_stage_bytes = 0;
-  int32_t* d_idx         = nullptr;
-  size_t   d_idx_cap     = 0;
+  Mem<char>    d_stage;  // staging for payload transposes
+  Mem<int32_t> d_idx;
 
   int  uniform_mode = MRSB_INPUT_UNKNOWN;  // INPUT_MODE shared by all UAVs, or -1 if mixed
   bool any_moment   = false;
@@ -154,17 +209,16 @@ struct mrsb_sim {
   unsigned long long*  d_flags   = nullptr;              // this rank's flag block, written by the peers
   unsigned long long** d_peer_flags = nullptr;           // device array [n_ranks] of the peers' flag blocks
   std::vector<void*>   ipc_opened;
-  int*                 h_status  = nullptr;              // pinned, mapped: set by the hand-shake on time-out
+  Mem<int, true>       h_status;                         // pinned, mapped: set by the hand-shake on time-out
 
   // pipelined host I/O (mrsb_set_input_async / mrsb_get_positions_async)
   cudaStream_t up_stream = nullptr, down_stream = nullptr;
-  double*      d_up[2]   = {nullptr, nullptr};  // staged command rows
-  size_t       d_up_bytes = 0;
-  double*      d_snap[2] = {nullptr, nullptr};  // position snapshots [n_local][3]
+  Mem<double>  d_up[2];    // staged command rows
+  Mem<double>  d_snap[2];  // position snapshots [n_local][3]
   cudaEvent_t  ev_up[2] = {nullptr, nullptr}, ev_applied[2] = {nullptr, nullptr}, ev_snap[2] = {nullptr, nullptr}, ev_down[2] = {nullptr, nullptr};
   uint64_t     n_up = 0, n_down = 0;
-  int32_t*     d_sub_idx = nullptr;  // mrsb_set_position_subset: the UAVs mrsb_get_positions_async downloads (nullptr: all)
-  int64_t      n_sub     = 0;
+  Mem<int32_t> d_sub_idx;  // mrsb_set_position_subset: the UAVs mrsb_get_positions_async downloads (its first n_sub; 0: all)
+  int64_t      n_sub = 0;
 
   // the collision pass is a fixed set of launches with fixed arguments: replayed as a CUDA graph (one per
   // gather-buffer parity; with neighbour lists the table rebuild sits in a conditional node of it);
@@ -180,7 +234,7 @@ struct mrsb_sim {
   int64_t  list_passes         = 0;     // passes that went through decide_kernel (it counts them too: NlCtl::n_passes)
   bool     list_graph_failed   = false; // conditional graph nodes unavailable: do not try again on every pass
   int64_t  rebuilds_counted    = 0;
-  uint32_t* h_one              = nullptr;  // pinned constant 1 (source of the async "force rebuild" copy)
+  Mem<uint32_t, true> h_one;               // pinned constant 1 (source of the async "force rebuild" copy)
   cudaGraphExec_t tick_graph[2] = {nullptr, nullptr};  // mrsb_run: stepping launch + collision pass as ONE graph per parity
   double   tick_dt = 0.0;
   int      tick_k = 0, tick_mode = -2, tick_own[2] = {0, 0};
@@ -275,25 +329,24 @@ static int flush_params(mrsb_sim* h) {
   if (!h->params_dirty) return MRSB_OK;
   int rc = collect_param_sets(h);
   if (rc) return rc;
-  const int n_sets = int(h->sets.size());
-  if (n_sets > h->d_params_cap) {
-    CU(cudaStreamSynchronize(h->stream));
-    if (h->d_params) CU(cudaFree(h->d_params));
-    if (h->d_takeoff0) CU(cudaFree(h->d_takeoff0));
-    h->d_params_cap = std::max(16, 2 * n_sets);
-    CU(cudaMalloc(&h->d_params, sizeof(DevParams) * h->d_params_cap));
-    CU(cudaMalloc(&h->d_takeoff0, size_t(h->d_params_cap)));
-    h->ds.params = h->d_params;
+  const int    n_sets = int(h->sets.size());
+  const size_t cap    = size_t(std::max(16, 2 * n_sets));
+  rc                  = h->d_params.grow(size_t(n_sets), cap, h->stream);
+  if (rc) return rc;
+  if (h->ds.params != h->d_params.get()) {  // the graphs hold the table's address
+    h->ds.params = h->d_params.get();
     drop_collision_graphs(h);
   }
+  rc = h->d_takeoff0.grow(size_t(n_sets), cap, h->stream);
+  if (rc) return rc;
   std::vector<DevParams> host(n_sets);
   std::vector<uint8_t>   takeoff0(size_t(n_sets), 0);
   for (int k = 0; k < n_sets; k++) {
     mrsb_derive(h->sets[k].mp, h->sets[k].cp, &host[k]);
     takeoff0[size_t(k)] = h->sets[k].mp.takeoff_patch_enabled != 0;
   }
-  CU(cudaMemcpyAsync(h->d_params, host.data(), sizeof(DevParams) * n_sets, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(h->d_takeoff0, takeoff0.data(), size_t(n_sets), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->d_params.get(), host.data(), sizeof(DevParams) * n_sets, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->d_takeoff0.get(), takeoff0.data(), size_t(n_sets), cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));  // `host` and `takeoff0` go out of scope
   h->filt_dt = -1.0;                     // DevParams::filt has to be prepared again (ensure_filt)
   for (mrsb_sim::Bucket& b : h->buckets) {
@@ -320,9 +373,9 @@ static int flush_params(mrsb_sim* h) {
 // the staged kernel takes the batch's one set by value, so its host copy gets the device's result.
 static int ensure_filt(mrsb_sim* h, double dt) {
   if (h->filt_dt == dt) return MRSB_OK;
-  h->n_launches += launch_prep_params(h->d_params, int(h->sets.size()), dt, h->stream);
+  h->n_launches += launch_prep_params(h->d_params.get(), int(h->sets.size()), dt, h->stream);
   for (mrsb_sim::Bucket& b : h->buckets)
-    if (b.pset >= 0) CU(cudaMemcpyAsync(&b.params.filt, &h->d_params[b.pset].filt, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    if (b.pset >= 0) CU(cudaMemcpyAsync(&b.params.filt, &h->d_params.get()[b.pset].filt, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   h->filt_dt = dt;
   for (int k = 0; k < 2; k++) {  // the tick graphs hold the parameter set by value
@@ -333,12 +386,7 @@ static int ensure_filt(mrsb_sim* h, double dt) {
 }
 
 static int ensure_stage(mrsb_sim* h, size_t bytes) {
-  if (bytes <= h->d_stage_bytes) return MRSB_OK;
-  CU(cudaStreamSynchronize(h->stream));
-  if (h->d_stage) CU(cudaFree(h->d_stage));
-  h->d_stage_bytes = std::max<size_t>(bytes, 1 << 16);
-  CU(cudaMalloc(&h->d_stage, h->d_stage_bytes));
-  return MRSB_OK;
+  return h->d_stage.grow(bytes, std::max<size_t>(bytes, 1 << 16), h->stream);
 }
 
 // copy an index list to the device (nullptr stays nullptr = identity) after validating it
@@ -348,14 +396,56 @@ static int stage_idx(mrsb_sim* h, int64_t n, const int32_t* idx, const int32_t**
   if (!idx || n == 0) return MRSB_OK;
   for (int64_t k = 0; k < n; k++)
     if (idx[k] < 0 || idx[k] >= h->ds.n) return fail(MRSB_ERR_INVALID, "idx[%lld]=%d outside 0..%lld", (long long)k, idx[k], (long long)h->ds.n - 1);
-  if (size_t(n) > h->d_idx_cap) {
-    CU(cudaStreamSynchronize(h->stream));
-    if (h->d_idx) CU(cudaFree(h->d_idx));
-    h->d_idx_cap = std::max<size_t>(size_t(n), 1024);
-    CU(cudaMalloc(&h->d_idx, sizeof(int32_t) * h->d_idx_cap));
+  int rc = h->d_idx.grow(size_t(n), std::max<size_t>(size_t(n), 1024), h->stream);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(h->d_idx.get(), idx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, h->stream));
+  *out = h->d_idx.get();
+  return MRSB_OK;
+}
+
+// n rows of `width` doubles in host memory
+struct HostRows {
+  const double* rows;
+  int           width;
+};
+
+// the parts back to back into the staging buffer; dev[k]: where part k went
+static int stage_rows(mrsb_sim* h, int64_t n, std::initializer_list<HostRows> parts, const double** dev) {
+  size_t total = 0;
+  for (const HostRows& p : parts) total += size_t(n) * size_t(p.width);
+  int rc = ensure_stage(h, sizeof(double) * total);
+  if (rc) return rc;
+  double* d = reinterpret_cast<double*>(h->d_stage.get());
+  for (const HostRows& p : parts) {
+    CU(cudaMemcpyAsync(d, p.rows, sizeof(double) * size_t(n) * size_t(p.width), cudaMemcpyHostToDevice, h->stream));
+    *dev++ = d;
+    d += size_t(n) * size_t(p.width);
   }
-  CU(cudaMemcpyAsync(h->d_idx, idx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, h->stream));
-  *out = h->d_idx;
+  return MRSB_OK;
+}
+
+// Host -> device for n addressed UAVs: the index list (validated), then, unless n == 0, the payload parts, none of which may be
+// null.  Nothing is launched.
+static int upload(mrsb_sim* h, int64_t n, const int32_t* idx, std::initializer_list<HostRows> parts, const int32_t** d_idx, const double** dev) {
+  int rc = stage_idx(h, n, idx, d_idx);
+  if (rc || n == 0) return rc;
+  for (const HostRows& p : parts)
+    if (!p.rows) return fail(MRSB_ERR_INVALID, "null payload");
+  return stage_rows(h, n, parts, dev);
+}
+
+// Device -> host for n addressed UAVs: the index list (validated), then, unless n == 0, `gather(d_idx, staging)` fills `bytes` of
+// the staging buffer, which are copied to `out` once they are complete.
+template <class Gather>
+static int download(mrsb_sim* h, int64_t n, const int32_t* idx, size_t bytes, void* out, Gather gather) {
+  const int32_t* d_idx = nullptr;
+  int            rc    = stage_idx(h, n, idx, &d_idx);
+  if (rc || n == 0) return rc;
+  rc = ensure_stage(h, bytes);
+  if (rc) return rc;
+  h->n_launches += gather(d_idx, static_cast<void*>(h->d_stage.get()));
+  CU(cudaMemcpyAsync(out, h->d_stage.get(), bytes, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return MRSB_OK;
 }
 
@@ -367,10 +457,16 @@ static int64_t round_up(int64_t v, int64_t m) {
   return (v + m - 1) / m * m;
 }
 
+// *p = a zeroed device array of `count` (at least one) elements that lives as long as the handle
 template <class T>
-static int dalloc(T** p, size_t count) {
-  CU(cudaMalloc(p, sizeof(T) * std::max<size_t>(count, 1)));
-  CU(cudaMemset(*p, 0, sizeof(T) * std::max<size_t>(count, 1)));
+static int dalloc(mrsb_sim* h, T** p, size_t count) {
+  const size_t       bytes = sizeof(T) * std::max<size_t>(count, 1);
+  Mem<unsigned char> m;
+  int                rc = m.alloc(bytes);
+  if (rc) return rc;
+  CU(cudaMemset(m.get(), 0, bytes));
+  *p = reinterpret_cast<T*>(m.get());
+  h->mem.push_back(std::move(m));
   return MRSB_OK;
 }
 
@@ -402,7 +498,7 @@ static int write_buf(const mrsb_sim* h) {
 }
 // geometry of the addressed local UAVs (idx == nullptr: all of them) from the device tables into buffer `b`
 static int apply_geom(mrsb_sim* h, int b, int64_t n, const int32_t* d_idx) {
-  h->n_launches += launch_set_geom(h->d_geom[b], n, d_idx, h->ds.shard_begin, h->d_pset, h->d_params, h->stream);
+  h->n_launches += launch_set_geom(h->d_geom[b], n, d_idx, h->ds.shard_begin, h->d_pset, h->d_params.get(), h->stream);
   CU(cudaGetLastError());
   return MRSB_OK;
 }
@@ -421,7 +517,6 @@ static int geometry_changed(mrsb_sim* h, int64_t n, const int32_t* idx, const in
   }
   return MRSB_OK;
 }
-static int stage_idx(mrsb_sim* h, int64_t n, const int32_t* idx, const int32_t** out);
 static int apply_pending_geom(mrsb_sim* h, int b) {
   std::vector<int32_t>& pend = h->pending_geom[b];
   if (pend.empty()) return MRSB_OK;
@@ -479,8 +574,8 @@ static int repoint(mrsb_sim* h, int64_t n, const int32_t* idx, Edit edit, Key va
   h->params_dirty = true;
   rc              = ensure_stage(h, sizeof(int32_t) * size_t(n));
   if (rc) return rc;
-  CU(cudaMemcpyAsync(h->d_stage, ids.data(), sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_set_pset(h->d_pset, n, d_idx, h->ds.shard_begin, reinterpret_cast<const int32_t*>(h->d_stage), h->stream);
+  CU(cudaMemcpyAsync(h->d_stage.get(), ids.data(), sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice, h->stream));
+  h->n_launches += launch_set_pset(h->d_pset, n, d_idx, h->ds.shard_begin, reinterpret_cast<const int32_t*>(h->d_stage.get()), h->stream);
   CU(cudaStreamSynchronize(h->stream));  // `ids` goes out of scope
   if (geometry) {
     rc = flush_params(h);  // the new sets have to be on the device before the geometry is derived from them
@@ -527,22 +622,23 @@ static void make_local_view(mrsb_sim* h) {
 // IPC mappings of every peer's (handles travel through one NCCL all-gather of raw bytes).
 static int setup_p2p(mrsb_sim* h) {
   const int    G     = h->n_ranks;
-  const size_t bytes = sizeof(double) * 3 * size_t(h->ds.n_global);
-  const size_t gbytes = sizeof(double) * 4 * size_t(h->ds.n_global);
-  const size_t bbytes = sizeof(uint32_t) * 6 * size_t(h->ds.ld / 32 + 1);  // the stepping kernel writes one row per warp of every tile
-  h->gbuf[0]          = h->ds.gpos;
-  CU(cudaMalloc(&h->gbuf[1], std::max<size_t>(bytes, 16)));
-  CU(cudaMemcpy(h->gbuf[1], h->gbuf[0], bytes, cudaMemcpyDeviceToDevice));
-  CU(cudaMalloc(&h->d_geom[1], std::max<size_t>(gbytes, 32)));
-  CU(cudaMemcpy(h->d_geom[1], h->d_geom[0], gbytes, cudaMemcpyDeviceToDevice));
+  const size_t ng    = size_t(h->ds.n_global);
+  h->gbuf[0]         = h->ds.gpos;
+  int rc             = dalloc(h, &h->gbuf[1], 3 * ng);
+  if (rc) return rc;
+  CU(cudaMemcpy(h->gbuf[1], h->gbuf[0], sizeof(double) * 3 * ng, cudaMemcpyDeviceToDevice));
+  rc = dalloc(h, &h->d_geom[1], 4 * ng);
+  if (rc) return rc;
+  CU(cudaMemcpy(h->d_geom[1], h->d_geom[0], sizeof(double) * 4 * ng, cudaMemcpyDeviceToDevice));
   for (int k = 0; k < 2; k++) {
-    CU(cudaMalloc(&h->d_gbox[k], std::max<size_t>(bbytes, 32)));
-    CU(cudaMemset(h->d_gbox[k], 0, std::max<size_t>(bbytes, 32)));
+    rc = dalloc(h, &h->d_gbox[k], 6 * size_t(h->ds.ld / 32 + 1));  // the stepping kernel writes one row per warp of every tile
+    if (rc) return rc;
   }
-  CU(cudaMalloc(&h->d_flags, sizeof(unsigned long long) * 3 * G));  // pass numbers [G] + displacement words [2G]
-  CU(cudaMemset(h->d_flags, 0, sizeof(unsigned long long) * 3 * G));
-  CU(cudaHostAlloc(&h->h_status, sizeof(int), cudaHostAllocMapped));
-  *h->h_status = 0;
+  rc = dalloc(h, &h->d_flags, 3 * size_t(G));  // pass numbers [G] + displacement words [2G]
+  if (rc) return rc;
+  rc = h->h_status.alloc(1);
+  if (rc) return rc;
+  *h->h_status.get() = 0;
   struct Handles {
     cudaIpcMemHandle_t buf[2], box[2], geom[2], flags;
   };
@@ -553,15 +649,15 @@ static int setup_p2p(mrsb_sim* h) {
     CU(cudaIpcGetMemHandle(&mine.geom[k], h->d_geom[k]));
   }
   CU(cudaIpcGetMemHandle(&mine.flags, h->d_flags));
-  Handles* d_all = nullptr;
-  CU(cudaMalloc(&d_all, sizeof(Handles) * G));
-  CU(cudaMemcpyAsync(d_all + h->rank, &mine, sizeof(Handles), cudaMemcpyHostToDevice, h->stream));
-  NC(g_nccl.AllGather(d_all + h->rank, d_all, sizeof(Handles), ncclChar, h->comm, h->stream));
+  Mem<Handles> d_all;
+  rc = d_all.alloc(size_t(G));
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(d_all.get() + h->rank, &mine, sizeof(Handles), cudaMemcpyHostToDevice, h->stream));
+  NC(g_nccl.AllGather(d_all.get() + h->rank, d_all.get(), sizeof(Handles), ncclChar, h->comm, h->stream));
   std::vector<Handles> all;
   all.resize(static_cast<size_t>(G));
-  CU(cudaMemcpyAsync(all.data(), d_all, sizeof(Handles) * G, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(all.data(), d_all.get(), sizeof(Handles) * G, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  CU(cudaFree(d_all));
   std::vector<unsigned long long*> pflags(static_cast<size_t>(G), nullptr);
   for (int k = 0; k < 2; k++) {
     PeerView& v = h->pv[k];
@@ -588,7 +684,7 @@ static int setup_p2p(mrsb_sim* h) {
     }
     void* p = nullptr;
     for (int k = 0; k < 2; k++) {
-      int rc = open(all[size_t(r)].buf[k], &p);
+      rc = open(all[size_t(r)].buf[k], &p);
       if (rc) return rc;
       h->pv[k].pos[r] = static_cast<const double*>(p);
       rc              = open(all[size_t(r)].box[k], &p);
@@ -598,23 +694,24 @@ static int setup_p2p(mrsb_sim* h) {
       if (rc) return rc;
       h->pv[k].geom[r] = static_cast<const double*>(p);
     }
-    int rc = open(all[size_t(r)].flags, &p);
+    rc = open(all[size_t(r)].flags, &p);
     if (rc) return rc;
     pflags[size_t(r)] = static_cast<unsigned long long*>(p);
   }
-  CU(cudaMalloc(&h->d_peer_flags, sizeof(unsigned long long*) * G));
+  rc = dalloc(h, &h->d_peer_flags, size_t(G));
+  if (rc) return rc;
   CU(cudaMemcpy(h->d_peer_flags, pflags.data(), sizeof(unsigned long long*) * G, cudaMemcpyHostToDevice));
   // everybody must have opened everybody's memory before the first hand-shake: one more (tiny) collective
-  unsigned long long* d_tmp = nullptr;
-  CU(cudaMalloc(&d_tmp, sizeof(unsigned long long) * G));
-  NC(g_nccl.AllGather(d_tmp + h->rank, d_tmp, sizeof(unsigned long long), ncclChar, h->comm, h->stream));
+  Mem<unsigned long long> d_tmp;
+  rc = d_tmp.alloc(size_t(G));
+  if (rc) return rc;
+  NC(g_nccl.AllGather(d_tmp.get() + h->rank, d_tmp.get(), sizeof(unsigned long long), ncclChar, h->comm, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  CU(cudaFree(d_tmp));
   h->p2pctl.peer_flags = h->d_peer_flags;
   h->p2pctl.flags      = h->d_flags;
   h->p2pctl.n_ranks    = G;
   h->p2pctl.rank       = h->rank;
-  h->p2pctl.status     = h->h_status;
+  h->p2pctl.status     = h->h_status.get();
   {
     const char* e    = getenv("MRSB_P2P_TIMEOUT_MS");
     h->p2pctl.budget = (e ? atoll(e) : 20000LL) * 2000000LL;  // default 20 s at ~2 GHz SM clock
@@ -647,42 +744,22 @@ int mrsb_version(void) {
 // ------------------------------------------------------------------------------------------
 // lifetime
 // ------------------------------------------------------------------------------------------
+// Nothing is freed while a stream, a graph or a peer's mapping can still reach it.
 int mrsb_destroy(mrsb_handle h) {
   if (!h) return MRSB_OK;
   cudaSetDevice(h->device);
-  if (h->stream) cudaStreamSynchronize(h->stream);
-  if (h->up_stream) cudaStreamSynchronize(h->up_stream);
-  if (h->down_stream) cudaStreamSynchronize(h->down_stream);
-  for (int k = 0; k < 2; k++) {
-    if (h->d_up[k]) cudaFree(h->d_up[k]);
-    if (h->d_snap[k]) cudaFree(h->d_snap[k]);
-    for (cudaEvent_t e : {h->ev_up[k], h->ev_applied[k], h->ev_snap[k], h->ev_down[k]})
-      if (e) cudaEventDestroy(e);
-  }
-  if (h->d_sub_idx) cudaFree(h->d_sub_idx);
-  if (h->up_stream) cudaStreamDestroy(h->up_stream);
-  if (h->down_stream) cudaStreamDestroy(h->down_stream);
+  const cudaStream_t streams[3] = {h->stream, h->up_stream, h->down_stream};
+  for (cudaStream_t s : streams)
+    if (s) cudaStreamSynchronize(s);
   drop_collision_graphs(h);
   for (void* p : h->ipc_opened) cudaIpcCloseMemHandle(p);
-  if (h->p2p || h->gbuf[1]) {  // ds.gpos / ds.geom point at one of the two copies
-    h->ds.gpos = nullptr;
-    for (int k = 0; k < 2; k++)
-      if (h->gbuf[k]) cudaFree(h->gbuf[k]);
-  }
-  for (void* p : {(void*)h->d_perm, (void*)h->d_inv, (void*)h->d_geom[0], (void*)h->d_geom[1], (void*)h->d_gbox[0], (void*)h->d_gbox[1], (void*)h->d_flags, (void*)h->d_peer_flags})
-    if (p) cudaFree(p);
-  if (h->h_status) cudaFreeHost(h->h_status);
-  if (h->h_one) cudaFreeHost(h->h_one);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
-  void* ptrs[] = {h->ds.st,     h->ds.vprev,  h->ds.rpm,      h->ds.pid,      h->ds.fext,         h->ds.mext,       h->ds.imu,    h->ds.initz,
-                  h->ds.cmd,    h->ds.ff,     h->ds.flags,    h->ds.mode,     h->ds.gpos,         h->d_params,      h->d_takeoff0, h->d_pset,    h->d_stage,
-                  h->d_idx,     h->grid.bucket, h->grid.rank, h->grid.count, h->grid.aabb, h->grid.begin, h->grid.rec, h->grid.pairs,
-                  h->grid.counters, h->grid.tl, h->grid.scan_state, h->grid.halo_rec, h->grid.halo_bucket, h->grid.halo_rank, h->grid.halo_n, h->grid.halo_work,
-                  h->grid.nl_count, h->grid.nl_items, h->grid.nl_active, h->grid.act_items, h->grid.ctl};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  if (h->stream) cudaStreamDestroy(h->stream);
-  delete h;
+  for (int k = 0; k < 2; k++)
+    for (cudaEvent_t e : {h->ev_up[k], h->ev_applied[k], h->ev_snap[k], h->ev_down[k]})
+      if (e) cudaEventDestroy(e);
+  delete h;  // frees the memory
+  for (cudaStream_t s : streams)
+    if (s) cudaStreamDestroy(s);
   return MRSB_OK;
 }
 
@@ -738,30 +815,11 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
   if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) return fail(MRSB_ERR_CUDA, "no CUDA device available (libmrsb has no CPU fallback)");
   if (info->device < 0 || info->device >= n_dev) return fail(MRSB_ERR_INVALID, "device %d outside 0..%d", info->device, n_dev - 1);
 
-  mrsb_sim* h = new mrsb_sim();
+  std::unique_ptr<mrsb_sim, int (*)(mrsb_handle)> guard(new mrsb_sim(), mrsb_destroy);  // destroys what a failed create made
+  mrsb_sim* h = guard.get();
   h->device   = info->device;
-#define CREATE_CU(call)                      \
-  do {                                       \
-    int rc_ = [&]() -> int {                 \
-      CU(call);                              \
-      return MRSB_OK;                        \
-    }();                                     \
-    if (rc_) {                               \
-      mrsb_destroy(h);                       \
-      return rc_;                            \
-    }                                        \
-  } while (0)
-#define CREATE_RC(expr)  \
-  do {                   \
-    int rc_ = (expr);    \
-    if (rc_) {           \
-      mrsb_destroy(h);   \
-      return rc_;        \
-    }                    \
-  } while (0)
-
-  CREATE_CU(cudaSetDevice(h->device));
-  CREATE_CU(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
 
   DevState& s   = h->ds;
   s.n           = info->n_local;
@@ -776,10 +834,7 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     std::vector<int32_t> slot_of(size_t(std::max<int64_t>(s.n, 1)), 0);
     int64_t              n_slots   = 0;
     const int            n_buckets = mrsb_bucket_layout(s.n, info->n_types, type_local.data(), slot_of.data(), &n_slots, first.data(), count.data());
-    if (n_buckets < 0) {
-      mrsb_destroy(h);
-      return n_buckets;
-    }
+    if (n_buckets < 0) return n_buckets;
     s.ld = n_slots;
     if (n_buckets > 1) {
       for (int t = 0; t < info->n_types; t++) {
@@ -798,28 +853,31 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     }
   }
   const size_t ld = size_t(s.ld);
+  int          rc = MRSB_OK;
   if (!h->perm_host.empty()) {
-    CREATE_RC(dalloc(&h->d_perm, size_t(s.n)));
-    CREATE_RC(dalloc(&h->d_inv, ld));
-    CREATE_CU(cudaMemcpy(h->d_perm, h->perm_host.data(), sizeof(int32_t) * size_t(s.n), cudaMemcpyHostToDevice));
-    CREATE_CU(cudaMemcpy(h->d_inv, h->inv_host.data(), sizeof(int32_t) * ld, cudaMemcpyHostToDevice));
+    rc = dalloc(h, &h->d_perm, size_t(s.n));
+    if (!rc) rc = dalloc(h, &h->d_inv, ld);
+    if (rc) return rc;
+    CU(cudaMemcpy(h->d_perm, h->perm_host.data(), sizeof(int32_t) * size_t(s.n), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(h->d_inv, h->inv_host.data(), sizeof(int32_t) * ld, cudaMemcpyHostToDevice));
     s.perm = h->d_perm;
     s.inv  = h->d_inv;
   }
-  CREATE_RC(dalloc(&s.st, 18 * ld));
-  CREATE_RC(dalloc(&s.vprev, 3 * ld));
-  CREATE_RC(dalloc(&s.rpm, MRSB_NM * ld));
-  CREATE_RC(dalloc(&s.pid, PID_ROWS * ld));
-  CREATE_RC(dalloc(&s.fext, 3 * ld));
-  CREATE_RC(dalloc(&s.mext, 3 * ld));
-  CREATE_RC(dalloc(&s.imu, 3 * ld));
-  CREATE_RC(dalloc(&s.initz, ld));
-  CREATE_RC(dalloc(&s.cmd, CMD_ROWS * ld));
-  CREATE_RC(dalloc(&s.ff, FF_ROWS * ld));
-  CREATE_RC(dalloc(&s.flags, ld));
-  CREATE_RC(dalloc(&s.mode, ld));
-  CREATE_RC(dalloc(&s.gpos, 3 * size_t(s.n_global)));
-  CREATE_RC(dalloc(&h->d_pset, size_t(s.n_global)));
+  rc = dalloc(h, &s.st, 18 * ld);
+  if (!rc) rc = dalloc(h, &s.vprev, 3 * ld);
+  if (!rc) rc = dalloc(h, &s.rpm, MRSB_NM * ld);
+  if (!rc) rc = dalloc(h, &s.pid, PID_ROWS * ld);
+  if (!rc) rc = dalloc(h, &s.fext, 3 * ld);
+  if (!rc) rc = dalloc(h, &s.mext, 3 * ld);
+  if (!rc) rc = dalloc(h, &s.imu, 3 * ld);
+  if (!rc) rc = dalloc(h, &s.initz, ld);
+  if (!rc) rc = dalloc(h, &s.cmd, CMD_ROWS * ld);
+  if (!rc) rc = dalloc(h, &s.ff, FF_ROWS * ld);
+  if (!rc) rc = dalloc(h, &s.flags, ld);
+  if (!rc) rc = dalloc(h, &s.mode, ld);
+  if (!rc) rc = dalloc(h, &s.gpos, 3 * size_t(s.n_global));
+  if (!rc) rc = dalloc(h, &h->d_pset, size_t(s.n_global));
+  if (rc) return rc;
   s.pset = h->d_pset;
 
   // parameter sets: one per airframe type with default controller gains (US:159-169)
@@ -830,18 +888,17 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
   h->pset_host.resize(size_t(s.n_global));
   for (int64_t j = 0; j < s.n_global; j++) {
     const int t = info->type_of_uav ? info->type_of_uav[j] : 0;
-    if (t < 0 || t >= info->n_types) {
-      mrsb_destroy(h);
-      return fail(MRSB_ERR_INVALID, "type_of_uav[%lld]=%d outside 0..%d", (long long)j, t, info->n_types - 1);
-    }
+    if (t < 0 || t >= info->n_types) return fail(MRSB_ERR_INVALID, "type_of_uav[%lld]=%d outside 0..%d", (long long)j, t, info->n_types - 1);
     h->pset_host[size_t(j)] = set_of_type[t];
   }
-  CREATE_CU(cudaMemcpy(h->d_pset, h->pset_host.data(), sizeof(int32_t) * size_t(s.n_global), cudaMemcpyHostToDevice));
-  CREATE_RC(flush_params(h));
+  CU(cudaMemcpy(h->d_pset, h->pset_host.data(), sizeof(int32_t) * size_t(s.n_global), cudaMemcpyHostToDevice));
+  rc = flush_params(h);
+  if (rc) return rc;
   // collision geometry of the whole swarm (the airframe of every UAV is known everywhere at create time)
-  CREATE_RC(dalloc(&h->d_geom[0], 4 * size_t(s.n_global)));
+  rc = dalloc(h, &h->d_geom[0], 4 * size_t(s.n_global));
+  if (rc) return rc;
   s.geom = h->d_geom[0];
-  h->n_launches += launch_set_geom(h->d_geom[0], s.n_global, nullptr, 0, h->d_pset, h->d_params, h->stream);
+  h->n_launches += launch_set_geom(h->d_geom[0], s.n_global, nullptr, 0, h->d_pset, h->d_params.get(), h->stream);
   s.opts = STEP_OPT_IMU | STEP_OPT_GPOS;
 
   // initial state (MM:183-198 + setStatePos MM:439-446): R = Rz(-heading), flags from the airframe
@@ -850,21 +907,22 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     for (int64_t i = 0; i < s.n; i++)
       fl[h->perm_host.empty() ? size_t(i) : size_t(h->perm_host[size_t(i)])] =
           h->sets[h->pset_host[size_t(s.shard_begin + i)]].mp.takeoff_patch_enabled ? FLAG_TAKEOFF : 0u;
-    CREATE_CU(cudaMemcpy(s.flags, fl.data(), sizeof(uint32_t) * ld, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s.flags, fl.data(), sizeof(uint32_t) * ld, cudaMemcpyHostToDevice));
     const size_t bytes = sizeof(double) * 4 * size_t(std::max<int64_t>(s.n, 1));
-    CREATE_RC(ensure_stage(h, bytes));
+    rc                 = ensure_stage(h, bytes);
+    if (rc) return rc;
     double* d_xyz = nullptr;
     double* d_hdg = nullptr;
     if (info->spawn_xyz && s.n) {
-      d_xyz = reinterpret_cast<double*>(h->d_stage);
-      CREATE_CU(cudaMemcpyAsync(d_xyz, info->spawn_xyz, sizeof(double) * 3 * s.n, cudaMemcpyHostToDevice, h->stream));
+      d_xyz = reinterpret_cast<double*>(h->d_stage.get());
+      CU(cudaMemcpyAsync(d_xyz, info->spawn_xyz, sizeof(double) * 3 * s.n, cudaMemcpyHostToDevice, h->stream));
     }
     if (info->spawn_heading && s.n) {
-      d_hdg = reinterpret_cast<double*>(h->d_stage) + 3 * s.n;
-      CREATE_CU(cudaMemcpyAsync(d_hdg, info->spawn_heading, sizeof(double) * s.n, cudaMemcpyHostToDevice, h->stream));
+      d_hdg = reinterpret_cast<double*>(h->d_stage.get()) + 3 * s.n;
+      CU(cudaMemcpyAsync(d_hdg, info->spawn_heading, sizeof(double) * s.n, cudaMemcpyHostToDevice, h->stream));
     }
     h->n_launches += launch_set_state_pos(s, s.n, nullptr, d_xyz, d_hdg, h->stream);
-    CREATE_CU(cudaStreamSynchronize(h->stream));
+    CU(cudaStreamSynchronize(h->stream));
   }
 
   // collision workspace
@@ -881,47 +939,47 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     while (2 * (size_t(1) << bits) < 3 * expect && bits < 30) bits++;
     g.bits      = bits;
     g.n_buckets = 1u << bits;
-    CREATE_RC(dalloc(&g.bucket, ng));
-    CREATE_RC(dalloc(&g.rank, ng));
-    CREATE_RC(dalloc(&g.count, size_t(g.n_buckets) + 4));  // + mirrors of buckets 0 and 1 + sentinel
-    CREATE_RC(dalloc(&g.begin, size_t(g.n_buckets) + 4));
-    CREATE_RC(dalloc(&g.aabb, 6));
-    CREATE_RC(dalloc(&g.rec, 2 * ng));  // worst case: every UAV in bucket 0 and mirrored
-    g.pair_cap = int64_t(std::max<size_t>(4096, 4 * size_t(std::max<int64_t>(s.n, 1))));
-    CREATE_RC(dalloc(&g.pairs, 2 * size_t(g.pair_cap)));
-    CREATE_RC(dalloc(&g.counters, 4));
+    g.pair_cap   = int64_t(std::max<size_t>(4096, 4 * size_t(std::max<int64_t>(s.n, 1))));
     g.scan_tiles = scan_tiles_for(int64_t(g.n_buckets) + 3);
-    CREATE_RC(dalloc(&g.scan_state, size_t(g.scan_tiles) + size_t(scan_tiles_for(s.n)) + 2));  // table scan + compaction scan
-    // remote UAVs a rebuild fetches from their owners (pull exchange): at most all of them
-    g.halo_cap = std::max<int64_t>(s.n_global - s.n, 1);
-    if (s.n_global > s.n) {
-      CREATE_RC(dalloc(&g.halo_rec, size_t(g.halo_cap)));
-      CREATE_RC(dalloc(&g.halo_bucket, size_t(g.halo_cap)));
-      CREATE_RC(dalloc(&g.halo_rank, size_t(g.halo_cap)));
-    }
-    CREATE_RC(dalloc(&g.halo_n, 2));
+    g.halo_cap   = std::max<int64_t>(s.n_global - s.n, 1);  // remote UAVs a rebuild fetches from their owners (pull exchange): at most all of them
+    rc = dalloc(h, &g.bucket, ng);
+    if (!rc) rc = dalloc(h, &g.rank, ng);
+    if (!rc) rc = dalloc(h, &g.count, size_t(g.n_buckets) + 4);  // + mirrors of buckets 0 and 1 + sentinel
+    if (!rc) rc = dalloc(h, &g.begin, size_t(g.n_buckets) + 4);
+    if (!rc) rc = dalloc(h, &g.aabb, 6);
+    if (!rc) rc = dalloc(h, &g.rec, 2 * ng);  // worst case: every UAV in bucket 0 and mirrored
+    if (!rc) rc = h->pairs.grow(2 * size_t(g.pair_cap), 2 * size_t(g.pair_cap), h->stream);
+    if (!rc) rc = dalloc(h, &g.counters, 4);
+    if (!rc) rc = dalloc(h, &g.scan_state, size_t(g.scan_tiles) + size_t(scan_tiles_for(s.n)) + 2);  // table scan + compaction scan
+    if (!rc && s.n_global > s.n) rc = dalloc(h, &g.halo_rec, size_t(g.halo_cap));
+    if (!rc && s.n_global > s.n) rc = dalloc(h, &g.halo_bucket, size_t(g.halo_cap));
+    if (!rc && s.n_global > s.n) rc = dalloc(h, &g.halo_rank, size_t(g.halo_cap));
+    if (!rc) rc = dalloc(h, &g.halo_n, 2);
+    if (!rc && s.n_global > s.n) rc = dalloc(h, &g.halo_work, size_t(g.halo_cap / 32 + MRSB_MAX_RANKS + 1));
+    if (!rc && getenv("MRSB_TIMELINE")) rc = dalloc(h, &g.tl, size_t(MRSB_TL_TICKS) * 8);
+    if (!rc) rc = dalloc(h, &g.ctl, 1);
+    if (!rc) rc = h->h_one.alloc(2);
+    if (rc) return rc;
+    g.pairs       = h->pairs.get();
     g.halo_work_n = g.halo_n + 1;
-    if (s.n_global > s.n) CREATE_RC(dalloc(&g.halo_work, size_t(g.halo_cap / 32 + MRSB_MAX_RANKS + 1)));
-    if (getenv("MRSB_TIMELINE")) CREATE_RC(dalloc(&g.tl, size_t(MRSB_TL_TICKS) * 8));
-    CREATE_RC(dalloc(&g.ctl, 1));
-    CREATE_CU(cudaHostAlloc(&h->h_one, 2 * sizeof(uint32_t), cudaHostAllocDefault));
-    h->h_one[0] = 1u;
-    h->h_one[1] = 0xFFFFFFFFu;  // "unbounded displacement"
+    h->h_one.get()[0] = 1u;
+    h->h_one.get()[1] = 0xFFFFFFFFu;  // "unbounded displacement"
     // neighbour lists: single-shard handles now, sharded ones once the pull exchange is up (setup_p2p)
     if (s.n > 0 && !getenv("MRSB_NO_NEIGHBOUR_LISTS")) {
       g.nl_ld = s.ld;
-      CREATE_RC(dalloc(&g.nl_count, size_t(g.nl_ld)));
-      CREATE_RC(dalloc(&g.nl_items, size_t(MRSB_NL_CAP) * size_t(g.nl_ld)));
-      CREATE_RC(dalloc(&g.nl_active, size_t(g.nl_ld)));
-      CREATE_RC(dalloc(&g.act_items, size_t(MRSB_NL_CAP) * size_t(g.nl_ld)));
+      rc      = dalloc(h, &g.nl_count, size_t(g.nl_ld));
+      if (!rc) rc = dalloc(h, &g.nl_items, size_t(MRSB_NL_CAP) * size_t(g.nl_ld));
+      if (!rc) rc = dalloc(h, &g.nl_active, size_t(g.nl_ld));
+      if (!rc) rc = dalloc(h, &g.act_items, size_t(MRSB_NL_CAP) * size_t(g.nl_ld));
+      if (rc) return rc;
     }
     set_collision_geometry(h, g.nl_count != nullptr && s.n_global == s.n);
   }
   make_local_view(h);
   h->shard_begin_of = {s.shard_begin};
   h->shard_count_of = {s.n};
-  CREATE_CU(cudaStreamSynchronize(h->stream));
-  *out = h;
+  CU(cudaStreamSynchronize(h->stream));
+  *out = guard.release();
   return MRSB_OK;
 }
 
@@ -933,16 +991,18 @@ int mrsb_sync(mrsb_handle h) {
   return MRSB_OK;
 }
 
+// Streams, events and snapshot buffers of the pipelined host I/O, made on first use.  A call that fails half-way keeps what it
+// made and the next one makes the rest: the pipeline is ready once the last of them, d_snap[1], exists.
 static int ensure_pipeline(mrsb_sim* h) {
-  if (h->up_stream) return MRSB_OK;
-  CU(cudaStreamCreateWithFlags(&h->up_stream, cudaStreamNonBlocking));
-  CU(cudaStreamCreateWithFlags(&h->down_stream, cudaStreamNonBlocking));
+  if (h->d_snap[1].get()) return MRSB_OK;
+  for (cudaStream_t* s : {&h->up_stream, &h->down_stream})
+    if (!*s) CU(cudaStreamCreateWithFlags(s, cudaStreamNonBlocking));
+  const size_t snap = 3 * size_t(std::max<int64_t>(h->ds.n, 1));
   for (int k = 0; k < 2; k++) {
-    CU(cudaEventCreateWithFlags(&h->ev_up[k], cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&h->ev_applied[k], cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&h->ev_snap[k], cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&h->ev_down[k], cudaEventDisableTiming));
-    CU(cudaMalloc(&h->d_snap[k], sizeof(double) * 3 * size_t(std::max<int64_t>(h->ds.n, 1))));
+    for (cudaEvent_t* e : {&h->ev_up[k], &h->ev_applied[k], &h->ev_snap[k], &h->ev_down[k]})
+      if (!*e) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    int rc = h->d_snap[k].grow(snap, snap, h->down_stream);
+    if (rc) return rc;
   }
   return MRSB_OK;
 }
@@ -955,23 +1015,22 @@ int mrsb_set_input_async(mrsb_handle h, int32_t mode, const double* payload, int
   int rc = ensure_pipeline(h);
   if (rc) return rc;
   const int64_t n     = h->ds.n;
-  const size_t  bytes = sizeof(double) * size_t(n) * size_t(stride);
-  if (bytes > h->d_up_bytes) {
-    CU(cudaStreamSynchronize(h->stream));
-    CU(cudaStreamSynchronize(h->up_stream));
-    for (int k = 0; k < 2; k++) {
-      if (h->d_up[k]) CU(cudaFree(h->d_up[k]));
-      CU(cudaMalloc(&h->d_up[k], std::max<size_t>(bytes, 256)));
+  const size_t  count = size_t(n) * size_t(stride);
+  if (count > std::min(h->d_up[0].cap(), h->d_up[1].cap())) {
+    CU(cudaStreamSynchronize(h->stream));     // the scatter reads the staging buffers,
+    CU(cudaStreamSynchronize(h->up_stream));  // the uploads write them
+    for (Mem<double>& b : h->d_up) {
+      rc = b.grow(count, count, h->up_stream);
+      if (rc) return rc;
     }
-    h->d_up_bytes = bytes;
-    h->n_up       = 0;
+    h->n_up = 0;
   }
   const int k = int(h->n_up & 1);
   if (h->n_up >= 2) CU(cudaStreamWaitEvent(h->up_stream, h->ev_applied[k], 0));  // the staging buffer was consumed two uploads ago
-  CU(cudaMemcpyAsync(h->d_up[k], payload, bytes, cudaMemcpyHostToDevice, h->up_stream));
+  CU(cudaMemcpyAsync(h->d_up[k].get(), payload, sizeof(double) * count, cudaMemcpyHostToDevice, h->up_stream));
   CU(cudaEventRecord(h->ev_up[k], h->up_stream));
   CU(cudaStreamWaitEvent(h->stream, h->ev_up[k], 0));
-  h->n_launches += launch_scatter_input(h->ds, mode, n, nullptr, h->d_up[k], stride, h->stream);
+  h->n_launches += launch_scatter_input(h->ds, mode, n, nullptr, h->d_up[k].get(), stride, h->stream);
   CU(cudaEventRecord(h->ev_applied[k], h->stream));
   h->n_up++;
   note_mode(h, mode, n, true);
@@ -985,19 +1044,19 @@ int mrsb_get_positions_async(mrsb_handle h, double* out_xyz) {
   int rc = ensure_pipeline(h);
   if (rc) return rc;
   const int    k     = int(h->n_down & 1);
-  const size_t bytes = sizeof(double) * 3 * size_t(h->d_sub_idx ? h->n_sub : h->ds.n);
+  const size_t bytes = sizeof(double) * 3 * size_t(h->n_sub ? h->n_sub : h->ds.n);
   if (h->n_down >= 2) CU(cudaStreamWaitEvent(h->stream, h->ev_down[k], 0));  // the snapshot buffer was downloaded two reads ago
   if (!(h->ds.opts & STEP_OPT_GPOS)) return fail(MRSB_ERR_STATE, "packed positions are switched off (mrsb_set_outputs)");
   // pull exchange: the buffer being written holds the latest positions only once something wrote it since the last pass
   const double* latest = (h->p2p && !h->wrote_since_pass) ? h->gbuf[h->pass_no & 1] : h->ds.gpos;
-  if (h->d_sub_idx) {
-    h->n_launches += launch_gather_xyz(latest + 3 * h->ds.shard_begin, h->n_sub, h->d_sub_idx, h->d_snap[k], h->stream);
+  if (h->n_sub) {
+    h->n_launches += launch_gather_xyz(latest + 3 * h->ds.shard_begin, h->n_sub, h->d_sub_idx.get(), h->d_snap[k].get(), h->stream);
   } else {
-    CU(cudaMemcpyAsync(h->d_snap[k], latest + 3 * h->ds.shard_begin, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_snap[k].get(), latest + 3 * h->ds.shard_begin, bytes, cudaMemcpyDeviceToDevice, h->stream));
   }
   CU(cudaEventRecord(h->ev_snap[k], h->stream));
   CU(cudaStreamWaitEvent(h->down_stream, h->ev_snap[k], 0));
-  CU(cudaMemcpyAsync(out_xyz, h->d_snap[k], bytes, cudaMemcpyDeviceToHost, h->down_stream));
+  CU(cudaMemcpyAsync(out_xyz, h->d_snap[k].get(), bytes, cudaMemcpyDeviceToHost, h->down_stream));
   CU(cudaEventRecord(h->ev_down[k], h->down_stream));
   h->n_down++;
   return MRSB_OK;
@@ -1007,15 +1066,14 @@ int mrsb_set_position_subset(mrsb_handle h, int64_t n, const int32_t* idx) {
   GUARD(h);
   if (h->down_stream) CU(cudaStreamSynchronize(h->down_stream));
   CU(cudaStreamSynchronize(h->stream));
-  if (h->d_sub_idx) CU(cudaFree(h->d_sub_idx));
-  h->d_sub_idx = nullptr;
-  h->n_sub     = 0;
+  h->n_sub = 0;
   if (!idx || n <= 0) return MRSB_OK;  // back to "all of them"
   for (int64_t k = 0; k < n; k++)
     if (idx[k] < 0 || idx[k] >= h->ds.n) return fail(MRSB_ERR_INVALID, "idx[%lld]=%d outside 0..%lld", (long long)k, idx[k], (long long)h->ds.n - 1);
   if (n > h->ds.n) return fail(MRSB_ERR_INVALID, "a subset of more than n_local UAVs");
-  CU(cudaMalloc(&h->d_sub_idx, sizeof(int32_t) * size_t(n)));
-  CU(cudaMemcpy(h->d_sub_idx, idx, sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice));
+  int rc = h->d_sub_idx.grow(size_t(n), size_t(n), h->stream);
+  if (rc) return rc;
+  CU(cudaMemcpy(h->d_sub_idx.get(), idx, sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice));
   h->n_sub = n;
   return MRSB_OK;
 }
@@ -1073,11 +1131,10 @@ int mrsb_set_input(mrsb_handle h, int32_t mode, int64_t n, const int32_t* idx, c
   if (!payload && n) return fail(MRSB_ERR_INVALID, "null payload");
   if (stride < (mode == MRSB_ACTUATOR_CMD ? 1 : stride_of(mode))) return fail(MRSB_ERR_INVALID, "stride %d too small for mode %d", stride, mode);
   if (n == 0) return MRSB_OK;
-  const size_t bytes = sizeof(double) * size_t(n) * size_t(stride);
-  rc                 = ensure_stage(h, bytes);
+  const double* d_rows = nullptr;
+  rc                   = stage_rows(h, n, {{payload, stride}}, &d_rows);
   if (rc) return rc;
-  CU(cudaMemcpyAsync(h->d_stage, payload, bytes, cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_scatter_input(h->ds, mode, n, d_idx, reinterpret_cast<const double*>(h->d_stage), stride, h->stream);
+  h->n_launches += launch_scatter_input(h->ds, mode, n, d_idx, d_rows, stride, h->stream);
   note_mode(h, mode, n, idx == nullptr);
   CU(cudaGetLastError());
   return MRSB_OK;
@@ -1106,33 +1163,20 @@ int mrsb_clear_input(mrsb_handle h, int64_t n, const int32_t* idx) {
 // host rows -> SoA rows [row0, row0+rows) of `dst`; then OR `flag` into the per-UAV flags
 static int put_rows(mrsb_sim* h, double* dst, int rows_total, int row0, int rows, int64_t n, const int32_t* idx, const double* payload, int stride,
                     uint32_t or_flag) {
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  if (!payload) return fail(MRSB_ERR_INVALID, "null payload");
-  const size_t bytes = sizeof(double) * size_t(n) * size_t(stride);
-  rc                 = ensure_stage(h, bytes);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(h->d_stage, payload, bytes, cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_scatter_rows(dst, rows_total, row0, rows, n, d_idx, reinterpret_cast<const double*>(h->d_stage), stride, h->ds.perm, h->stream);
+  const int32_t* d_idx  = nullptr;
+  const double*  d_rows = nullptr;
+  int            rc     = upload(h, n, idx, {{payload, stride}}, &d_idx, &d_rows);
+  if (rc || n == 0) return rc;
+  h->n_launches += launch_scatter_rows(dst, rows_total, row0, rows, n, d_idx, d_rows, stride, h->ds.perm, h->stream);
   if (or_flag) h->n_launches += launch_flag_update(h->ds, n, d_idx, 0xffffffffu, or_flag, h->stream);
   CU(cudaGetLastError());
   return MRSB_OK;
 }
 
 static int get_rows(mrsb_sim* h, const double* src, int rows_total, int row0, int rows, int64_t n, const int32_t* idx, double* out) {
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  const size_t bytes = sizeof(double) * size_t(n) * size_t(rows);
-  rc                 = ensure_stage(h, bytes);
-  if (rc) return rc;
-  h->n_launches += launch_gather_rows(src, rows_total, row0, rows, n, d_idx, reinterpret_cast<double*>(h->d_stage), rows, h->ds.perm, h->stream);
-  CU(cudaMemcpyAsync(out, h->d_stage, bytes, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  return MRSB_OK;
+  return download(h, n, idx, sizeof(double) * size_t(n) * size_t(rows), out, [&](const int32_t* d_idx, void* d_out) {
+    return launch_gather_rows(src, rows_total, row0, rows, n, d_idx, static_cast<double*>(d_out), rows, h->ds.perm, h->stream);
+  });
 }
 
 int mrsb_set_feedforward_acceleration_hdg_rate(mrsb_handle h, int64_t n, const int32_t* idx, const double* payload) {
@@ -1153,16 +1197,11 @@ int mrsb_set_feedforward_velocity_hdg_rate(mrsb_handle h, int64_t n, const int32
 }
 int mrsb_set_tracker_cmd(mrsb_handle h, int64_t n, const int32_t* idx, const double* rows) {
   GUARD(h);
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);  // validates n and idx before anything is read
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  if (!rows) return fail(MRSB_ERR_INVALID, "null payload");
-  const size_t bytes = sizeof(double) * size_t(n) * MRSB_TRACKER_CMD_STRIDE;
-  rc                 = ensure_stage(h, bytes);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(h->d_stage, rows, bytes, cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_tracker_cmd(h->ds, n, d_idx, reinterpret_cast<const double*>(h->d_stage), h->stream);  // ROSW:995-1021 in one kernel
+  const int32_t* d_idx  = nullptr;
+  const double*  d_rows = nullptr;
+  int            rc     = upload(h, n, idx, {{rows, MRSB_TRACKER_CMD_STRIDE}}, &d_idx, &d_rows);  // validates n and idx before anything is read
+  if (rc || n == 0) return rc;
+  h->n_launches += launch_tracker_cmd(h->ds, n, d_idx, d_rows, h->stream);  // ROSW:995-1021 in one kernel
   CU(cudaGetLastError());
   return MRSB_OK;
 }
@@ -1288,7 +1327,7 @@ static cudaGraphExec_t build_pass_graph(mrsb_sim* h, const PassView& v, bool wit
 static int before_list_pass(mrsb_sim* h) {
   // anything but exactly one stepping launch since the last pass: the displacement bound does not cover it
   if (h->positions_touched || h->steps_since_pass != 1)
-    CU(cudaMemcpyAsync(&h->grid.ctl->force, h->h_one, sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(&h->grid.ctl->force, h->h_one.get(), sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
   h->positions_touched = false;
   h->steps_since_pass  = 0;
   h->list_passes++;
@@ -1395,7 +1434,7 @@ static int before_step(mrsb_sim* h, double dt, int32_t k_substeps) {
   if (rc) return rc;
   rc = ensure_filt(h, dt);
   if (rc) return rc;
-  if (h->p2p && *h->h_status) return fail(MRSB_ERR_STATE, "peer hand-shake timed out (a rank stopped calling the collision pass)");
+  if (h->p2p && *h->h_status.get()) return fail(MRSB_ERR_STATE, "peer hand-shake timed out (a rank stopped calling the collision pass)");
   return MRSB_OK;
 }
 
@@ -1418,7 +1457,7 @@ static int before_collisions(mrsb_sim* h) {
   if (h->lists_on && (h->positions_touched || h->steps_since_pass != 1))
     // anything but exactly one stepping launch since the last pass: this rank's displacement is unbounded —
     // said through the displacement word, so that every peer rebuilds as well
-    CU(cudaMemcpyAsync(&h->grid.ctl->disp_max_bits, h->h_one + 1, sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(&h->grid.ctl->disp_max_bits, h->h_one.get() + 1, sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
   return MRSB_OK;
 }
 
@@ -1513,16 +1552,9 @@ int mrsb_get_state(mrsb_handle h, int64_t n, const int32_t* idx, double* x, doub
 
 int mrsb_get_v_prev(mrsb_handle h, int64_t n, const int32_t* idx, double* v_prev) {
   GUARD(h);
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  rc = ensure_stage(h, sizeof(double) * 3 * size_t(n));
-  if (rc) return rc;
-  h->n_launches += launch_gather_vprev(h->ds, n, d_idx, reinterpret_cast<double*>(h->d_stage), h->stream);
-  CU(cudaMemcpyAsync(v_prev, h->d_stage, sizeof(double) * 3 * size_t(n), cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  return MRSB_OK;
+  return download(h, n, idx, sizeof(double) * 3 * size_t(n), v_prev, [&](const int32_t* d_idx, void* d_out) {
+    return launch_gather_vprev(h->ds, n, d_idx, static_cast<double*>(d_out), h->stream);
+  });
 }
 
 int mrsb_get_imu_acceleration(mrsb_handle h, int64_t n, const int32_t* idx, double* acc) {
@@ -1557,17 +1589,10 @@ int mrsb_set_state(mrsb_handle h, int64_t n, const int32_t* idx, const double* x
 int mrsb_set_state_pos(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading) {
   GUARD(h);
   const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  if (!xyz || !heading) return fail(MRSB_ERR_INVALID, "null payload");
-  rc = ensure_stage(h, sizeof(double) * 4 * size_t(n));
-  if (rc) return rc;
-  double* d_xyz = reinterpret_cast<double*>(h->d_stage);
-  double* d_hdg = d_xyz + 3 * n;
-  CU(cudaMemcpyAsync(d_xyz, xyz, sizeof(double) * 3 * size_t(n), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(d_hdg, heading, sizeof(double) * size_t(n), cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_set_state_pos(h->ds, n, d_idx, d_xyz, d_hdg, h->stream);
+  const double*  d[2]  = {nullptr, nullptr};  // xyz, heading
+  int            rc    = upload(h, n, idx, {{xyz, 3}, {heading, 1}}, &d_idx, d);
+  if (rc || n == 0) return rc;
+  h->n_launches += launch_set_state_pos(h->ds, n, d_idx, d[0], d[1], h->stream);
   if (h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);  // the whole slice of the buffer being written, and its group boxes
   h->wrote_since_pass  = true;
   h->positions_touched = true;
@@ -1586,19 +1611,12 @@ static int respawned(mrsb_sim* h) {
 int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading) {
   GUARD(h);
   const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  if (!xyz || !heading) return fail(MRSB_ERR_INVALID, "null payload");
+  const double*  d[2]  = {nullptr, nullptr};  // xyz, heading
+  int            rc    = upload(h, n, idx, {{xyz, 3}, {heading, 1}}, &d_idx, d);
+  if (rc || n == 0) return rc;
   rc = flush_params(h);  // the kernel reads the take-off flag of every UAV's parameter set
   if (rc) return rc;
-  rc = ensure_stage(h, sizeof(double) * 4 * size_t(n));
-  if (rc) return rc;
-  double* d_xyz = reinterpret_cast<double*>(h->d_stage);
-  double* d_hdg = d_xyz + 3 * n;
-  CU(cudaMemcpyAsync(d_xyz, xyz, sizeof(double) * 3 * size_t(n), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(d_hdg, heading, sizeof(double) * size_t(n), cudaMemcpyHostToDevice, h->stream));
-  h->n_launches += launch_respawn(h->ds, h->d_takeoff0, n, d_idx, d_xyz, d_hdg, h->stream);
+  h->n_launches += launch_respawn(h->ds, h->d_takeoff0.get(), n, d_idx, d[0], d[1], h->stream);
   h->positions_touched = true;
   note_mode(h, MRSB_INPUT_UNKNOWN, n, idx == nullptr);
   return respawned(h);
@@ -1611,37 +1629,22 @@ int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const dou
   if (rc) return rc;
   // the host does not learn who was respawned: the kernel raises the displacement word itself (no forced rebuild from here), and
   // the batch can no longer be assumed to share one input mode unless it is already INPUT_UNKNOWN
-  h->n_launches += launch_respawn_masked(h->ds, h->d_takeoff0, mask_dev, xyz_dev, heading_dev, h->stream);
+  h->n_launches += launch_respawn_masked(h->ds, h->d_takeoff0.get(), mask_dev, xyz_dev, heading_dev, h->stream);
   note_mode(h, MRSB_INPUT_UNKNOWN, 1, false);
   return respawned(h);
 }
 
 int mrsb_get_input_mode(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* mode) {
   GUARD(h);
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  rc = ensure_stage(h, sizeof(int32_t) * size_t(n));
-  if (rc) return rc;
-  h->n_launches += launch_gather_u8(h->ds.mode, n, d_idx, reinterpret_cast<int32_t*>(h->d_stage), h->ds.perm, h->stream);
-  CU(cudaMemcpyAsync(mode, h->d_stage, sizeof(int32_t) * size_t(n), cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  return MRSB_OK;
+  return download(h, n, idx, sizeof(int32_t) * size_t(n), mode, [&](const int32_t* d_idx, void* d_out) {
+    return launch_gather_u8(h->ds.mode, n, d_idx, static_cast<int32_t*>(d_out), h->ds.perm, h->stream);
+  });
 }
 
-static int get_flags(mrsb_sim* h, int64_t n, const int32_t* idx, std::vector<uint32_t>& out) {
-  const int32_t* d_idx = nullptr;
-  int            rc    = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  out.resize(size_t(n));
-  if (n == 0) return MRSB_OK;
-  rc = ensure_stage(h, sizeof(uint32_t) * size_t(n));
-  if (rc) return rc;
-  h->n_launches += launch_gather_u32(h->ds.flags, n, d_idx, reinterpret_cast<uint32_t*>(h->d_stage), h->ds.perm, h->stream);
-  CU(cudaMemcpyAsync(out.data(), h->d_stage, sizeof(uint32_t) * size_t(n), cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  return MRSB_OK;
+static int get_flags(mrsb_sim* h, int64_t n, const int32_t* idx, uint32_t* out) {
+  return download(h, n, idx, sizeof(uint32_t) * size_t(n), out, [&](const int32_t* d_idx, void* d_out) {
+    return launch_gather_u32(h->ds.flags, n, d_idx, static_cast<uint32_t*>(d_out), h->ds.perm, h->stream);
+  });
 }
 
 int mrsb_crash(mrsb_handle h, int64_t n, const int32_t* idx) {
@@ -1655,10 +1658,9 @@ int mrsb_crash(mrsb_handle h, int64_t n, const int32_t* idx) {
 
 int mrsb_has_crashed(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* crashed) {
   GUARD(h);
-  std::vector<uint32_t> fl;
-  int                   rc = get_flags(h, n, idx, fl);
+  int rc = get_flags(h, n, idx, reinterpret_cast<uint32_t*>(crashed));  // the flags, then in place what they say
   if (rc) return rc;
-  for (int64_t k = 0; k < n; k++) crashed[k] = (fl[size_t(k)] & FLAG_CRASHED) ? 1 : 0;
+  for (int64_t k = 0; k < n; k++) crashed[k] = (uint32_t(crashed[k]) & FLAG_CRASHED) ? 1 : 0;
   return MRSB_OK;
 }
 
@@ -1707,11 +1709,11 @@ int mrsb_get_params(mrsb_handle h, int64_t uav, mrsb_model_params* out) {
   int rc = check_uav(h, uav);
   if (rc) return rc;
   *out = h->sets[h->pset_host[size_t(h->ds.shard_begin + uav)]].mp;
-  std::vector<uint32_t> fl;
-  const int32_t         one = int32_t(uav);
-  rc                        = get_flags(h, 1, &one, fl);
+  uint32_t      fl  = 0;
+  const int32_t one = int32_t(uav);
+  rc                = get_flags(h, 1, &one, &fl);
   if (rc) return rc;
-  out->takeoff_patch_enabled = (fl[0] & FLAG_TAKEOFF) ? 1 : 0;
+  out->takeoff_patch_enabled = (fl & FLAG_TAKEOFF) ? 1 : 0;
   return MRSB_OK;
 }
 
@@ -1816,17 +1818,9 @@ static int observe(mrsb_sim* h, int what, int width, int64_t n, const int32_t* i
   if ((what == 1 || what == 3) && !(h->ds.opts & STEP_OPT_IMU)) return fail(MRSB_ERR_STATE, "the IMU rows are switched off (mrsb_set_outputs)");
   int rc = flush_params(h);
   if (rc) return rc;
-  const int32_t* d_idx = nullptr;
-  rc                   = stage_idx(h, n, idx, &d_idx);
-  if (rc) return rc;
-  if (n == 0) return MRSB_OK;
-  const size_t bytes = sizeof(double) * size_t(n) * size_t(width);
-  rc                 = ensure_stage(h, bytes);
-  if (rc) return rc;
-  h->n_launches += launch_observe(h->ds, what, n, d_idx, reinterpret_cast<double*>(h->d_stage), width, h->stream);
-  CU(cudaMemcpyAsync(out, h->d_stage, bytes, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  return MRSB_OK;
+  return download(h, n, idx, sizeof(double) * size_t(n) * size_t(width), out, [&](const int32_t* d_idx, void* d_out) {
+    return launch_observe(h->ds, what, n, d_idx, static_cast<double*>(d_out), width, h->stream);
+  });
 }
 int mrsb_get_odometry(mrsb_handle h, int64_t n, const int32_t* idx, double* out13) {
   GUARD(h);
@@ -1965,10 +1959,9 @@ int mrsb_set_pair_capacity(mrsb_handle h, int64_t max_pairs) {
   GUARD(h);
   if (max_pairs < 1) return fail(MRSB_ERR_INVALID, "max_pairs must be >= 1");
   CU(cudaStreamSynchronize(h->stream));
-  int32_t* fresh = nullptr;
-  CU(cudaMalloc(&fresh, sizeof(int32_t) * 2 * size_t(max_pairs)));
-  if (h->grid.pairs) CU(cudaFree(h->grid.pairs));
-  h->grid.pairs    = fresh;
+  int rc = h->pairs.grow(2 * size_t(max_pairs), 2 * size_t(max_pairs), h->stream);
+  if (rc) return rc;
+  h->grid.pairs    = h->pairs.get();
   h->grid.pair_cap = max_pairs;
   drop_collision_graphs(h);
   CU(cudaMemsetAsync(h->grid.counters, 0, sizeof(unsigned long long), h->stream));
@@ -1979,8 +1972,8 @@ int mrsb_get_counters(mrsb_handle h, int64_t* out5) {
   GUARD(h);
   unsigned long long found = 0;
   CU(cudaMemcpyAsync(&found, h->grid.counters, sizeof(found), cudaMemcpyDeviceToHost, h->stream));
-  std::vector<uint32_t> fl;
-  int                   rc = get_flags(h, h->ds.n, nullptr, fl);
+  std::vector<uint32_t> fl(size_t(h->ds.n));
+  int                   rc = get_flags(h, h->ds.n, nullptr, fl.data());
   if (rc) return rc;
   int64_t crashed = 0;
   for (uint32_t f : fl) crashed += (f & FLAG_CRASHED) ? 1 : 0;
@@ -2065,15 +2058,15 @@ int mrsb_comm_init_nccl(mrsb_handle h, int32_t n_ranks, int32_t rank, const void
   h->n_ranks = n_ranks;
   h->rank    = rank;
   // learn every rank's shard with one tiny all-gather
-  int64_t* d_tab = nullptr;
-  CU(cudaMalloc(&d_tab, sizeof(int64_t) * 2 * n_ranks));
+  Mem<int64_t> d_tab;
+  rc = d_tab.alloc(2 * size_t(n_ranks));
+  if (rc) return rc;
   const int64_t mine[2] = {h->ds.shard_begin, h->ds.n};
-  CU(cudaMemcpyAsync(d_tab + 2 * rank, mine, sizeof(mine), cudaMemcpyHostToDevice, h->stream));
-  NC(g_nccl.AllGather(d_tab + 2 * rank, d_tab, 2, ncclInt64, h->comm, h->stream));
+  CU(cudaMemcpyAsync(d_tab.get() + 2 * rank, mine, sizeof(mine), cudaMemcpyHostToDevice, h->stream));
+  NC(g_nccl.AllGather(d_tab.get() + 2 * rank, d_tab.get(), 2, ncclInt64, h->comm, h->stream));
   std::vector<int64_t> tab(2 * size_t(n_ranks));
-  CU(cudaMemcpyAsync(tab.data(), d_tab, sizeof(int64_t) * tab.size(), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(tab.data(), d_tab.get(), sizeof(int64_t) * tab.size(), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  CU(cudaFree(d_tab));
   h->shard_begin_of.assign(size_t(n_ranks), 0);
   h->shard_count_of.assign(size_t(n_ranks), 0);
   h->equal_shards = true;
