@@ -325,6 +325,31 @@ int mrsb_pack_observations_device(mrsb_handle h, double* out_dev, int32_t stride
 int mrsb_set_mass(mrsb_handle h, int64_t n, const int32_t* idx, const double* mass);
 int mrsb_set_ground_z(mrsb_handle h, int64_t n, const int32_t* idx, const double* ground_z);
 
+/* ---- neighbour observations (multi-agent RL) -------------------------------------------------
+ * For every local UAV i, the UAVs j != i of this handle with d2 < radius*radius, where
+ *   d2 = ((dx*dx) + dy*dy) + dz*dz,  dx = x_j - x_i (likewise y, z), in FP64 without contraction (the collision predicate's
+ *   metric); radius*radius is rounded once, on the host, and the comparison is strict.
+ * The set is sorted by (d2, j) ascending (ties go to the lower index) and its first min(count, k) are reported.  Crashed UAVs are
+ * included (they are still bodies in the world).  A UAV with a non-finite position (NaN or Inf in any coordinate) has no
+ * neighbours and is nobody's neighbour.
+ * Outputs, all DEVICE arrays, any of them NULL but not all three:
+ *   idx_dev[n_local][k]   neighbour indices (local = global on a single shard), -1 past the last neighbour;
+ *   rows_dev              row i starts at i*stride (stride >= 6*k); block m of it = [x_j - x_i (3) | v_j - v_i (3)] in the world
+ *                         frame, zero past the last neighbour; doubles past 6*k are not written (a caller can keep its own
+ *                         observation columns beside them);
+ *   count_dev[n_local]    how many UAVs are within the radius (not capped by k).
+ * Positions and velocities are read from the state (mrsb_get_device_view's state rows 0-5), so the result is current right after
+ * mrsb_set_state*, mrsb_respawn*, or a write through the device view, without mrsb_publish_positions, and also with
+ * mrsb_set_outputs(h, 0) and collisions off.  Enqueued on the handle's stream; never synchronises the host.  Its workspace grows
+ * on the first call for a batch size and is reused after that.  The collision pass' state (table, neighbour lists, pair list,
+ * forces, counters [0-3]) is not touched; counter [4] counts the five kernels of a call.
+ * Exact over the coordinate range |x|, |y|, |z| <= 2^30 * radius (beyond it the grid's cell arithmetic may leave out a true
+ * neighbour; the table's reach exceeds the radius by a relative 2^-20 to absorb the rounding inside that range).
+ * MRSB_ERR_INVALID: radius not finite or <= 0, k outside [1, MRSB_MAX_NEIGHBOURS], rows_dev with stride < 6*k, all outputs NULL.
+ * MRSB_ERR_STATE: a sharded handle (n_global > n_local). */
+#define MRSB_MAX_NEIGHBOURS 16
+int mrsb_pack_neighbours_device(mrsb_handle h, double radius, int32_t k, int32_t* idx_dev, double* rows_dev, int32_t stride, int32_t* count_dev);
+
 /* ---- collisions: MultirotorSimulator::handleCollisions (SIM:295-359) -----------------------
  * knobs = collisions/enabled, collisions/crash, collisions/rebounce (SIM:124-126,
  * cfg/multirotor_simulator.cfg:12-20).  The pass runs on the CURRENT positions: uniform-grid

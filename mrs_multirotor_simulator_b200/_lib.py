@@ -117,6 +117,7 @@ SIGNATURES = {
     "mrsb_pack_observations_device": (C.c_int, [H, C.c_void_p, C.c_int32]),
     "mrsb_set_mass": (C.c_int, _N_IDX + [C.c_void_p]),
     "mrsb_set_ground_z": (C.c_int, _N_IDX + [C.c_void_p]),
+    "mrsb_pack_neighbours_device": (C.c_int, [H, C.c_double, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "mrsb_set_collisions": (C.c_int, [H, C.c_int32, C.c_int32, C.c_double]),
     "mrsb_handle_collisions": (C.c_int, [H]),
     "mrsb_get_collision_pairs": (C.c_int, [H, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),

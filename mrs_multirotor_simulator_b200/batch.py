@@ -318,6 +318,13 @@ class UavBatch:
         """odometry 13 | IMU acceleration 3 | range 1 for every UAV into a device buffer (no host round trip)."""
         check(self._L.mrsb_pack_observations_device(self.h, out_ptr, stride))
 
+    def pack_neighbours_device(self, radius, k, idx_ptr=None, rows_ptr=None, count_ptr=None, stride=None):
+        """The k nearest UAVs within `radius` of every UAV, by (d2, index), into device buffers (raw addresses, e.g. torch tensor
+        .data_ptr(); any may be None, not all): indices int32 [n][k] (-1 past the last), rows float64 [n][stride >= 6k] of
+        [x_j - x_i | v_j - v_i] per neighbour (zero past the last), counts int32 [n] (not capped by k).  No host round trip."""
+        check(self._L.mrsb_pack_neighbours_device(self.h, float(radius), int(k), idx_ptr, rows_ptr, 6 * int(k) if stride is None else int(stride),
+                                                  count_ptr))
+
     def set_mass(self, mass, idx=None):
         idx = _idx(idx)
         m = np.ascontiguousarray(np.broadcast_to(mass, (self._n(idx),)), dtype=np.float64)

@@ -242,6 +242,14 @@ struct mrsb_sim {
   uint32_t tick_opts = 0;
   bool     tick_failed = false;
 
+  // neighbour observations (mrsb_pack_neighbours_device): a table of its own, sized for n_local on the first call
+  struct NbWorkspace {
+    Mem<double>             pos, vel;  // [n_local][3] packed from the state rows, external order
+    Mem<uint32_t>           bucket, rank, count, begin;
+    Mem<double4>            rec;
+    Mem<unsigned long long> scan;
+  } nb;
+
   int64_t n_steps = 0, n_passes = 0, n_launches = 0;
   int     step_info[4] = {0, 0, 0, 0};  // last stepping launch: variant, grid, NM_T, MODE_T (mrsb_get_step_info)
 };
@@ -1841,6 +1849,50 @@ int mrsb_pack_observations_device(mrsb_handle h, double* out_dev, int32_t stride
   int rc = flush_params(h);
   if (rc) return rc;
   h->n_launches += launch_observe(h->ds, 3, h->ds.n, nullptr, out_dev, stride, h->stream);
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
+// The neighbour table's workspace for this handle's n_local UAVs: >= 1.5 buckets per UAV, as the collision table.
+static int grow_neighbour_table(mrsb_sim* h, DevGrid* t) {
+  const size_t n    = size_t(h->ds.n);
+  uint32_t     bits = 10;
+  while (2 * (size_t(1) << bits) < 3 * n && bits < 30) bits++;
+  t->n_buckets        = 1u << bits;
+  t->scan_tiles       = scan_tiles_for(int64_t(t->n_buckets) + 3);
+  auto&        w      = h->nb;
+  const size_t nbk    = size_t(t->n_buckets) + 4;  // + mirrors of buckets 0 and 1 + sentinel
+  int          rc     = w.pos.grow(3 * n, 3 * n, h->stream);
+  if (!rc) rc = w.vel.grow(3 * n, 3 * n, h->stream);
+  if (!rc) rc = w.bucket.grow(n, n, h->stream);
+  if (!rc) rc = w.rank.grow(n, n, h->stream);
+  if (!rc) rc = w.count.grow(nbk, nbk, h->stream);
+  if (!rc) rc = w.begin.grow(nbk, nbk, h->stream);
+  if (!rc) rc = w.rec.grow(2 * n, 2 * n, h->stream);  // worst case: every UAV in bucket 0 and mirrored
+  if (!rc) rc = w.scan.grow(size_t(t->scan_tiles) + 1, size_t(t->scan_tiles) + 1, h->stream);
+  if (rc) return rc;
+  t->bucket = w.bucket.get(), t->rank = w.rank.get(), t->count = w.count.get(), t->begin = w.begin.get();
+  t->rec = w.rec.get(), t->scan_state = w.scan.get();
+  return MRSB_OK;
+}
+
+int mrsb_pack_neighbours_device(mrsb_handle h, double radius, int32_t k, int32_t* idx_dev, double* rows_dev, int32_t stride, int32_t* count_dev) {
+  GUARD(h);
+  if (!idx_dev && !rows_dev && !count_dev) return fail(MRSB_ERR_INVALID, "all outputs are NULL");
+  if (!std::isfinite(radius) || !(radius > 0.0)) return fail(MRSB_ERR_INVALID, "radius=%g is not a finite positive number", radius);
+  if (k < 1 || k > MRSB_MAX_NEIGHBOURS) return fail(MRSB_ERR_INVALID, "k=%d outside 1..%d", k, MRSB_MAX_NEIGHBOURS);
+  if (rows_dev && stride < 6 * k) return fail(MRSB_ERR_INVALID, "stride=%d below 6*k=%d", stride, 6 * k);
+  if (h->ds.n_global > h->ds.n) return fail(MRSB_ERR_STATE, "neighbour observations of a sharded handle (n_global > n_local) are not supported");
+  if (h->ds.n <= 0) return MRSB_OK;
+  DevGrid t{};
+  int     rc = grow_neighbour_table(h, &t);
+  if (rc) return rc;
+  // The stencil covers [q - reach, q + reach) per axis.  A neighbour differs from q by less than radius * (1 + 2^-51) per axis
+  // (rounding of d2 and of radius * radius), and the rounding of q - reach and of v * inv_cell moves a cell boundary by at most
+  // 3 * 2^-53 * |v| in length: a relative margin of 2^-20 covers both for |coordinates| <= 2^30 * radius.
+  t.reach    = radius * (1.0 + 0x1p-20);
+  t.inv_cell = 1.0 / (2.0 * t.reach);  // the collision pass' layout: 2 x 2 stencil rows of 2 cells
+  h->n_launches += launch_neighbours(h->ds, t, h->nb.pos.get(), h->nb.vel.get(), radius * radius, k, idx_dev, rows_dev, stride, count_dev, h->stream);
   CU(cudaGetLastError());
   return MRSB_OK;
 }

@@ -964,6 +964,96 @@ __global__ void __launch_bounds__(32) decide_kernel(NlCtl* __restrict__ c, unsig
   c->n_passes = n_passes + 1ull;
 }
 
+// ---- neighbour observations (mrsb_pack_neighbours_device) -----------------------------------------------
+// The k nearest UAVs within a caller-chosen radius, for every UAV of a single-shard handle.  The table is the collision pass'
+// (count_kernel, scan_kernel<false>, scatter_kernel) over a workspace of its own — `t` is a DevGrid that holds only the table
+// fields — so nothing the collision pass keeps is read or written.  Positions and velocities come from the state rows, not from
+// the packed positions, which may be stale or switched off.
+
+// One thread per slot, in tile order (the state loads coalesce); padding slots are skipped.  Writes the positions and velocities in
+// external order: the table is built on the former, the query reads the winners' rows from both.
+__global__ void __launch_bounds__(256) nb_pack_kernel(DevState s, double* __restrict__ pos, double* __restrict__ vel) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= s.ld) return;
+  const int64_t e = s.inv ? int64_t(s.inv[i]) : (i < s.n ? i : -1);
+  if (e < 0) return;
+#pragma unroll
+  for (int c = 0; c < 3; c++) {
+    pos[3 * e + c] = s.st[tix(ST_ROWS, c, i)];
+    vel[3 * e + c] = s.st[tix(ST_ROWS, 3 + c, i)];
+  }
+}
+
+// (d2, j) ordering of the neighbour set: ties go to the lower index
+DEV bool nb_before(double da, int32_t ja, double db, int32_t jb) { return da < db || (da == db && ja < jb); }
+
+// One thread per record, as collide_kernel (neighbouring threads walk the same cells), for UAV i of the record: every candidate of
+// its stencil (the collision pass' layout: 2 x 2 rows of 2 cells of edge 2 * reach) gets the exact predicate d2 < r2 (nf_dist2 with
+// dx = x_j - x_i), j != i, and the row check that rejects bucket aliases; the K best by (d2, j) stay in registers (K >= k, sorted,
+// unrolled insert).  Positions and velocities of the k winners are fetched after the walk, so a candidate costs one record.
+template <int K>
+__global__ void __launch_bounds__(128) nb_query_kernel(DevGrid t, int64_t n, const double* __restrict__ pos, const double* __restrict__ vel, double r2,
+                                                        int k, int32_t* __restrict__ idx_out, double* __restrict__ rows_out, int64_t stride,
+                                                        int32_t* __restrict__ count_out) {
+  const int64_t p = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (p >= n) return;
+  const double4 q = t.rec[p];  // every UAV is inserted: records [0, n) are the primary ones
+  const int64_t i = __double_as_longlong(q.w);
+  double        bd[K];
+  int32_t       bj[K];
+#pragma unroll
+  for (int u = 0; u < K; u++) bd[u] = __longlong_as_double(0x7FF0000000000000ll), bj[u] = INT32_MAX;
+  int32_t cnt = 0;
+  // a UAV with a non-finite position has no neighbours (and is nobody's: its d2 is never < r2)
+  if (isfinite(q.x) && isfinite(q.y) && isfinite(q.z)) {
+    const Stencil st = stencil_of(t, q.x, q.y, q.z);
+    for (int a = 0; a < 4; a++) {
+      for (uint32_t r = st.lo[a]; r < st.hi[a]; r++) {
+        const double4 c  = t.rec[r];
+        const double  d2 = nf_dist2(c.x, c.y, c.z, q.x, q.y, q.z);
+        if (!(d2 < r2)) continue;
+        const int32_t j = int32_t(__double_as_longlong(c.w));
+        if (int64_t(j) == i || cell_of(c.y, t.inv_cell) != st.rcy[a] || cell_of(c.z, t.inv_cell) != st.rcz[a]) continue;  // self, alias
+        cnt++;
+        if (!nb_before(d2, j, bd[K - 1], bj[K - 1])) continue;
+        bd[K - 1] = d2, bj[K - 1] = j;
+#pragma unroll
+        for (int u = K - 1; u > 0; u--) {
+          if (nb_before(bd[u], bj[u], bd[u - 1], bj[u - 1])) {
+            const double  td = bd[u];
+            const int32_t tj = bj[u];
+            bd[u] = bd[u - 1], bj[u] = bj[u - 1];
+            bd[u - 1] = td, bj[u - 1] = tj;
+          }
+        }
+      }
+    }
+  }
+  const int m = min(cnt, k);
+  if (count_out) count_out[i] = cnt;
+  if (idx_out) {
+#pragma unroll
+    for (int u = 0; u < K; u++)
+      if (u < k) idx_out[i * k + u] = u < m ? bj[u] : -1;
+  }
+  if (rows_out) {
+    double*      o  = rows_out + i * stride;
+    const double vx = m > 0 ? vel[3 * i] : 0.0, vy = m > 0 ? vel[3 * i + 1] : 0.0, vz = m > 0 ? vel[3 * i + 2] : 0.0;
+#pragma unroll
+    for (int u = 0; u < K; u++) {
+      if (u >= k) break;
+      double b[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+      if (u < m) {
+        const int64_t j = bj[u];
+        b[0] = __dsub_rn(pos[3 * j], q.x), b[1] = __dsub_rn(pos[3 * j + 1], q.y), b[2] = __dsub_rn(pos[3 * j + 2], q.z);
+        b[3] = __dsub_rn(vel[3 * j], vx), b[4] = __dsub_rn(vel[3 * j + 1], vy), b[5] = __dsub_rn(vel[3 * j + 2], vz);
+      }
+#pragma unroll
+      for (int c = 0; c < 6; c++) o[6 * u + c] = b[c];
+    }
+  }
+}
+
 }  // namespace
 
 int scan_tiles_for(int64_t n_items) {
@@ -1066,4 +1156,26 @@ int launch_collide_check(const DevState& s, const DevGrid& g, const PeerView& pv
   check_kernel<<<unsigned(std::min<int64_t>((s.n + MRSB_CHECK_THREADS - 1) / MRSB_CHECK_THREADS, 148 * MRSB_CHECK_MINB)), MRSB_CHECK_THREADS, 0, stream>>>(s, g, crash_mode, rebounce,
                                                                                                                                                        beside_rebuild);
   return own + 1;
+}
+
+// Neighbour observations: pack, table (count, scan, scatter), query.  `t` holds the workspace's table fields; pos / vel the
+// workspace's packed rows.  Enqueued on `stream`, no host synchronisation.
+int launch_neighbours(const DevState& s, const DevGrid& t, double* pos, double* vel, double r2, int k, int32_t* idx, double* rows, int stride,
+                      int32_t* count, cudaStream_t stream) {
+  const int64_t n = s.n;
+  if (n <= 0) return 0;
+  const int      T      = 256;
+  const unsigned nb     = unsigned((n + T - 1) / T);
+  const int64_t  n_scan = int64_t(t.n_buckets) + 3;
+  cudaMemsetAsync(t.count, 0, sizeof(uint32_t) * size_t(n_scan), stream);
+  cudaMemsetAsync(t.scan_state, 0, sizeof(unsigned long long) * size_t(1 + t.scan_tiles), stream);
+  nb_pack_kernel<<<unsigned((s.ld + T - 1) / T), T, 0, stream>>>(s, pos, vel);
+  count_kernel<<<nb, T, 0, stream>>>(pos, 0, n, 0, n, 0, nullptr, t.n_buckets - 1, t.inv_cell, t.reach, t.count, t.bucket, t.rank);
+  scan_kernel<false><<<unsigned(t.scan_tiles), 256, 0, stream>>>(t.count, t.begin, n_scan, t.scan_state);
+  scatter_kernel<<<nb, T, 0, stream>>>(pos, 0, n, t.bucket, t.rank, t.begin, t.n_buckets, t.rec);
+  const unsigned nq = unsigned((n + 127) / 128);
+  if (k <= 4) nb_query_kernel<4><<<nq, 128, 0, stream>>>(t, n, pos, vel, r2, k, idx, rows, stride, count);
+  else if (k <= 8) nb_query_kernel<8><<<nq, 128, 0, stream>>>(t, n, pos, vel, r2, k, idx, rows, stride, count);
+  else nb_query_kernel<MRSB_MAX_NEIGHBOURS><<<nq, 128, 0, stream>>>(t, n, pos, vel, r2, k, idx, rows, stride, count);
+  return 5;
 }

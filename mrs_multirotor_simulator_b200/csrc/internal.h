@@ -205,6 +205,11 @@ int launch_collide_decide(const DevGrid& g, const P2PCtl& p2p, int always, cudaG
 int launch_collide_rebuild(const DevState& s, const DevGrid& g, const PeerView& pv, cudaStream_t stream);
 int launch_collide_check(const DevState& s, const DevGrid& g, const PeerView& pv, int crash_mode, double rebounce, int beside_rebuild, cudaStream_t stream);
 int scan_tiles_for(int64_t n_items);
+// Neighbour observations (mrsb_pack_neighbours_device) of a single-shard handle: the table over the workspace `t` (only its table
+// fields are read: n_buckets, inv_cell, reach, bucket, rank, count, begin, rec, scan_state, scan_tiles), pos / vel its packed rows
+// [n][3]; r2 = radius * radius; outputs as in include/mrsb.h (any may be nullptr)
+int launch_neighbours(const DevState& s, const DevGrid& t, double* pos, double* vel, double r2, int k, int32_t* idx, double* rows, int stride,
+                      int32_t* count, cudaStream_t stream);
 int launch_publish_positions(const DevState& s, cudaStream_t stream);
 
 int launch_scatter_input(const DevState& s, int mode, int64_t n, const int32_t* idx_dev, const double* payload_dev, int stride, cudaStream_t stream);
