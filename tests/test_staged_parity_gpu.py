@@ -128,8 +128,83 @@ def test_position_cmd_staged_10s():
     assert_parity(orc, gpu, what="PositionCmd staged")
 
 
-def _run_variant(staging, frame, mode, k, n, launches):
-    """One flight on the GPU with or without the staged kernel; returns (full state, crash flags, variant that ran)."""
+FF_KIND = {"acceleration_hdg_rate": 0, "acceleration_hdg": 1, "velocity_hdg": 2, "velocity_hdg_rate": 3}  # the oracle's numbering
+DT_PHASES = (0.01, 0.005, 0.02)  # the edited flights change dt twice: DevParams::filt of the set passed by value must follow
+
+
+def edited_airframe(frame):
+    """The airframe with every constant the kernel derives something from changed: mass, kf, km, tau, drag, ground_z, and a
+    symmetric positive-definite J with off-diagonal terms (the j_diagonal == 0 branch of derivative(), step_kernel.cuh)."""
+    d = af(frame, ground_enabled=True, ground_z=-0.25, takeoff_patch_enabled=True)
+    d.update(mass=1.13 * d["mass"], kf=1.07 * d["kf"], km=0.9 * d["km"], motor_time_constant=0.04, air_resistance_coeff=0.35)
+    m, a, bh = d["mass"], d["arm_length"], d["body_height"]
+    jxy, jz = m * (3.0 * a * a + bh * bh) / 12.0, m * a * a / 2.0
+    J = np.array([[jxy, 0.12 * jxy, -0.08 * jxy], [0.12 * jxy, 1.1 * jxy, 0.1 * jxy], [-0.08 * jxy, 0.1 * jxy, jz]])
+    assert np.all(np.linalg.eigvalsh(J) > 0)
+    d["J"] = J.tolist()
+    return d
+
+
+def apply_edits(s, gidx, frame, edits):
+    """Batch-wide edits of the "edited" flights on a system that holds the UAVs `gidx` of the batch (all of them, or the oracle's
+    sample): set_params with edited_airframe, then all five gain sets with every ki != 0 (rate included: the three rate-integral rows
+    become live), an external moment on a third of the UAVs and the four feed-forwards on overlapping subsets (UAVs with both
+    acceleration feed-forwards take each branch of use_a / use_ar, step_kernel.cuh).  edits == "no_desaturation": the mixer's
+    desaturation off as well."""
+    gpu = not isinstance(s, O.OracleSwarm)
+    sel = lambda mask: np.flatnonzero(mask).astype(np.int32)
+    u = lambda stream, idx, lo, hi: lo + (hi - lo) * O.u01(31, stream, gidx[idx])
+    s.set_params(edited_airframe(frame))
+    s.set_controller_params("rate", [4.2, 0.045, 0.6])
+    s.set_controller_params("attitude", [6.5, 0.06, 0.05, 9.0, 1.2])
+    s.set_controller_params("velocity", [2.2, 0.06, 0.05, 4.5])
+    s.set_controller_params("position", [1.8, 0.12, 0.25, 5.0])
+    if edits == "no_desaturation":
+        s.set_controller_params("mixer", [0.0])
+    m = sel(gidx % 3 == 2)
+    s.set_external_moment(np.stack([u(0, m, -0.02, 0.02), u(1, m, -0.02, 0.02), u(2, m, -0.01, 0.01)], axis=1), idx=m)
+    for stream, (kind, mask) in enumerate([("acceleration_hdg", gidx % 4 < 2), ("acceleration_hdg_rate", (gidx % 4 == 1) | (gidx % 4 == 2)),
+                                           ("velocity_hdg", gidx % 5 < 2), ("velocity_hdg_rate", (gidx % 5 == 1) | (gidx % 5 == 2))]):
+        i = sel(mask)
+        ff = np.stack([u(10 + 4 * stream + c, i, -0.3, 0.3) for c in range(4)], axis=1)
+        s.set_feedforward(kind if gpu else FF_KIND[kind], ff, idx=i)
+
+
+def setup_flight(s, gidx, n, frame, mode, edits):
+    """The flight's set-up on a system that holds the UAVs `gidx` of an n-UAV batch: every UAV on the ground with the take-off patch
+    flag; a third given a state whose v_prev differs from v (FLAG_VPREV) and a tilted, spinning start in the air; the command of
+    `mode`; a few crashed UAVs; an external force on everybody; then the edits, if any."""
+    sel = lambda mask: np.flatnonzero(mask).astype(np.int32)
+    idx = sel(gidx % 3 == 0)
+    k3 = gidx[idx] // 3  # position in arange(0, n, 3)
+    u = lambda stream, lo, hi: lo + (hi - lo) * O.u01(5, stream, k3)
+    st = s.get_state(idx)
+    x = st["x"] + np.stack([np.zeros(len(idx)), np.zeros(len(idx)), u(1, 0.5, 6.0)], axis=1)
+    v = np.stack([u(2, -2, 2), u(3, -2, 2), u(4, -1, 1)], axis=1)
+    w = np.stack([u(5, -0.5, 0.5), u(6, -0.5, 0.5), u(7, -0.5, 0.5)], axis=1)
+    s.set_state(idx, x=x, v=v, omega=w)
+    s.set_input(mode, commands(mode, n)[gidx])
+    s.crash(sel(gidx % 997 == 5))  # 5, 1002, 1999, ...
+    s.apply_force(np.stack([rand(5, 8, n, -1, 1), rand(5, 9, n, -1, 1), rand(5, 10, n, -1, 1)], axis=1)[gidx])
+    if edits:
+        apply_edits(s, gidx, frame, edits)
+
+
+def flight_phases(launches, edits):
+    """(dt, launches) of a flight: dt = 0.01 throughout, or the edited flights' three dt phases."""
+    if not edits:
+        return [(0.01, launches)]
+    split = [launches - 2 * (launches // 3), launches // 3, launches // 3]
+    return list(zip(DT_PHASES, split))
+
+
+def spawn_of(n):
+    return big_grid(n, 0.0), rand(5, 0, n, -3, 3)
+
+
+def _run_variant(staging, frame, mode, k, n, launches, edits=None):
+    """One flight on the GPU with or without the staged kernel; returns (full state, crash flags, the variant that ran in each dt
+    phase)."""
     from mrs_multirotor_simulator_b200 import UavBatch
 
     if staging:
@@ -138,44 +213,40 @@ def _run_variant(staging, frame, mode, k, n, launches):
         os.environ["MRSB_NO_STAGING"] = "1"
     try:
         a = af(frame, ground_enabled=True, ground_z=0.0, takeoff_patch_enabled=True)  # FLAG_TAKEOFF on every UAV at spawn
-        b = UavBatch([a], spawn_xyz=big_grid(n, 0.0), spawn_heading=rand(5, 0, n, -3, 3), n=n)
-        # a third of the UAVs get a state whose v_prev differs from v (FLAG_VPREV) and a tilted, spinning start in the air
-        idx = np.arange(0, n, 3, dtype=np.int32)
-        m = len(idx)
-        st = b.get_state(idx)
-        x = st["x"] + np.stack([np.zeros(m), np.zeros(m), rand(5, 1, m, 0.5, 6.0)], axis=1)
-        v = np.stack([rand(5, 2, m, -2, 2), rand(5, 3, m, -2, 2), rand(5, 4, m, -1, 1)], axis=1)
-        w = np.stack([rand(5, 5, m, -0.5, 0.5), rand(5, 6, m, -0.5, 0.5), rand(5, 7, m, -0.5, 0.5)], axis=1)
-        b.set_state(idx, x=x, v=v, omega=w)
-        # a few crashed UAVs and a few without a command (US:308-310: motors driven to zero)
-        b.set_input(mode, commands(mode, n))
-        b.crash(np.arange(5, n, 997, dtype=np.int32))
-        b.apply_force(np.stack([rand(5, 8, n, -1, 1), rand(5, 9, n, -1, 1), rand(5, 10, n, -1, 1)], axis=1))
-        for _ in range(launches):
-            b.make_step(0.01, k)
-        info = b.step_info()
+        xyz, hdg = spawn_of(n)
+        b = UavBatch([a], spawn_xyz=xyz, spawn_heading=hdg, n=n)
+        setup_flight(b, np.arange(n), n, frame, mode, edits)
+        infos = []
+        for dt, count in flight_phases(launches, edits):
+            for _ in range(count):
+                b.make_step(dt, k)
+            infos.append(b.step_info())
         out = b.get_full_state()
         out["crashed"] = b.has_crashed()
         takeoff = np.array([b.get_params(int(i)).takeoff_patch_enabled for i in (0, 1, 2, 3, n - 1)])
         out["takeoff_flag_sample"] = takeoff
         b.close()
-        return out, info
+        return out, infos
     finally:
         os.environ.pop("MRSB_NO_STAGING", None)
 
 
+@pytest.mark.parametrize("edits", [None, "edited", "no_desaturation"])
 @pytest.mark.parametrize("frame,nm", [("x500", 4), ("f550", 6), ("naki", 8)])
 @pytest.mark.parametrize("mode", [O.ACTUATOR_CMD, O.VELOCITY_HDG_RATE_CMD, O.VELOCITY_HDG_CMD, O.POSITION_CMD])
 @pytest.mark.parametrize("k", [1, 10])
-def test_staged_equals_direct_bit_for_bit(frame, nm, mode, k):
+def test_staged_equals_direct_bit_for_bit(frame, nm, mode, k, edits):
     """Same swarm, same calls, staged kernel vs MRSB_NO_STAGING=1 (direct kernel): every state component, IMU, v_prev
-    and crash flag identical in every bit.  58,001 UAVs: 454 tiles, the last one holds 17 UAVs."""
+    and crash flag identical in every bit.  58,001 UAVs: 454 tiles, the last one holds 17 UAVs.  `edits`: the flights of
+    apply_edits (the staged kernel's parameter set passed by value after set_params and gain edits, live rate integrals, external
+    moments, feed-forwards), flown at dt = 0.01, 0.005, 0.02 in turn; the staged kernel must run in every dt phase."""
     n = 58001
     launches = 40 if k == 1 else 6
-    direct, info_d = _run_variant(False, frame, mode, k, n, launches)
-    staged, info_s = _run_variant(True, frame, mode, k, n, launches)
-    assert info_d["variant"] == "direct", info_d
-    assert info_s["variant"] == "staged" and info_s["n_motors"] == nm and info_s["mode"] == mode, info_s
+    direct, info_d = _run_variant(False, frame, mode, k, n, launches, edits)
+    staged, info_s = _run_variant(True, frame, mode, k, n, launches, edits)
+    for d, s in zip(info_d, info_s):
+        assert d["variant"] == "direct", d
+        assert s["variant"] == "staged" and s["n_motors"] == nm and s["mode"] == mode, s
     for key in direct:
         assert np.array_equal(direct[key], staged[key], equal_nan=True), f"{key} differs between the staged and the direct kernel"
     assert np.all(np.isfinite(staged["x"]))
