@@ -12,6 +12,7 @@
 #include <map>
 #include <memory>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -144,6 +145,56 @@ struct ParamSet {
   mrsb_controller_params cp;
 };
 
+// Buckets of the tiled arrays: one per airframe type present at create (a single one for a uniform batch), each a whole number
+// of tiles, so that the stepping kernel specialised for (motor count, parameter set) runs on each.
+#define MAX_BUCKETS 8
+struct Bucket {
+  int64_t   slot0 = 0, count = 0;  // first slot (multiple of 128), UAVs
+  int       nm    = 0;             // n_motors shared by its UAVs, or 0 if mixed (after per-UAV setParams)
+  int       pset  = -1;            // parameter set shared by its UAVs, or -1 if mixed
+  DevParams params{};              // host copy of that set (goes to the staged kernel by value)
+};
+
+// Everything the launches of a collision pass, and of a tick of mrsb_run (stepping launch + pass), take by value.  Those launches
+// take their arguments from this value alone, so a captured graph whose key equals what graph_args() gives now replays exactly
+// what would be launched now.  graph_args() zeroes it and copies whole structs in: equal keys are equal byte for byte (memcmp).
+static_assert(std::is_trivially_copyable_v<DevState> && std::is_trivially_copyable_v<DevGrid> && std::is_trivially_copyable_v<PeerView> &&
+              std::is_trivially_copyable_v<P2PCtl> && std::is_trivially_copyable_v<DevParams> && std::is_trivially_copyable_v<Bucket>);
+struct GraphArgs {
+  DevState s;  // its position buffers are the ones of the pass' parity
+  DevGrid  grid;
+  PeerView pv;
+  P2PCtl   p2p;
+  int32_t  crash, lists;
+  double   rebounce;
+  // the stepping launch (zero in a pass graph's key); publish: publish_positions follows (bucketed pull-exchange handles)
+  int32_t with_step, k_substeps, uniform_mode, any_moment, publish, n_buckets;
+  double  dt;
+  Bucket  buckets[MAX_BUCKETS];
+};
+static_assert(std::is_trivially_copyable_v<GraphArgs>);
+
+// A captured graph (exec, nullptr if not captured) and the GraphArgs it launches.  Move-only; the destructor destroys the graph.
+struct Graph {
+  cudaGraphExec_t exec = nullptr;
+  int             own  = 0;  // own kernels per replay (for the launch counter)
+  GraphArgs       key{};
+
+  Graph() = default;
+  explicit Graph(const GraphArgs& a) { std::memcpy(&key, &a, sizeof(a)); }
+  Graph(Graph&& o) noexcept { *this = std::move(o); }
+  Graph& operator=(Graph&& o) noexcept {
+    if (exec) cudaGraphExecDestroy(exec);
+    exec = std::exchange(o.exec, nullptr), own = o.own;
+    std::memcpy(&key, &o.key, sizeof(key));
+    return *this;
+  }
+  ~Graph() {
+    if (exec) cudaGraphExecDestroy(exec);
+  }
+  bool holds(const GraphArgs& a) const { return std::memcmp(&key, &a, sizeof(a)) == 0; }
+};
+
 struct mrsb_sim {
   int          device = 0;
   cudaStream_t stream = nullptr;
@@ -167,14 +218,6 @@ struct mrsb_sim {
 
   int  uniform_mode = MRSB_INPUT_UNKNOWN;  // INPUT_MODE shared by all UAVs, or -1 if mixed
   bool any_moment   = false;
-  // Buckets of the tiled arrays: one per airframe type present at create (a single one for a uniform batch), each a whole number
-  // of tiles, so that the stepping kernel specialised for (motor count, parameter set) runs on each.
-  struct Bucket {
-    int64_t   slot0 = 0, count = 0;  // first slot (multiple of 128), UAVs
-    int       nm    = 0;             // n_motors shared by its UAVs, or 0 if mixed (after per-UAV setParams)
-    int       pset  = -1;            // parameter set shared by its UAVs, or -1 if mixed
-    DevParams params{};              // host copy of that set (goes to the staged kernel by value)
-  };
   std::vector<Bucket>  buckets;
   std::vector<int32_t> perm_host, inv_host;  // external local index -> slot, slot -> external (-1 = padding); empty = identity
   int32_t*             d_perm = nullptr;
@@ -220,27 +263,19 @@ struct mrsb_sim {
   Mem<int32_t> d_sub_idx;  // mrsb_set_position_subset: the UAVs mrsb_get_positions_async downloads (its first n_sub; 0: all)
   int64_t      n_sub = 0;
 
-  // the collision pass is a fixed set of launches with fixed arguments: replayed as a CUDA graph (one per
-  // gather-buffer parity; with neighbour lists the table rebuild sits in a conditional node of it);
-  // invalidated when its arguments change
-  cudaGraphExec_t coll_graph[2]     = {nullptr, nullptr};
-  int             coll_graph_own[2] = {0, 0};  // own kernels per replay (for the launch counter)
+  // the collision pass, and mrsb_run's tick (stepping launch + pass), replayed as CUDA graphs, one per buffer parity (write_buf); with
+  // neighbour lists the table rebuild sits in a conditional node.  Captured again when the key is not the GraphArgs of now.
+  Graph pass[2], tick[2];
+  bool  graph_failed = false;  // a capture failed (e.g. conditional nodes unavailable): no more graphs for this handle
 
-  // neighbour lists (single-shard handles): the table rebuild sits in a conditional node of the graph
+  // neighbour lists (single-shard handles)
   bool     lists_on            = false;
   int      steps_since_pass    = 0;     // stepping launches since the last collision pass
   bool     positions_touched   = true;  // positions were written by something else than ONE stepping launch
   int      rebuild_own         = 0;     // own kernels of one rebuild (for the launch counter)
   int64_t  list_passes         = 0;     // passes that went through decide_kernel (it counts them too: NlCtl::n_passes)
-  bool     list_graph_failed   = false; // conditional graph nodes unavailable: do not try again on every pass
   int64_t  rebuilds_counted    = 0;
   Mem<uint32_t, true> h_one;               // pinned constant 1 (source of the async "force rebuild" copy)
-  cudaGraphExec_t tick_graph[2] = {nullptr, nullptr};  // mrsb_run: stepping launch + collision pass as ONE graph per parity
-  double   tick_dt = 0.0;
-  int      tick_k = 0, tick_mode = -2, tick_own[2] = {0, 0};
-  uint64_t tick_pset = ~0ull;  // fingerprint of the buckets' parameter sets the graphs were built for
-  uint32_t tick_opts = 0;
-  bool     tick_failed = false;
 
   // neighbour observations (mrsb_pack_neighbours_device): a table of its own, sized for n_local on the first call
   struct NbWorkspace {
@@ -253,15 +288,6 @@ struct mrsb_sim {
   int64_t n_steps = 0, n_passes = 0, n_launches = 0;
   int     step_info[4] = {0, 0, 0, 0};  // last stepping launch: variant, grid, NM_T, MODE_T (mrsb_get_step_info)
 };
-
-static void drop_collision_graphs(mrsb_sim* h) {
-  for (int k = 0; k < 2; k++) {
-    if (h->coll_graph[k]) cudaGraphExecDestroy(h->coll_graph[k]);
-    h->coll_graph[k] = nullptr;
-    if (h->tick_graph[k]) cudaGraphExecDestroy(h->tick_graph[k]);
-    h->tick_graph[k] = nullptr;
-  }
-}
 
 static std::string set_key(const ParamSet& s) {
   return std::string(reinterpret_cast<const char*>(&s), sizeof(ParamSet));
@@ -325,7 +351,6 @@ static int collect_param_sets(mrsb_sim* h) {
     kept.push_back(h->sets[size_t(k)]);
   }
   h->sets.swap(kept);
-  h->tick_pset = ~0ull;  // ids mean something else now
   for (int32_t& id : h->pset_host) id = remap[size_t(id)];
   CU(cudaMemcpyAsync(h->d_pset, h->pset_host.data(), sizeof(int32_t) * h->pset_host.size(), cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
@@ -341,11 +366,8 @@ static int flush_params(mrsb_sim* h) {
   const size_t cap    = size_t(std::max(16, 2 * n_sets));
   rc                  = h->d_params.grow(size_t(n_sets), cap, h->stream);
   if (rc) return rc;
-  if (h->ds.params != h->d_params.get()) {  // the graphs hold the table's address
-    h->ds.params = h->d_params.get();
-    drop_collision_graphs(h);
-  }
-  rc = h->d_takeoff0.grow(size_t(n_sets), cap, h->stream);
+  h->ds.params = h->d_params.get();
+  rc           = h->d_takeoff0.grow(size_t(n_sets), cap, h->stream);
   if (rc) return rc;
   std::vector<DevParams> host(n_sets);
   std::vector<uint8_t>   takeoff0(size_t(n_sets), 0);
@@ -357,7 +379,7 @@ static int flush_params(mrsb_sim* h) {
   CU(cudaMemcpyAsync(h->d_takeoff0.get(), takeoff0.data(), size_t(n_sets), cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));  // `host` and `takeoff0` go out of scope
   h->filt_dt = -1.0;                     // DevParams::filt has to be prepared again (ensure_filt)
-  for (mrsb_sim::Bucket& b : h->buckets) {
+  for (Bucket& b : h->buckets) {
     int nm = -1, ps = -2;
     for (int64_t k = 0; k < b.count; k++) {
       const int64_t e  = h->inv_host.empty() ? b.slot0 + k : h->inv_host[size_t(b.slot0 + k)];
@@ -382,14 +404,10 @@ static int flush_params(mrsb_sim* h) {
 static int ensure_filt(mrsb_sim* h, double dt) {
   if (h->filt_dt == dt) return MRSB_OK;
   h->n_launches += launch_prep_params(h->d_params.get(), int(h->sets.size()), dt, h->stream);
-  for (mrsb_sim::Bucket& b : h->buckets)
+  for (Bucket& b : h->buckets)
     if (b.pset >= 0) CU(cudaMemcpyAsync(&b.params.filt, &h->d_params.get()[b.pset].filt, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   h->filt_dt = dt;
-  for (int k = 0; k < 2; k++) {  // the tick graphs hold the parameter set by value
-    if (h->tick_graph[k]) cudaGraphExecDestroy(h->tick_graph[k]);
-    h->tick_graph[k] = nullptr;
-  }
   return MRSB_OK;
 }
 
@@ -735,7 +753,6 @@ static int setup_p2p(mrsb_sim* h) {
   // remote geometry is read from its owner from now on; the hand-shake also carries every rank's displacement bound, so
   // neighbour lists work across shards
   set_collision_geometry(h, h->grid.nl_count != nullptr);
-  drop_collision_graphs(h);
   CU(cudaStreamSynchronize(h->stream));
   return MRSB_OK;
 }
@@ -759,7 +776,7 @@ int mrsb_destroy(mrsb_handle h) {
   const cudaStream_t streams[3] = {h->stream, h->up_stream, h->down_stream};
   for (cudaStream_t s : streams)
     if (s) cudaStreamSynchronize(s);
-  drop_collision_graphs(h);
+  for (int k = 0; k < 2; k++) h->pass[k] = Graph(), h->tick[k] = Graph();  // the graphs before the memory they launch on
   for (void* p : h->ipc_opened) cudaIpcCloseMemHandle(p);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
   for (int k = 0; k < 2; k++)
@@ -786,7 +803,7 @@ int mrsb_bucket_layout(int64_t n, int32_t n_types, const int32_t* type_of_local_
     if (bucket_first_slot) bucket_first_slot[t] = -1;
     if (bucket_count) bucket_count[t] = per_type[size_t(t)];
   }
-  if (present < 2 || present > 8 || getenv("MRSB_NO_BUCKETS")) {
+  if (present < 2 || present > MAX_BUCKETS || getenv("MRSB_NO_BUCKETS")) {
     // one airframe (or too many to launch one kernel each): slots in the caller's order
     *n_slots = std::max<int64_t>(MRSB_TILE, round_up(n, MRSB_TILE));
     for (int64_t i = 0; i < n && slot_of_uav; i++) slot_of_uav[i] = int32_t(i);
@@ -847,7 +864,7 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     if (n_buckets > 1) {
       for (int t = 0; t < info->n_types; t++) {
         if (first[size_t(t)] < 0) continue;
-        mrsb_sim::Bucket b;
+        Bucket b;
         b.slot0 = first[size_t(t)], b.count = count[size_t(t)];
         h->buckets.push_back(b);
       }
@@ -855,7 +872,7 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
       h->inv_host.assign(size_t(s.ld), -1);
       for (int64_t i = 0; i < s.n; i++) h->inv_host[size_t(slot_of[size_t(i)])] = int32_t(i);
     } else {
-      mrsb_sim::Bucket b;
+      Bucket b;
       b.slot0 = 0, b.count = s.n;
       h->buckets.push_back(b);
     }
@@ -1243,39 +1260,55 @@ static int exchange_positions(mrsb_sim* h) {
   return MRSB_OK;
 }
 
-static int launch_step_buckets(mrsb_sim* h, double dt, int k_substeps);
+// What the launches of the collision pass that comes next take (with_step: of a tick, its stepping launch first).  With the pull
+// exchange, h->ds already points at the buffers of that pass' parity (after_pass).
+static void graph_args(const mrsb_sim* h, bool with_step, double dt, int k_substeps, GraphArgs* a) {
+  std::memset(static_cast<void*>(a), 0, sizeof(*a));  // padding included
+  std::memcpy(&a->s, &h->ds, sizeof(DevState));
+  std::memcpy(&a->grid, &h->grid, sizeof(DevGrid));
+  std::memcpy(&a->pv, h->p2p ? &h->pv[write_buf(h)] : &h->pv_local, sizeof(PeerView));
+  std::memcpy(&a->p2p, &h->p2pctl, sizeof(P2PCtl));
+  a->crash = h->coll_crash, a->lists = h->lists_on, a->rebounce = h->coll_rebounce;
+  if (!with_step) return;
+  a->with_step = 1, a->k_substeps = k_substeps, a->uniform_mode = h->uniform_mode, a->any_moment = h->any_moment, a->dt = dt;
+  a->publish   = h->p2p && h->ds.perm;  // bucketed: the per-group boxes follow the EXTERNAL order
+  a->n_buckets = int(h->buckets.size());
+  std::memcpy(a->buckets, h->buckets.data(), sizeof(Bucket) * h->buckets.size());
+}
 
-// what the kernels of the collision pass that comes next read: with the pull exchange, the buffers of that pass' parity
-struct PassView {
-  DevState        s;
-  const PeerView* pv;
-  int             k;  // graph slot
-};
-static PassView pass_view(mrsb_sim* h) {
-  PassView v;
-  v.s = h->ds;
-  if (h->p2p) {
-    v.k      = int((h->pass_no + 1) & 1);
-    v.s.gpos = h->gbuf[v.k];
-    v.s.gbox = h->d_gbox[v.k];
-    v.s.geom = h->d_geom[v.k];
-    v.pv     = &h->pv[v.k];
-  } else {
-    v.k  = 0;
-    v.pv = &h->pv_local;
+// the stepping launch: one kernel per bucket, each on its own view of the tiled arrays
+static int launch_step_buckets(const GraphArgs& a, cudaStream_t stream, int* info) {
+  int own = 0;
+  for (int i = 0; i < a.n_buckets; i++) {
+    const Bucket& b = a.buckets[i];
+    if (b.count <= 0) continue;
+    DevState v = a.s;
+    if (b.slot0 > 0) {
+      const int64_t t0 = b.slot0 / MRSB_TILE;
+      v.st += t0 * ST_ROWS * MRSB_TILE, v.vprev += t0 * VPREV_ROWS * MRSB_TILE, v.rpm += t0 * MRSB_NM * MRSB_TILE, v.pid += t0 * PID_ROWS * MRSB_TILE;
+      v.fext += t0 * F3_ROWS * MRSB_TILE, v.mext += t0 * F3_ROWS * MRSB_TILE, v.imu += t0 * F3_ROWS * MRSB_TILE, v.cmd += t0 * CMD_ROWS * MRSB_TILE;
+      v.ff += t0 * FF_ROWS * MRSB_TILE, v.initz += b.slot0, v.flags += b.slot0, v.mode += b.slot0;
+    }
+    if (v.inv) {
+      v.inv += b.slot0;
+      v.gbox = nullptr;  // its warps are not the external 32-UAV groups: publish_positions_kernel writes the boxes (below)
+    }
+    v.n = b.count;
+    own += launch_step(v, b.pset >= 0 ? &b.params : nullptr, a.dt, a.k_substeps, a.uniform_mode, b.nm, a.any_moment, stream, info);
   }
-  return v;
+  if (a.publish) own += launch_publish_positions(a.s, stream);
+  return own;
 }
 
 // decide -> IF (rebuild) { table, lists } -> check, captured into the graph being built on h->stream.
 // The IF node's condition is set on the device by decide_kernel (cudaGraphSetConditional).
-static bool capture_list_pass(mrsb_sim* h, const PassView& v, cudaGraph_t graph, cudaStream_t* side, int* own_fixed, int* own_rebuild) {
+static bool capture_list_pass(mrsb_sim* h, const GraphArgs& a, cudaGraph_t graph, cudaStream_t* side, int* own_fixed, int* own_rebuild) {
   cudaStreamCaptureStatus status;
   const cudaGraphNode_t*  deps  = nullptr;
   size_t                  n_dep = 0;
   cudaGraphConditionalHandle handle;
   if (cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault) != cudaSuccess) return false;
-  *own_fixed += launch_collide_decide(h->grid, h->p2pctl, 0, handle, 1, h->stream);
+  *own_fixed += launch_collide_decide(a.grid, a.p2p, 0, handle, 1, h->stream);
   if (cudaStreamGetCaptureInfo_v2(h->stream, &status, nullptr, &graph, &deps, &n_dep) != cudaSuccess) return false;
   cudaGraphNodeParams cp = {};
   cp.type                = cudaGraphNodeTypeConditional;
@@ -1287,15 +1320,15 @@ static bool capture_list_pass(mrsb_sim* h, const PassView& v, cudaGraph_t graph,
   cudaGraph_t body = cp.conditional.phGraph_out[0];
   if (!*side && cudaStreamCreateWithFlags(side, cudaStreamNonBlocking) != cudaSuccess) return false;
   if (cudaStreamBeginCaptureToGraph(*side, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal) != cudaSuccess) return false;
-  *own_rebuild = launch_collide_rebuild(v.s, h->grid, *v.pv, *side);
-  *own_rebuild += launch_collide_check(v.s, h->grid, *v.pv, h->coll_crash, h->coll_rebounce, 0, *side);  // the rebuilding pass' own list check
+  *own_rebuild = launch_collide_rebuild(a.s, a.grid, a.pv, *side);
+  *own_rebuild += launch_collide_check(a.s, a.grid, a.pv, a.crash, a.rebounce, 0, *side);  // the rebuilding pass' own list check
   cudaGraph_t body_out = nullptr;
   if (cudaStreamEndCapture(*side, &body_out) != cudaSuccess) return false;
   // The list check of an ordinary pass is captured BESIDE the conditional node (both depend on decide only): evaluating a
   // conditional node that is not taken takes ~10 us, which then overlaps the check instead of preceding it.  On a rebuilding
   // pass this launch returns at once (the body above ends with its own check).  The graph has two leaves; it is complete when
   // both are.
-  *own_fixed += launch_collide_check(v.s, h->grid, *v.pv, h->coll_crash, h->coll_rebounce, 1, h->stream);
+  *own_fixed += launch_collide_check(a.s, a.grid, a.pv, a.crash, a.rebounce, 1, h->stream);
   cudaGraphNode_t both[2] = {cond, nullptr};
   const cudaGraphNode_t* tail = nullptr;
   size_t                 n_tail = 0;
@@ -1305,30 +1338,35 @@ static bool capture_list_pass(mrsb_sim* h, const PassView& v, cudaGraph_t graph,
   return true;
 }
 
-// The pass with neighbour lists as ONE graph; with_step: preceded by the stepping launch (mrsb_run's tick graph).
-static cudaGraphExec_t build_pass_graph(mrsb_sim* h, const PassView& v, bool with_step, double dt, int k_sub, int* own_fixed, int* own_rebuild) {
-  cudaGraph_t     graph = nullptr;
-  cudaGraphExec_t exec  = nullptr;
-  cudaStream_t    side  = nullptr;
-  bool            ok    = false;
-  *own_fixed            = 0;
+// The graph of `a`: the stepping launch if a.with_step (mrsb_run's tick graph), then the pass with neighbour lists, or the full
+// pass.  exec stays nullptr if the capture fails.
+static Graph build_pass_graph(mrsb_sim* h, const GraphArgs& a) {
+  Graph        g(a);
+  cudaGraph_t  graph = nullptr;
+  cudaStream_t side  = nullptr;
+  bool         ok    = false;
   if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
     cudaGetLastError();
-    return nullptr;
+    return g;
   }
   do {
     cudaStreamCaptureStatus status;
     if (cudaStreamGetCaptureInfo_v2(h->stream, &status, nullptr, &graph, nullptr, nullptr) != cudaSuccess || !graph) break;
-    if (with_step) *own_fixed += launch_step_buckets(h, dt, k_sub);
-    ok = capture_list_pass(h, v, graph, &side, own_fixed, own_rebuild);
+    if (a.with_step) g.own += launch_step_buckets(a, h->stream, h->step_info);
+    if (a.lists) {
+      ok = capture_list_pass(h, a, graph, &side, &g.own, &h->rebuild_own);
+    } else {
+      g.own += launch_collide(a.s, a.grid, a.pv, a.p2p, a.crash, a.rebounce, h->stream);
+      ok = true;
+    }
   } while (false);
   cudaGraph_t captured = nullptr;
   const bool  ended    = cudaStreamEndCapture(h->stream, &captured) == cudaSuccess && captured;
-  if (ok && ended && cudaGraphInstantiate(&exec, captured, 0) != cudaSuccess) exec = nullptr;
+  if (ok && ended && cudaGraphInstantiate(&g.exec, captured, 0) != cudaSuccess) g.exec = nullptr;
   if (captured) cudaGraphDestroy(captured);
   if (side) cudaStreamDestroy(side);
   cudaGetLastError();
-  return exec;
+  return g;
 }
 
 // host bookkeeping before a pass that goes through decide_kernel
@@ -1365,75 +1403,33 @@ static int collide_local(mrsb_sim* h) {
     h->n_launches += launch_publish_positions(h->ds, h->stream);
     h->wrote_since_pass = true;
   }
-  const PassView v = pass_view(h);
-  const int      k = v.k;
   if (h->lists_on) {
     int rc = before_list_pass(h);
     if (rc) return rc;
-    if (!h->coll_graph[k] && !h->list_graph_failed && !getenv("MRSB_NO_GRAPH")) {
-      h->coll_graph[k]     = build_pass_graph(h, v, false, 0.0, 0, &h->coll_graph_own[k], &h->rebuild_own);
-      h->list_graph_failed = h->coll_graph[k] == nullptr;
-    }
-    if (h->coll_graph[k]) {
-      CU(cudaGraphLaunch(h->coll_graph[k], h->stream));
-      h->n_launches += h->coll_graph_own[k];  // the rebuilds are added from the device-side count (mrsb_get_counters)
-    } else {
-      // no graph (MRSB_NO_GRAPH, or conditional nodes unavailable): rebuild every pass
-      h->n_launches += launch_collide_decide(h->grid, h->p2pctl, 1, cudaGraphConditionalHandle{}, 0, h->stream);
-      h->rebuild_own = launch_collide_rebuild(v.s, h->grid, *v.pv, h->stream);
-      h->rebuild_own += launch_collide_check(v.s, h->grid, *v.pv, h->coll_crash, h->coll_rebounce, 0, h->stream);
-    }
-    return after_pass(h);
-  }
-  if (!h->coll_graph[k] && !getenv("MRSB_NO_GRAPH")) {
-    cudaGraph_t graph = nullptr;
-    if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-      const int own = launch_collide(v.s, h->grid, *v.pv, h->p2pctl, h->coll_crash, h->coll_rebounce, h->stream);
-      if (cudaStreamEndCapture(h->stream, &graph) == cudaSuccess && graph) {
-        if (cudaGraphInstantiate(&h->coll_graph[k], graph, 0) != cudaSuccess) h->coll_graph[k] = nullptr;
-        cudaGraphDestroy(graph);
-        h->coll_graph_own[k] = own;
-      }
-    }
-    cudaGetLastError();
-  }
-  if (h->coll_graph[k]) {
-    CU(cudaGraphLaunch(h->coll_graph[k], h->stream));
-    h->n_launches += h->coll_graph_own[k];
   } else {
-    h->n_launches += launch_collide(v.s, h->grid, *v.pv, h->p2pctl, h->coll_crash, h->coll_rebounce, h->stream);
+    h->steps_since_pass = 0;
   }
-  h->steps_since_pass = 0;
+  GraphArgs a;
+  graph_args(h, false, 0.0, 0, &a);
+  Graph& g       = h->pass[write_buf(h)];
+  bool   graphed = !h->graph_failed && !getenv("MRSB_NO_GRAPH");
+  if (graphed && !(g.exec && g.holds(a))) {
+    g               = build_pass_graph(h, a);
+    graphed         = g.exec != nullptr;
+    h->graph_failed = !graphed;
+  }
+  if (graphed) {
+    CU(cudaGraphLaunch(g.exec, h->stream));
+    h->n_launches += g.own;  // with neighbour lists the rebuilds are added from the device-side count (mrsb_get_counters)
+  } else if (a.lists) {
+    // no graph (MRSB_NO_GRAPH, or a capture failed): rebuild every pass
+    h->n_launches += launch_collide_decide(a.grid, a.p2p, 1, cudaGraphConditionalHandle{}, 0, h->stream);
+    h->rebuild_own = launch_collide_rebuild(a.s, a.grid, a.pv, h->stream);
+    h->rebuild_own += launch_collide_check(a.s, a.grid, a.pv, a.crash, a.rebounce, 0, h->stream);
+  } else {
+    h->n_launches += launch_collide(a.s, a.grid, a.pv, a.p2p, a.crash, a.rebounce, h->stream);
+  }
   return after_pass(h);
-}
-
-// the stepping launch: one kernel per bucket, each on its own view of the tiled arrays
-static int launch_step_buckets(mrsb_sim* h, double dt, int k_substeps) {
-  int own = 0;
-  for (const mrsb_sim::Bucket& b : h->buckets) {
-    if (b.count <= 0) continue;
-    DevState v = h->ds;
-    if (b.slot0 > 0) {
-      const int64_t t0 = b.slot0 / MRSB_TILE;
-      v.st += t0 * ST_ROWS * MRSB_TILE, v.vprev += t0 * VPREV_ROWS * MRSB_TILE, v.rpm += t0 * MRSB_NM * MRSB_TILE, v.pid += t0 * PID_ROWS * MRSB_TILE;
-      v.fext += t0 * F3_ROWS * MRSB_TILE, v.mext += t0 * F3_ROWS * MRSB_TILE, v.imu += t0 * F3_ROWS * MRSB_TILE, v.cmd += t0 * CMD_ROWS * MRSB_TILE;
-      v.ff += t0 * FF_ROWS * MRSB_TILE, v.initz += b.slot0, v.flags += b.slot0, v.mode += b.slot0;
-    }
-    if (v.inv) {
-      v.inv += b.slot0;
-      v.gbox = nullptr;  // its warps are not the external 32-UAV groups: publish_positions_kernel writes the boxes (below)
-    }
-    v.n = b.count;
-    own += launch_step(v, b.pset >= 0 ? &b.params : nullptr, dt, k_substeps, h->uniform_mode, b.nm, h->any_moment, h->stream, h->step_info);
-  }
-  if (h->p2p && h->ds.perm) own += launch_publish_positions(h->ds, h->stream);  // bucketed: the per-group boxes follow the EXTERNAL order
-  return own;
-}
-
-static uint64_t bucket_fingerprint(const mrsb_sim* h) {
-  uint64_t f = 1469598103934665603ull;
-  for (const mrsb_sim::Bucket& b : h->buckets) f = (f ^ uint64_t(uint32_t(b.pset + 1) * 16u + uint32_t(b.nm))) * 1099511628211ull;
-  return f;
 }
 
 static int before_step(mrsb_sim* h, double dt, int32_t k_substeps) {
@@ -1450,7 +1446,9 @@ int mrsb_make_step(mrsb_handle h, double dt, int32_t k_substeps) {
   GUARD(h);
   int rc = before_step(h, dt, k_substeps);
   if (rc) return rc;
-  h->n_launches += launch_step_buckets(h, dt, k_substeps);
+  GraphArgs a;
+  graph_args(h, true, dt, k_substeps, &a);
+  h->n_launches += launch_step_buckets(a, h->stream, h->step_info);
   h->wrote_since_pass = true;
   h->n_steps += k_substeps;
   h->steps_since_pass++;
@@ -1489,26 +1487,22 @@ int mrsb_handle_collisions_gathered(mrsb_handle h) {
 
 // One tick = stepping launch + collision pass.  With neighbour lists the two are ONE graph (per buffer parity): a single
 // cudaGraphLaunch per tick instead of a kernel launch plus a graph launch, and no gap between the stepping kernel and the
-// pass' first kernel.  The graph holds its arguments by value, so it is rebuilt when any of them changes.
+// pass' first kernel.
 static int run_tick_graph(mrsb_sim* h, double dt, int32_t k_substeps, bool* done) {
   *done = false;
-  if (!h->lists_on || h->tick_failed || h->list_graph_failed || getenv("MRSB_NO_GRAPH") || getenv("MRSB_NO_TICK_GRAPH")) return MRSB_OK;
+  if (!h->lists_on || h->graph_failed || getenv("MRSB_NO_GRAPH")) return MRSB_OK;
   if (h->positions_touched || h->steps_since_pass != 0) return MRSB_OK;  // let the ordinary path sort that out first
-  if (h->tick_dt != dt || h->tick_k != k_substeps || h->tick_mode != h->uniform_mode || h->tick_pset != bucket_fingerprint(h) ||
-      h->tick_opts != (h->ds.opts | (h->any_moment ? 0x10000u : 0u))) {
-    for (int k = 0; k < 2; k++) {
-      if (h->tick_graph[k]) cudaGraphExecDestroy(h->tick_graph[k]);
-      h->tick_graph[k] = nullptr;
-    }
-    h->tick_dt = dt, h->tick_k = k_substeps, h->tick_mode = h->uniform_mode, h->tick_pset = bucket_fingerprint(h),
-    h->tick_opts = h->ds.opts | (h->any_moment ? 0x10000u : 0u);
-    return MRSB_OK;  // this tick goes the ordinary way (first launches set up function attributes: not inside a capture); the next one builds the graph
+  GraphArgs a;
+  graph_args(h, true, dt, k_substeps, &a);
+  Graph& g = h->tick[write_buf(h)];
+  if (!g.holds(a)) {
+    g = Graph(a);
+    return MRSB_OK;  // this tick goes the ordinary way (first launches set up function attributes: not inside a capture); the next one of this parity builds the graph
   }
-  const PassView v = pass_view(h);
-  if (!h->tick_graph[v.k]) {
-    h->tick_graph[v.k] = build_pass_graph(h, v, true, dt, k_substeps, &h->tick_own[v.k], &h->rebuild_own);
-    if (!h->tick_graph[v.k]) {
-      h->tick_failed = true;
+  if (!g.exec) {
+    g = build_pass_graph(h, a);
+    if (!g.exec) {
+      h->graph_failed = true;
       return MRSB_OK;
     }
   }
@@ -1516,8 +1510,8 @@ static int run_tick_graph(mrsb_sim* h, double dt, int32_t k_substeps, bool* done
   h->wrote_since_pass = true;
   h->n_steps += k_substeps;
   h->list_passes++;
-  CU(cudaGraphLaunch(h->tick_graph[v.k], h->stream));
-  h->n_launches += h->tick_own[v.k];
+  CU(cudaGraphLaunch(g.exec, h->stream));
+  h->n_launches += g.own;
   *done = true;
   return after_pass(h);
 }
@@ -1953,7 +1947,6 @@ static int refresh_opts(mrsb_sim* h) {
   if (opts == h->ds.opts) return MRSB_OK;
   const bool pos_back = (opts & STEP_OPT_GPOS) && !(h->ds.opts & STEP_OPT_GPOS);
   h->ds.opts          = opts;
-  drop_collision_graphs(h);
   if (pos_back) {  // the packed positions were not kept up to date meanwhile
     h->n_launches += launch_publish_positions(h->ds, h->stream);
     h->wrote_since_pass  = true;
@@ -1968,7 +1961,6 @@ int mrsb_set_collisions(mrsb_handle h, int32_t enabled, int32_t crash, double re
   h->coll_enabled  = enabled != 0;
   h->coll_crash    = crash != 0;
   h->coll_rebounce = rebounce;
-  drop_collision_graphs(h);
   return refresh_opts(h);
 }
 
@@ -2015,7 +2007,6 @@ int mrsb_set_pair_capacity(mrsb_handle h, int64_t max_pairs) {
   if (rc) return rc;
   h->grid.pairs    = h->pairs.get();
   h->grid.pair_cap = max_pairs;
-  drop_collision_graphs(h);
   CU(cudaMemsetAsync(h->grid.counters, 0, sizeof(unsigned long long), h->stream));
   return MRSB_OK;
 }
