@@ -275,6 +275,53 @@ int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz
  * counts as mixed-mode afterwards: an RL loop sets its commands for the whole batch next (mrsb_set_input_device with
  * idx_dev == NULL), which keeps the stepping kernel specialised for that mode. */
 int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const double* xyz_dev, const double* heading_dev);
+
+/* ---- snapshots: save and restore every UAV's full dynamic state (checkpoint / resume, branching rollouts) ----
+ * MultirotorModel::setState (MM:424-433) puts back x, v, R, omega and motor RPM only; v_prev, the twelve PIDs, the active
+ * command, the feed-forwards and the take-off flag of a UavSystem (US:16-118 members) cannot be set from outside.  A snapshot
+ * holds all of it for every local UAV of one handle, as one record per UAV in external (caller) order, whatever the bucketing:
+ *   88 doubles — x, v, R (column-major), omega [18] | motor RPM [8] | PID last errors [12] and integrals [12] | command payload
+ *   [10] and cached cos/sin of its heading [2] | the four feed-forwards [13] | external force [3] | external moment [3] | IMU
+ *   acceleration [3] | v_prev [3] | spawn z [1] — plus a uint32 of flags (crashed, take-off patch, v_prev, feed-forwards, had a
+ *   command) and the uint8 INPUT_MODE: 709 bytes per UAV (743 MB of device memory at 1 Mi UAVs).
+ * Restoring a UAV puts back its record and nothing else.  Like a respawn, it keeps the UAV's airframe, parameter set
+ * (mrsb_set_params / mrsb_set_mass / mrsb_set_ground_z and the gain setters keep the values they set) and collision geometry;
+ * handle-level options (collisions, iterate_without_input, outputs, position subset) are not part of a snapshot either.  This is
+ * deliberate: parameters stay host-side bookkeeping, which a restore on the device could not update without a synchronisation.
+ * The integrals of the rate PIDs are not stored while rate ki == 0; they are zero then (every change of ki resets them), so a
+ * record saved with ki == 0 restores them as zero.  A record copied between UAVs of different motor counts is copied
+ * verbatim: defined, but not the continuation of any flight.
+ * Save and restore are local to this shard (not collective) and may be issued anywhere between two collision passes.  A
+ * restore makes the next collision pass rebuild its neighbour table (on every rank of a pull-exchange run) and replace every
+ * UAV's external force.  Afterwards the batch counts as single-mode if every UAV took its own record (src NULL: the mode it
+ * had at the save) or if it had, at the save and now, the same single mode; otherwise as mixed-mode.  The RL order (restore,
+ * then commands for the whole batch, then step) keeps the specialised stepping kernel either way. */
+
+/* A snapshot of this handle's UAVs (709 bytes per UAV of device memory; nothing saved yet).  It belongs to the handle:
+ * mrsb_snapshot_free or, at the latest, mrsb_destroy releases it.  Unknown or freed ids are MRSB_ERR_INVALID everywhere. */
+int mrsb_snapshot_create(mrsb_handle h, int32_t* id);
+int mrsb_snapshot_free(mrsb_handle h, int32_t id);
+/* Save the state of every local UAV into snapshot `id` (replacing what it held).  Enqueued on the handle's stream, no host
+ * synchronisation; changes nothing in the simulation (no displacement word, graph or counter but the launch counter).  It
+ * records the batch's input-mode and external-moment hints of the moment. */
+int mrsb_snapshot_save(mrsb_handle h, int32_t id);
+/* Host form: UAV idx[k] (idx NULL: UAV k) takes saved record src[k] (src NULL: its own), k < n.  Indices and records outside
+ * 0..n_local-1 are MRSB_ERR_INVALID; n == 0 is a no-op; duplicate idx entries are undefined.  MRSB_ERR_STATE if the snapshot was
+ * never saved or uploaded. */
+int mrsb_snapshot_restore(mrsb_handle h, int32_t id, int64_t n, const int32_t* idx, const int32_t* src);
+/* Device form, per UAV: src_dev[e] (int32, n_local entries, DEVICE memory) in 0..n_local-1 makes UAV e take that record; any
+ * other value leaves UAV e untouched.  src_dev NULL: every UAV takes its own record.  Enqueued on the handle's stream; no host
+ * synchronisation, no host round trip. */
+int mrsb_snapshot_restore_device(mrsb_handle h, int32_t id, const int32_t* src_dev);
+/* Host image of a snapshot, to resume in another process: a 48-byte header {char magic[8] "MRSBSNAP"; uint32 version, rows;
+ * int64 n_local, n_global, shard_begin; int32 input-mode hint, external-moment hint} followed by the snapshot's device bytes
+ * verbatim (rows [88][n_local] doubles, flags [n_local] uint32, mode [n_local] uint8).  *bytes = the image size of this handle.
+ * download synchronises and needs exactly that many bytes; upload checks them, the magic, the version and that the image was made
+ * by a handle of the same shard (n_local, n_global, shard_begin): MRSB_ERR_INVALID otherwise.  An uploaded snapshot restores as
+ * a saved one. */
+int mrsb_snapshot_image_size(mrsb_handle h, size_t* bytes);
+int mrsb_snapshot_download(mrsb_handle h, int32_t id, void* host, size_t bytes);
+int mrsb_snapshot_upload(mrsb_handle h, int32_t id, const void* host, size_t bytes);
 /* Current INPUT_MODE of each UAV (US:95). */
 int mrsb_get_input_mode(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* mode);
 

@@ -176,6 +176,27 @@ public:
   void forcesWritten() { check(mrsb_forces_written(h_)); }
   // episode reset of n UAVs (idx == nullptr: 0..n-1) at xyz[n][3], heading[n] (mrsb_respawn)
   void respawn(int64_t n, const int32_t* idx, const double* xyz, const double* heading) { check(mrsb_respawn(h_, n, idx, xyz, heading)); }
+  // snapshots of every UAV's full state (mrsb_snapshot_*); a snapshot lives until snapshotFree or the Swarm's end
+  int32_t snapshotCreate() {
+    int32_t id = 0;
+    check(mrsb_snapshot_create(h_, &id));
+    return id;
+  }
+  void snapshotFree(int32_t id) { check(mrsb_snapshot_free(h_, id)); }
+  void snapshotSave(int32_t id) { check(mrsb_snapshot_save(h_, id)); }
+  // UAV idx[k] (idx == nullptr: k) takes saved record src[k] (src == nullptr: its own), k < n
+  void snapshotRestore(int32_t id, int64_t n, const int32_t* idx = nullptr, const int32_t* src = nullptr) {
+    check(mrsb_snapshot_restore(h_, id, n, idx, src));
+  }
+  void snapshotRestoreDevice(int32_t id, const int32_t* src_dev = nullptr) { check(mrsb_snapshot_restore_device(h_, id, src_dev)); }
+  std::vector<unsigned char> snapshotImage(int32_t id) {
+    size_t bytes = 0;
+    check(mrsb_snapshot_image_size(h_, &bytes));
+    std::vector<unsigned char> out(bytes);
+    check(mrsb_snapshot_download(h_, id, out.data(), out.size()));
+    return out;
+  }
+  void snapshotLoad(int32_t id, const std::vector<unsigned char>& image) { check(mrsb_snapshot_upload(h_, id, image.data(), image.size())); }
   mrsb_handle handle() { return h_; }
 
 private:

@@ -95,6 +95,14 @@ SIGNATURES = {
     "mrsb_set_state_pos": (C.c_int, _N_IDX + [C.c_void_p, C.c_void_p]),
     "mrsb_respawn": (C.c_int, _N_IDX + [C.c_void_p, C.c_void_p]),
     "mrsb_respawn_masked_device": (C.c_int, [H, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mrsb_snapshot_create": (C.c_int, [H, C.POINTER(C.c_int32)]),
+    "mrsb_snapshot_free": (C.c_int, [H, C.c_int32]),
+    "mrsb_snapshot_save": (C.c_int, [H, C.c_int32]),
+    "mrsb_snapshot_restore": (C.c_int, [H, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
+    "mrsb_snapshot_restore_device": (C.c_int, [H, C.c_int32, C.c_void_p]),
+    "mrsb_snapshot_image_size": (C.c_int, [H, C.POINTER(C.c_size_t)]),
+    "mrsb_snapshot_download": (C.c_int, [H, C.c_int32, C.c_void_p, C.c_size_t]),
+    "mrsb_snapshot_upload": (C.c_int, [H, C.c_int32, C.c_void_p, C.c_size_t]),
     "mrsb_get_input_mode": (C.c_int, _N_IDX + [C.c_void_p]),
     "mrsb_crash": (C.c_int, _N_IDX),
     "mrsb_has_crashed": (C.c_int, _N_IDX + [C.c_void_p]),

@@ -221,6 +221,11 @@ class UavBatch:
         uint8 / bool [n], xyz float64 [n][3], heading float64 [n].  Enqueued on the handle's stream, no host synchronisation."""
         check(self._L.mrsb_respawn_masked_device(self.h, mask_ptr, xyz_ptr, heading_ptr))
 
+    def snapshot(self):
+        """A new Snapshot of this batch (709 bytes of device memory per UAV, nothing saved yet); see mrsb_snapshot_create for
+        what it holds and what a restore keeps."""
+        return Snapshot(self)
+
     def get_input_mode(self, idx=None):
         idx = _idx(idx)
         out = np.empty(self._n(idx), dtype=np.int32)
@@ -412,3 +417,48 @@ class UavBatch:
         v = DeviceView()
         check(self._L.mrsb_get_device_view(self.h, C.byref(v)))
         return v
+
+
+class Snapshot:
+    """The full dynamic state of every UAV of a UavBatch (mrsb_snapshot_*): state, motors, PIDs, command, feed-forwards, forces,
+    v_prev, flags and input mode.  A restore keeps each UAV's airframe, parameters, gains and collision geometry, as respawn does."""
+
+    def __init__(self, batch):
+        self.batch = batch
+        sid = C.c_int32(0)
+        check(batch._L.mrsb_snapshot_create(batch.h, C.byref(sid)))
+        self.id = sid.value
+
+    def save(self):
+        """Save every UAV's state; enqueued on the batch's stream, no host synchronisation."""
+        check(self.batch._L.mrsb_snapshot_save(self.batch.h, self.id))
+
+    def restore(self, idx=None, src=None):
+        """UAV idx[k] (None: every UAV) takes the saved record src[k] (None: its own)."""
+        idx = _idx(idx)
+        src = _idx(src)
+        n = self.batch.n if idx is None and src is None else len(idx if idx is not None else src)
+        check(self.batch._L.mrsb_snapshot_restore(self.batch.h, self.id, n, _ptr(idx), _ptr(src)))
+
+    def restore_device(self, src_ptr=None):
+        """UAV e takes the saved record src[e] where 0 <= src[e] < n and is left alone elsewhere; src_ptr is a raw device address
+        of int32 [n] (e.g. torch tensor .data_ptr()), None: every UAV takes its own.  Enqueued on the batch's stream, no host
+        synchronisation."""
+        check(self.batch._L.mrsb_snapshot_restore_device(self.batch.h, self.id, src_ptr))
+
+    def to_bytes(self):
+        """Host image of the snapshot (header + device bytes) for load_bytes() on a handle of the same shard, e.g. in another process."""
+        size = C.c_size_t(0)
+        check(self.batch._L.mrsb_snapshot_image_size(self.batch.h, C.byref(size)))
+        buf = np.empty(size.value, dtype=np.uint8)
+        check(self.batch._L.mrsb_snapshot_download(self.batch.h, self.id, _ptr(buf), size.value))
+        return buf.tobytes()
+
+    def load_bytes(self, b):
+        buf = np.frombuffer(b, dtype=np.uint8)
+        check(self.batch._L.mrsb_snapshot_upload(self.batch.h, self.id, _ptr(buf), len(buf)))
+
+    def free(self):
+        if self.id is not None and getattr(self.batch, "h", None):
+            check(self.batch._L.mrsb_snapshot_free(self.batch.h, self.id))
+        self.id = None

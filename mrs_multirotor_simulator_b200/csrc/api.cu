@@ -276,6 +276,7 @@ struct mrsb_sim {
   int64_t  list_passes         = 0;     // passes that went through decide_kernel (it counts them too: NlCtl::n_passes)
   int64_t  rebuilds_counted    = 0;
   Mem<uint32_t, true> h_one;               // pinned constant 1 (source of the async "force rebuild" copy)
+  Mem<unsigned long long, true> h_until;   // pinned source of NlCtl::write_all_until (forces_written)
 
   // neighbour observations (mrsb_pack_neighbours_device): a table of its own, sized for n_local on the first call
   struct NbWorkspace {
@@ -284,6 +285,16 @@ struct mrsb_sim {
     Mem<double4>            rec;
     Mem<unsigned long long> scan;
   } nb;
+
+  // snapshots (mrsb_snapshot_*), by id; ids are not reused
+  struct Snapshot {
+    Mem<unsigned char> mem;  // rows [SNAP_ROWS][n] doubles | flags uint32 [n] | mode uint8 [n], external order (n = n_local)
+    bool    filled       = false;               // saved or uploaded at least once
+    int32_t uniform_mode = MRSB_INPUT_UNKNOWN;  // the host hints when it was saved
+    bool    any_moment   = false;
+  };
+  std::map<int32_t, Snapshot> snapshots;
+  int32_t                     next_snapshot = 1;
 
   int64_t n_steps = 0, n_passes = 0, n_launches = 0;
   int     step_info[4] = {0, 0, 0, 0};  // last stepping launch: variant, grid, NM_T, MODE_T (mrsb_get_step_info)
@@ -984,6 +995,7 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     if (!rc && getenv("MRSB_TIMELINE")) rc = dalloc(h, &g.tl, size_t(MRSB_TL_TICKS) * 8);
     if (!rc) rc = dalloc(h, &g.ctl, 1);
     if (!rc) rc = h->h_one.alloc(2);
+    if (!rc) rc = h->h_until.alloc(1);
     if (rc) return rc;
     g.pairs       = h->pairs.get();
     g.halo_work_n = g.halo_n + 1;
@@ -1602,6 +1614,24 @@ int mrsb_set_state_pos(mrsb_handle h, int64_t n, const int32_t* idx, const doubl
   return MRSB_OK;
 }
 
+// The next pass that goes through decide_kernel replaces every force it visits (SIM:356-358), not only the ones it knows to be
+// non-zero.  No host synchronisation: the copy reads the pinned word when it runs.  If a later call has raised the word by then,
+// more passes than needed write every force they visit, which writes the values they would have left in place.
+static int write_all_forces_next_pass(mrsb_sim* h) {
+  if (!h->grid.ctl) return MRSB_OK;
+  *h->h_until.get() = (unsigned long long)h->list_passes + 1ull;  // index of the next pass that goes through decide_kernel
+  CU(cudaMemcpyAsync(&h->grid.ctl->write_all_until, h->h_until.get(), sizeof(unsigned long long), cudaMemcpyHostToDevice, h->stream));
+  return MRSB_OK;
+}
+
+// forces were written by something else than the collision pass: the next pass must replace every UAV's force
+static int forces_written(mrsb_sim* h) {
+  int rc = write_all_forces_next_pass(h);
+  if (rc) return rc;
+  h->positions_touched = true;  // that pass rebuilds: UAVs without candidates are only visited by a rebuild
+  return MRSB_OK;
+}
+
 // after a respawn: the buffer peers read has to show the new positions, and their per-group boxes (pull exchange)
 static int respawned(mrsb_sim* h) {
   if (h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);
@@ -1636,6 +1666,174 @@ int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const dou
   return respawned(h);
 }
 
+// ---- snapshots ------------------------------------------------------------------------------
+static size_t snapshot_bytes(const mrsb_sim* h) {
+  return size_t(h->ds.n) * (sizeof(double) * SNAP_ROWS + sizeof(uint32_t) + sizeof(uint8_t));
+}
+
+// the snapshot `id` of this handle, or nullptr (and MRSB_ERR_INVALID in *rc)
+static mrsb_sim::Snapshot* find_snapshot(mrsb_sim* h, int32_t id, int* rc) {
+  auto it = h->snapshots.find(id);
+  if (it != h->snapshots.end()) return &it->second;
+  *rc = fail(MRSB_ERR_INVALID, "no snapshot %d on this handle", id);
+  return nullptr;
+}
+
+struct SnapshotParts {
+  double*   rows;
+  uint32_t* flags;
+  uint8_t*  mode;
+};
+static SnapshotParts parts_of(const mrsb_sim* h, mrsb_sim::Snapshot& s) {
+  const size_t n = size_t(h->ds.n);
+  double*      r = reinterpret_cast<double*>(s.mem.get());
+  uint32_t*    f = reinterpret_cast<uint32_t*>(r + SNAP_ROWS * n);
+  return {r, f, reinterpret_cast<uint8_t*>(f + n)};
+}
+
+// The header of a snapshot image; the snapshot's device bytes follow it verbatim.
+struct SnapshotImageHeader {
+  char     magic[8];  // "MRSBSNAP"
+  uint32_t version, rows;
+  int64_t  n_local, n_global, shard_begin;
+  int32_t  uniform_mode, any_moment;
+};
+static const char     kSnapshotMagic[8]  = {'M', 'R', 'S', 'B', 'S', 'N', 'A', 'P'};
+static const uint32_t kSnapshotVersion = 1;
+
+int mrsb_snapshot_create(mrsb_handle h, int32_t* id) {
+  GUARD(h);
+  if (!id) return fail(MRSB_ERR_INVALID, "null id");
+  mrsb_sim::Snapshot s;
+  int rc = s.mem.alloc(std::max<size_t>(snapshot_bytes(h), 1));
+  if (rc) return rc;
+  *id = h->next_snapshot++;
+  h->snapshots.emplace(*id, std::move(s));
+  return MRSB_OK;
+}
+
+int mrsb_snapshot_free(mrsb_handle h, int32_t id) {
+  GUARD(h);
+  int rc = MRSB_OK;
+  if (!find_snapshot(h, id, &rc)) return rc;
+  CU(cudaStreamSynchronize(h->stream));  // a save or restore may still read or write it
+  h->snapshots.erase(id);
+  return MRSB_OK;
+}
+
+int mrsb_snapshot_save(mrsb_handle h, int32_t id) {
+  GUARD(h);
+  int                 rc = MRSB_OK;
+  mrsb_sim::Snapshot* s  = find_snapshot(h, id, &rc);
+  if (!s) return rc;
+  const SnapshotParts p = parts_of(h, *s);
+  h->n_launches += launch_snapshot_save(h->ds, p.rows, p.flags, p.mode, h->stream);
+  s->filled       = true;
+  s->uniform_mode = h->uniform_mode;
+  s->any_moment   = h->any_moment;
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
+// host bookkeeping after a restore.  all_own: every UAV took its own record.
+static int restored(mrsb_sim* h, const mrsb_sim::Snapshot& s, bool all_own) {
+  h->any_moment   = h->any_moment || s.any_moment;
+  h->uniform_mode = (all_own || h->uniform_mode == s.uniform_mode) ? s.uniform_mode : -1;
+  return respawned(h);
+}
+
+int mrsb_snapshot_restore(mrsb_handle h, int32_t id, int64_t n, const int32_t* idx, const int32_t* src) {
+  GUARD(h);
+  int                 rc = MRSB_OK;
+  mrsb_sim::Snapshot* s  = find_snapshot(h, id, &rc);
+  if (!s) return rc;
+  if (!s->filled) return fail(MRSB_ERR_STATE, "snapshot %d was never saved or uploaded", id);
+  const int32_t* d_idx = nullptr;
+  rc                   = stage_idx(h, n, idx, &d_idx);
+  if (rc || n == 0) return rc;
+  const int32_t* d_src = nullptr;
+  if (src) {
+    for (int64_t k = 0; k < n; k++)
+      if (src[k] < 0 || src[k] >= h->ds.n) return fail(MRSB_ERR_INVALID, "src[%lld]=%d outside 0..%lld", (long long)k, src[k], (long long)h->ds.n - 1);
+    rc = ensure_stage(h, sizeof(int32_t) * size_t(n));
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(h->d_stage.get(), src, sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice, h->stream));
+    d_src = reinterpret_cast<const int32_t*>(h->d_stage.get());
+  }
+  rc = forces_written(h);  // a restored external force may be non-zero where the next list-only pass would not look
+  if (rc) return rc;
+  const SnapshotParts p = parts_of(h, *s);
+  h->n_launches += launch_snapshot_restore(h->ds, p.rows, p.flags, p.mode, n, d_idx, d_src, h->stream);
+  h->positions_touched = true;
+  return restored(h, *s, !idx && !src && n == h->ds.n);
+}
+
+int mrsb_snapshot_restore_device(mrsb_handle h, int32_t id, const int32_t* src_dev) {
+  GUARD(h);
+  int                 rc = MRSB_OK;
+  mrsb_sim::Snapshot* s  = find_snapshot(h, id, &rc);
+  if (!s) return rc;
+  if (!s->filled) return fail(MRSB_ERR_STATE, "snapshot %d was never saved or uploaded", id);
+  // the host does not learn who was restored: the kernel raises the displacement word itself (the next pass rebuilds only if
+  // somebody was), and the next pass that goes through decide_kernel writes every force it visits
+  rc = write_all_forces_next_pass(h);
+  if (rc) return rc;
+  const SnapshotParts p = parts_of(h, *s);
+  h->n_launches += launch_snapshot_restore_masked(h->ds, p.rows, p.flags, p.mode, src_dev, h->stream);
+  return restored(h, *s, src_dev == nullptr);
+}
+
+int mrsb_snapshot_image_size(mrsb_handle h, size_t* bytes) {
+  GUARD(h);
+  if (!bytes) return fail(MRSB_ERR_INVALID, "null output");
+  *bytes = sizeof(SnapshotImageHeader) + snapshot_bytes(h);
+  return MRSB_OK;
+}
+
+int mrsb_snapshot_download(mrsb_handle h, int32_t id, void* host, size_t bytes) {
+  GUARD(h);
+  int                 rc = MRSB_OK;
+  mrsb_sim::Snapshot* s  = find_snapshot(h, id, &rc);
+  if (!s) return rc;
+  if (!host || bytes != sizeof(SnapshotImageHeader) + snapshot_bytes(h))
+    return fail(MRSB_ERR_INVALID, "image buffer of %zu bytes, need %zu (mrsb_snapshot_image_size)", bytes, sizeof(SnapshotImageHeader) + snapshot_bytes(h));
+  if (!s->filled) return fail(MRSB_ERR_STATE, "snapshot %d was never saved or uploaded", id);
+  SnapshotImageHeader hd;
+  std::memset(&hd, 0, sizeof(hd));
+  std::memcpy(hd.magic, kSnapshotMagic, sizeof(hd.magic));
+  hd.version = kSnapshotVersion, hd.rows = SNAP_ROWS;
+  hd.n_local = h->ds.n, hd.n_global = h->ds.n_global, hd.shard_begin = h->ds.shard_begin;
+  hd.uniform_mode = s->uniform_mode, hd.any_moment = s->any_moment ? 1 : 0;
+  std::memcpy(host, &hd, sizeof(hd));
+  if (h->ds.n) CU(cudaMemcpyAsync(static_cast<char*>(host) + sizeof(hd), s->mem.get(), snapshot_bytes(h), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return MRSB_OK;
+}
+
+int mrsb_snapshot_upload(mrsb_handle h, int32_t id, const void* host, size_t bytes) {
+  GUARD(h);
+  int                 rc = MRSB_OK;
+  mrsb_sim::Snapshot* s  = find_snapshot(h, id, &rc);
+  if (!s) return rc;
+  if (!host || bytes != sizeof(SnapshotImageHeader) + snapshot_bytes(h))
+    return fail(MRSB_ERR_INVALID, "image of %zu bytes, this handle's are %zu", bytes, sizeof(SnapshotImageHeader) + snapshot_bytes(h));
+  SnapshotImageHeader hd;
+  std::memcpy(&hd, host, sizeof(hd));
+  if (std::memcmp(hd.magic, kSnapshotMagic, sizeof(hd.magic)) != 0 || hd.version != kSnapshotVersion || hd.rows != SNAP_ROWS)
+    return fail(MRSB_ERR_INVALID, "not a snapshot image of this library version");
+  if (hd.n_local != h->ds.n || hd.n_global != h->ds.n_global || hd.shard_begin != h->ds.shard_begin)
+    return fail(MRSB_ERR_INVALID, "image of a shard of %lld UAVs at %lld of %lld, this handle has %lld at %lld of %lld", (long long)hd.n_local,
+                (long long)hd.shard_begin, (long long)hd.n_global, (long long)h->ds.n, (long long)h->ds.shard_begin, (long long)h->ds.n_global);
+  if (hd.uniform_mode < -1 || hd.uniform_mode > MRSB_POSITION_CMD || (hd.any_moment != 0 && hd.any_moment != 1))
+    return fail(MRSB_ERR_INVALID, "corrupt snapshot image header");
+  if (h->ds.n) CU(cudaMemcpyAsync(s->mem.get(), static_cast<const char*>(host) + sizeof(hd), snapshot_bytes(h), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaStreamSynchronize(h->stream));  // the caller may release `host` on return
+  s->filled       = true;
+  s->uniform_mode = hd.uniform_mode;
+  s->any_moment   = hd.any_moment != 0;
+  return MRSB_OK;
+}
+
 int mrsb_get_input_mode(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* mode) {
   GUARD(h);
   return download(h, n, idx, sizeof(int32_t) * size_t(n), mode, [&](const int32_t* d_idx, void* d_out) {
@@ -1663,17 +1861,6 @@ int mrsb_has_crashed(mrsb_handle h, int64_t n, const int32_t* idx, int32_t* cras
   int rc = get_flags(h, n, idx, reinterpret_cast<uint32_t*>(crashed));  // the flags, then in place what they say
   if (rc) return rc;
   for (int64_t k = 0; k < n; k++) crashed[k] = (uint32_t(crashed[k]) & FLAG_CRASHED) ? 1 : 0;
-  return MRSB_OK;
-}
-
-// forces were written by something else than the collision pass: the next pass must replace every UAV's
-// force (SIM:356-358), not only the ones it knows to be non-zero
-static int forces_written(mrsb_sim* h) {
-  if (!h->grid.ctl) return MRSB_OK;
-  const unsigned long long until = (unsigned long long)h->list_passes + 1ull;  // index of the next pass that goes through decide_kernel
-  CU(cudaMemcpyAsync(&h->grid.ctl->write_all_until, &until, sizeof(until), cudaMemcpyHostToDevice, h->stream));
-  CU(cudaStreamSynchronize(h->stream));  // `until` lives on this stack frame
-  h->positions_touched = true;           // that pass rebuilds: UAVs without candidates are only visited by a rebuild
   return MRSB_OK;
 }
 

@@ -229,6 +229,15 @@ int launch_respawn(const DevState& s, const uint8_t* takeoff0, int64_t n, const 
                    cudaStream_t stream);
 int launch_respawn_masked(const DevState& s, const uint8_t* takeoff0, const uint8_t* mask_dev, const double* xyz_dev, const double* hdg_dev,
                           cudaStream_t stream);
+// Snapshots (mrsb_snapshot_*): rows [SNAP_ROWS][s.n] doubles, flags [s.n], mode [s.n], all in external order.  save: every UAV.
+// restore: UAV idx[k] (nullptr: k) takes record src[k] (nullptr: its own), k < n.  restore_masked: UAV e takes record src[e]
+// when 0 <= src[e] < s.n (src == nullptr: its own), else is left alone; raises the displacement word when it restored anybody.
+#define SNAP_ROWS 88
+int launch_snapshot_save(const DevState& s, double* rows, uint32_t* flags, uint8_t* mode, cudaStream_t stream);
+int launch_snapshot_restore(const DevState& s, const double* rows, const uint32_t* flags, const uint8_t* mode, int64_t n, const int32_t* idx_dev,
+                            const int32_t* src_dev, cudaStream_t stream);
+int launch_snapshot_restore_masked(const DevState& s, const double* rows, const uint32_t* flags, const uint8_t* mode, const int32_t* src_dev,
+                                   cudaStream_t stream);
 int launch_stash_vprev(const DevState& s, int64_t n, const int32_t* idx_dev, cudaStream_t stream);
 int launch_gather_vprev(const DevState& s, int64_t n, const int32_t* idx_dev, double* out_dev, cudaStream_t stream);
 // zero the state (last error and integral) of PIDs [pid0, pid0 + n_pids)

@@ -160,6 +160,81 @@ __global__ void respawn_masked_kernel(DevState s, const uint8_t* __restrict__ ta
   if (s.disp_max && __ballot_sync(0xffffffffu, hit) && (threadIdx.x & 31) == 0) atomicMax(s.disp_max, 0xFFFFFFFFu);
 }
 
+// Snapshot record of the UAV in slot i (mrsb_snapshot_*): f(row, element) for every double row in record order — st 0-17, rpm
+// 18-25, pid 26-49, cmd 50-61, ff 62-74, fext 75-77, mext 78-80, imu 81-83, vprev 84-86, initz 87 (SNAP_ROWS).
+template <class F>
+DEV void for_each_record_row(const DevState& s, int64_t i, F f) {
+  int r = 0;
+#pragma unroll
+  for (int k = 0; k < ST_ROWS; k++) f(r++, s.st[tix(ST_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < MRSB_NM; k++) f(r++, s.rpm[tix(MRSB_NM, k, i)]);
+#pragma unroll
+  for (int k = 0; k < PID_ROWS; k++) f(r++, s.pid[tix(PID_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < CMD_ROWS; k++) f(r++, s.cmd[tix(CMD_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < FF_ROWS; k++) f(r++, s.ff[tix(FF_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < F3_ROWS; k++) f(r++, s.fext[tix(F3_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < F3_ROWS; k++) f(r++, s.mext[tix(F3_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < F3_ROWS; k++) f(r++, s.imu[tix(F3_ROWS, k, i)]);
+#pragma unroll
+  for (int k = 0; k < VPREV_ROWS; k++) f(r++, s.vprev[tix(VPREV_ROWS, k, i)]);
+  f(r, s.initz[i]);
+}
+static_assert(ST_ROWS + MRSB_NM + PID_ROWS + CMD_ROWS + FF_ROWS + 3 * F3_ROWS + VPREV_ROWS + 1 == SNAP_ROWS, "snapshot record rows");
+
+// One thread per slot (tile order): the reads of the tiled rows are coalesced, the writes go to the external index, which is
+// contiguous within a bucket.  Padding slots are skipped.
+__global__ void snapshot_save_kernel(DevState s, double* __restrict__ rows, uint32_t* __restrict__ flags, uint8_t* __restrict__ mode) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= s.ld) return;
+  const int64_t e = s.inv ? int64_t(s.inv[i]) : (i < s.n ? i : -1);
+  if (e < 0) return;
+  for_each_record_row(s, i, [&](int r, const double& v) { rows[r * s.n + e] = v; });
+  flags[e] = s.flags[i];
+  mode[e]  = s.mode[i];
+}
+
+// the UAV in slot i, external index e, takes saved record j: every row of the record, its flags and input mode, and its packed
+// position (what the collision pass, position downloads and publish_positions read), as write_pose does for a respawn
+DEV void restore_one(const DevState& s, const double* __restrict__ rows, const uint32_t* __restrict__ flags, const uint8_t* __restrict__ mode,
+                     int64_t i, int64_t e, int64_t j) {
+  for_each_record_row(s, i, [&](int r, double& v) { v = rows[r * s.n + j]; });
+  s.flags[i] = flags[j];
+  s.mode[i]  = mode[j];
+  double* gp = s.gpos + 3 * (s.shard_begin + e);
+  gp[0]      = rows[0 * s.n + j];
+  gp[1]      = rows[1 * s.n + j];
+  gp[2]      = rows[2 * s.n + j];
+}
+
+// host form: pair k = (UAV idx[k], record src[k]); idx == nullptr: UAV k, src == nullptr: its own record
+__global__ void snapshot_restore_kernel(DevState s, const double* __restrict__ rows, const uint32_t* __restrict__ flags, const uint8_t* __restrict__ mode,
+                                        int64_t n, const int32_t* __restrict__ idx, const int32_t* __restrict__ src) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int64_t e = ext(idx, k);
+  restore_one(s, rows, flags, mode, s.perm ? int64_t(s.perm[e]) : e, e, src ? int64_t(src[k]) : e);
+}
+
+// device form, one thread per slot: UAV e takes record src[e] when 0 <= src[e] < n (src == nullptr: its own), else is left alone.
+// A restored UAV moved behind the stepping kernel's displacement bound: as in respawn_masked_kernel, one atomic per warp that
+// restored anybody raises the displacement word to "unbounded".
+__global__ void snapshot_restore_masked_kernel(DevState s, const double* __restrict__ rows, const uint32_t* __restrict__ flags,
+                                               const uint8_t* __restrict__ mode, const int32_t* __restrict__ src) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  int64_t       e = -1, j = -1;
+  if (i < s.ld) e = s.inv ? int64_t(s.inv[i]) : (i < s.n ? i : -1);
+  if (e >= 0) j = src ? int64_t(src[e]) : e;
+  const bool hit = j >= 0 && j < s.n;
+  if (hit) restore_one(s, rows, flags, mode, i, e, j);
+  if (s.disp_max && __ballot_sync(0xffffffffu, hit) && (threadIdx.x & 31) == 0) atomicMax(s.disp_max, 0xFFFFFFFFu);
+}
+
 // before set_state overwrites v: remember the old v as v_prev (MM:424-433 leaves v_prev alone)
 __global__ void stash_vprev_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx) {
   const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -410,6 +485,23 @@ int launch_respawn(const DevState& s, const uint8_t* takeoff0, int64_t n, const 
 int launch_respawn_masked(const DevState& s, const uint8_t* takeoff0, const uint8_t* mask, const double* xyz, const double* hdg, cudaStream_t st) {
   if (s.n <= 0) return 0;
   respawn_masked_kernel<<<nblk(s.ld), 256, 0, st>>>(s, takeoff0, mask, xyz, hdg);  // s.ld is a whole number of warps
+  return 1;
+}
+int launch_snapshot_save(const DevState& s, double* rows, uint32_t* flags, uint8_t* mode, cudaStream_t st) {
+  if (s.n <= 0) return 0;
+  snapshot_save_kernel<<<nblk(s.ld), 256, 0, st>>>(s, rows, flags, mode);
+  return 1;
+}
+int launch_snapshot_restore(const DevState& s, const double* rows, const uint32_t* flags, const uint8_t* mode, int64_t n, const int32_t* idx,
+                            const int32_t* src, cudaStream_t st) {
+  if (n <= 0) return 0;
+  snapshot_restore_kernel<<<nblk(n), 256, 0, st>>>(s, rows, flags, mode, n, idx, src);
+  return 1;
+}
+int launch_snapshot_restore_masked(const DevState& s, const double* rows, const uint32_t* flags, const uint8_t* mode, const int32_t* src,
+                                   cudaStream_t st) {
+  if (s.n <= 0) return 0;
+  snapshot_restore_masked_kernel<<<nblk(s.ld), 256, 0, st>>>(s, rows, flags, mode, src);  // s.ld is a whole number of warps
   return 1;
 }
 int launch_stash_vprev(const DevState& s, int64_t n, const int32_t* idx, cudaStream_t st) {
