@@ -196,8 +196,24 @@ int mrsb_set_input_device(mrsb_handle h, int32_t mode, int64_t n, const int32_t*
  *    compute; `out_xyz` is valid after mrsb_sync (or mrsb_wait_downloads). */
 int mrsb_set_input_async(mrsb_handle h, int32_t mode, const double* payload, int32_t stride);
 int mrsb_get_positions_async(mrsb_handle h, double* out_xyz);
-/* Which UAVs mrsb_get_positions_async downloads from now on: the n UAVs idx[] (out_xyz then holds [n][3], in idx order) — a viewer
- * that follows part of the swarm does not pay PCIe for all of it.  idx == NULL or n == 0: all of them again.  Synchronises. */
+/* Pipelined sparse commands, for a node whose commands arrive one UAV at a time in any of the ten input modes (ROSW:679-981).
+ * Row k sets UAV idx[k] to input mode modes[k] (1..10) with payload row payload[k*stride ...], exactly as if
+ * mrsb_set_input(h, modes[k], 1, &idx[k], row k, stride) were called for k = 0..n-1 in order: a later row for the same UAV wins.
+ * Host arrays, pinned recommended; they must stay untouched until mrsb_wait_uploads / mrsb_sync.  Returns at once: the arrays
+ * go through the upload ring of mrsb_set_input_async (the two calls mix freely), and duplicates are resolved on the device.
+ * Checked on the host before anything is enqueued (MRSB_ERR_INVALID, nothing changes): NULL arrays, n outside 0..INT32_MAX,
+ * idx outside 0..n_local-1, mode 0 or outside 1..10, stride below the row length of any row's mode (actuator rows accept any
+ * stride >= 1; motors past the stride get 0).  n == 0 is a no-op.  The batch stays single-mode (specialised stepping kernel,
+ * cached tick graph) only if every row carries its mode; a later whole-batch call makes it single-mode again. */
+int mrsb_set_input_rows_async(mrsb_handle h, int64_t n, const int32_t* idx, const int32_t* modes, const double* payload, int32_t stride);
+/* Pipelined sensor rows (publishOdometry, publishIMU, publishRangefinder of every UAV's makeStep, ROSW:278-282): [m][17] =
+ * odometry 13 | IMU linear acceleration 3 | range 1 (the rows of mrsb_pack_observations_device) of the work enqueued so far, for the
+ * UAVs of mrsb_set_position_subset in its order (m = its n), or for all n_local UAVs.  Copied on the download stream with a
+ * two-deep ring of its own; valid after mrsb_sync / mrsb_wait_downloads.  Either download call may be issued every tick, in any
+ * order.  MRSB_ERR_STATE when the IMU rows are switched off (mrsb_set_outputs). */
+int mrsb_get_observations_async(mrsb_handle h, double* out17);
+/* The UAVs the async downloads deliver from now on: the n UAVs idx[] (out_xyz then holds [n][3], out17 [n][17], in idx order) — a
+ * viewer that follows part of the swarm does not pay PCIe for all of it.  idx == NULL or n == 0: all of them again.  Synchronises. */
 int mrsb_set_position_subset(mrsb_handle h, int64_t n, const int32_t* idx);
 int mrsb_wait_uploads(mrsb_handle h);
 int mrsb_wait_downloads(mrsb_handle h);

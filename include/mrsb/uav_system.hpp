@@ -164,6 +164,22 @@ public:
   void setIterateWithoutInput(bool enabled) { check(mrsb_set_iterate_without_input(h_, enabled)); }
   // optional per-step rows: the fabricated accelerometer (multirotor_model.hpp:280-281) and the packed positions
   void setOutputs(bool imu, bool positions) { check(mrsb_set_outputs(h_, (imu ? MRSB_OUT_IMU : 0u) | (positions ? MRSB_OUT_POSITIONS : 0u))); }
+  // ---- pipelined host I/O for a node loop (mrsb_*_async): every call returns at once; host arrays (pinned recommended) must stay
+  // untouched until waitUploads / sync, results are valid after waitDownloads / sync
+  // whole-batch command rows [size()][stride] of one mode
+  void setInputAsync(int32_t mode, const double* payload, int32_t stride) { check(mrsb_set_input_async(h_, mode, payload, stride)); }
+  // row k sets UAV idx[k] to mode modes[k] with payload row k, k < n; a later row for the same UAV wins
+  void setInputRowsAsync(int64_t n, const int32_t* idx, const int32_t* modes, const double* payload, int32_t stride) {
+    check(mrsb_set_input_rows_async(h_, n, idx, modes, payload, stride));
+  }
+  // positions [m][3] and odometry 13 | IMU acceleration 3 | range 1 rows [m][17] of the position subset (m = its size, else size())
+  void getPositionsAsync(double* out_xyz) { check(mrsb_get_positions_async(h_, out_xyz)); }
+  void getObservationsAsync(double* out17) { check(mrsb_get_observations_async(h_, out17)); }
+  // the UAVs the async downloads deliver (idx == nullptr or n == 0: all of them)
+  void setPositionSubset(int64_t n, const int32_t* idx) { check(mrsb_set_position_subset(h_, n, idx)); }
+  void waitUploads() { check(mrsb_wait_uploads(h_)); }
+  void waitDownloads() { check(mrsb_wait_downloads(h_)); }
+  void sync() { check(mrsb_sync(h_)); }
   std::vector<std::array<int32_t, 2>> collisionPairs() {
     int64_t n = 0;
     check(mrsb_get_collision_pairs(h_, nullptr, 0, &n));

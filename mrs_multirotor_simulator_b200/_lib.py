@@ -75,6 +75,8 @@ SIGNATURES = {
     "mrsb_set_input_device": (C.c_int, [H, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32]),
     "mrsb_set_input_async": (C.c_int, [H, C.c_int32, C.c_void_p, C.c_int32]),
     "mrsb_get_positions_async": (C.c_int, [H, C.c_void_p]),
+    "mrsb_set_input_rows_async": (C.c_int, [H, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),
+    "mrsb_get_observations_async": (C.c_int, [H, C.c_void_p]),
     "mrsb_set_position_subset": (C.c_int, [H, C.c_int64, C.c_void_p]),
     "mrsb_wait_uploads": (C.c_int, [H]),
     "mrsb_wait_downloads": (C.c_int, [H]),

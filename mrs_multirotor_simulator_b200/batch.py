@@ -125,8 +125,19 @@ class UavBatch:
         """Positions [n][3] -> host address `out_ptr` (pinned), downloaded on its own stream; valid after sync()."""
         check(self._L.mrsb_get_positions_async(self.h, out_ptr))
 
+    def set_input_rows_async(self, n, idx_ptr, modes_ptr, payload_ptr, stride):
+        """Row k sets UAV idx[k] to input mode modes[k] with payload row k, k < n, a later row for the same UAV winning: host
+        addresses (pinned) of int32 idx [n], int32 modes [n] and float64 rows [n][stride], uploaded on the upload stream; they
+        must stay untouched until sync()."""
+        check(self._L.mrsb_set_input_rows_async(self.h, int(n), idx_ptr, modes_ptr, payload_ptr, int(stride)))
+
+    def get_observations_async(self, out_ptr):
+        """odometry 13 | IMU acceleration 3 | range 1 of the position subset (all UAVs without one) -> host address `out_ptr`
+        (pinned, [m][17]), downloaded on the download stream; valid after sync()."""
+        check(self._L.mrsb_get_observations_async(self.h, out_ptr))
+
     def set_position_subset(self, idx=None):
-        """The UAVs get_positions_async downloads from now on (None: all)."""
+        """The UAVs get_positions_async and get_observations_async deliver from now on (None: all)."""
         idx = _idx(idx)
         check(self._L.mrsb_set_position_subset(self.h, 0 if idx is None else len(idx), _ptr(idx)))
 

@@ -254,13 +254,17 @@ struct mrsb_sim {
   std::vector<void*>   ipc_opened;
   Mem<int, true>       h_status;                         // pinned, mapped: set by the hand-shake on time-out
 
-  // pipelined host I/O (mrsb_set_input_async / mrsb_get_positions_async)
+  // pipelined host I/O (mrsb_set_input_async, mrsb_set_input_rows_async / mrsb_get_positions_async, mrsb_get_observations_async)
   cudaStream_t up_stream = nullptr, down_stream = nullptr;
-  Mem<double>  d_up[2];    // staged command rows
-  Mem<double>  d_snap[2];  // position snapshots [n_local][3]
+  Mem<double>  d_up[2];      // staged command rows
+  Mem<int32_t> d_up_idx[2];  // beside them, the index list [n] and the mode list [n] of a row upload
+  Mem<int32_t> d_last;       // one word per slot: the last row of a row upload addressed to it, -1 between uploads (made on first use)
+  Mem<double>  d_snap[2];    // position snapshots [n_local][3]
+  Mem<double>  d_obs[2];     // observation snapshots [n_local][17] (made on first use)
   cudaEvent_t  ev_up[2] = {nullptr, nullptr}, ev_applied[2] = {nullptr, nullptr}, ev_snap[2] = {nullptr, nullptr}, ev_down[2] = {nullptr, nullptr};
-  uint64_t     n_up = 0, n_down = 0;
-  Mem<int32_t> d_sub_idx;  // mrsb_set_position_subset: the UAVs mrsb_get_positions_async downloads (its first n_sub; 0: all)
+  cudaEvent_t  ev_obs_snap[2] = {nullptr, nullptr}, ev_obs_down[2] = {nullptr, nullptr};
+  uint64_t     n_up = 0, n_down = 0, n_obs = 0;
+  Mem<int32_t> d_sub_idx;  // mrsb_set_position_subset: the UAVs the async downloads deliver (its first n_sub; 0: all)
   int64_t      n_sub = 0;
 
   // the collision pass, and mrsb_run's tick (stepping launch + pass), replayed as CUDA graphs, one per buffer parity (write_buf); with
@@ -791,7 +795,7 @@ int mrsb_destroy(mrsb_handle h) {
   for (void* p : h->ipc_opened) cudaIpcCloseMemHandle(p);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
   for (int k = 0; k < 2; k++)
-    for (cudaEvent_t e : {h->ev_up[k], h->ev_applied[k], h->ev_snap[k], h->ev_down[k]})
+    for (cudaEvent_t e : {h->ev_up[k], h->ev_applied[k], h->ev_snap[k], h->ev_down[k], h->ev_obs_snap[k], h->ev_obs_down[k]})
       if (e) cudaEventDestroy(e);
   delete h;  // frees the memory
   for (cudaStream_t s : streams)
@@ -1044,6 +1048,37 @@ static int ensure_pipeline(mrsb_sim* h) {
   return MRSB_OK;
 }
 
+// Room for `rows` doubles and `words` int32 in both staging buffers of the upload ring.  Growing first waits for everything that may
+// still use them (the stream applies them, the upload stream fills them), then starts the ring afresh.
+static int reserve_upload(mrsb_sim* h, size_t rows, size_t words) {
+  if (rows <= std::min(h->d_up[0].cap(), h->d_up[1].cap()) && words <= std::min(h->d_up_idx[0].cap(), h->d_up_idx[1].cap())) return MRSB_OK;
+  CU(cudaStreamSynchronize(h->stream));     // the scatter reads the staging buffers,
+  CU(cudaStreamSynchronize(h->up_stream));  // the uploads write them
+  for (int k = 0; k < 2; k++) {
+    int rc = h->d_up[k].grow(rows, rows, h->up_stream);
+    if (!rc) rc = h->d_up_idx[k].grow(words, words, h->up_stream);
+    if (rc) return rc;
+  }
+  h->n_up = 0;
+  return MRSB_OK;
+}
+
+// The snapshot buffers and events of mrsb_get_observations_async on top of ensure_pipeline, made on first use; ready once the last
+// of them, d_obs[1], exists.  Sized for every local UAV, so that a position subset never makes them grow.
+static int ensure_obs_pipeline(mrsb_sim* h) {
+  if (h->d_obs[1].get()) return MRSB_OK;
+  int rc = ensure_pipeline(h);
+  if (rc) return rc;
+  const size_t rows = 17 * size_t(std::max<int64_t>(h->ds.n, 1));
+  for (int k = 0; k < 2; k++) {
+    for (cudaEvent_t* e : {&h->ev_obs_snap[k], &h->ev_obs_down[k]})
+      if (!*e) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    rc = h->d_obs[k].grow(rows, rows, h->down_stream);
+    if (rc) return rc;
+  }
+  return MRSB_OK;
+}
+
 int mrsb_set_input_async(mrsb_handle h, int32_t mode, const double* payload, int32_t stride) {
   GUARD(h);
   if (mode <= MRSB_INPUT_UNKNOWN || mode > MRSB_POSITION_CMD) return fail(MRSB_ERR_INVALID, "mode %d carries no payload", mode);
@@ -1053,15 +1088,8 @@ int mrsb_set_input_async(mrsb_handle h, int32_t mode, const double* payload, int
   if (rc) return rc;
   const int64_t n     = h->ds.n;
   const size_t  count = size_t(n) * size_t(stride);
-  if (count > std::min(h->d_up[0].cap(), h->d_up[1].cap())) {
-    CU(cudaStreamSynchronize(h->stream));     // the scatter reads the staging buffers,
-    CU(cudaStreamSynchronize(h->up_stream));  // the uploads write them
-    for (Mem<double>& b : h->d_up) {
-      rc = b.grow(count, count, h->up_stream);
-      if (rc) return rc;
-    }
-    h->n_up = 0;
-  }
+  rc                  = reserve_upload(h, count, 0);
+  if (rc) return rc;
   const int k = int(h->n_up & 1);
   if (h->n_up >= 2) CU(cudaStreamWaitEvent(h->up_stream, h->ev_applied[k], 0));  // the staging buffer was consumed two uploads ago
   CU(cudaMemcpyAsync(h->d_up[k].get(), payload, sizeof(double) * count, cudaMemcpyHostToDevice, h->up_stream));
@@ -1071,6 +1099,48 @@ int mrsb_set_input_async(mrsb_handle h, int32_t mode, const double* payload, int
   CU(cudaEventRecord(h->ev_applied[k], h->stream));
   h->n_up++;
   note_mode(h, mode, n, true);
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
+// The same ring as mrsb_set_input_async: index list, mode list and rows go into staging buffer n_up & 1, which the stream has
+// finished reading two uploads ago; the stream waits for the copies, then the claim and apply kernels resolve duplicate UAVs.
+int mrsb_set_input_rows_async(mrsb_handle h, int64_t n, const int32_t* idx, const int32_t* modes, const double* payload, int32_t stride) {
+  GUARD(h);
+  if (n < 0 || n > INT32_MAX) return fail(MRSB_ERR_INVALID, "n=%lld outside 0..%d", (long long)n, INT32_MAX);
+  if (n == 0) return MRSB_OK;
+  if (!idx || !modes || !payload) return fail(MRSB_ERR_INVALID, "null idx, modes or payload");
+  bool uniform = true;  // every row carries the batch's single mode
+  for (int64_t k = 0; k < n; k++) {
+    if (idx[k] < 0 || idx[k] >= h->ds.n) return fail(MRSB_ERR_INVALID, "idx[%lld]=%d outside 0..%lld", (long long)k, idx[k], (long long)h->ds.n - 1);
+    const int m = modes[k];
+    if (m <= MRSB_INPUT_UNKNOWN || m > MRSB_POSITION_CMD) return fail(MRSB_ERR_INVALID, "modes[%lld]=%d carries no payload", (long long)k, m);
+    if (stride < (m == MRSB_ACTUATOR_CMD ? 1 : stride_of(m))) return fail(MRSB_ERR_INVALID, "stride %d too small for modes[%lld]=%d", stride, (long long)k, m);
+    uniform = uniform && m == h->uniform_mode;
+  }
+  int rc = ensure_pipeline(h);
+  if (rc) return rc;
+  if (!h->d_last.get()) {
+    const size_t slots = size_t(std::max<int64_t>(h->ds.ld, 1));
+    rc                 = h->d_last.alloc(slots);
+    if (rc) return rc;
+    CU(cudaMemsetAsync(h->d_last.get(), 0xFF, sizeof(int32_t) * slots, h->stream));  // -1 everywhere
+  }
+  const size_t rows = size_t(n) * size_t(stride);
+  rc                = reserve_upload(h, rows, 2 * size_t(n));
+  if (rc) return rc;
+  const int k = int(h->n_up & 1);
+  if (h->n_up >= 2) CU(cudaStreamWaitEvent(h->up_stream, h->ev_applied[k], 0));  // the staging buffer was consumed two uploads ago
+  int32_t* d_idx = h->d_up_idx[k].get();
+  CU(cudaMemcpyAsync(d_idx, idx, sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice, h->up_stream));
+  CU(cudaMemcpyAsync(d_idx + n, modes, sizeof(int32_t) * size_t(n), cudaMemcpyHostToDevice, h->up_stream));
+  CU(cudaMemcpyAsync(h->d_up[k].get(), payload, sizeof(double) * rows, cudaMemcpyHostToDevice, h->up_stream));
+  CU(cudaEventRecord(h->ev_up[k], h->up_stream));
+  CU(cudaStreamWaitEvent(h->stream, h->ev_up[k], 0));
+  h->n_launches += launch_input_rows(h->ds, n, d_idx, d_idx + n, h->d_up[k].get(), stride, h->d_last.get(), h->stream);
+  CU(cudaEventRecord(h->ev_applied[k], h->stream));
+  h->n_up++;
+  if (!uniform) h->uniform_mode = -1;  // rows never make a batch uniform: only a whole-batch call does
   CU(cudaGetLastError());
   return MRSB_OK;
 }
@@ -1096,6 +1166,28 @@ int mrsb_get_positions_async(mrsb_handle h, double* out_xyz) {
   CU(cudaMemcpyAsync(out_xyz, h->d_snap[k].get(), bytes, cudaMemcpyDeviceToHost, h->down_stream));
   CU(cudaEventRecord(h->ev_down[k], h->down_stream));
   h->n_down++;
+  return MRSB_OK;
+}
+
+// The protocol of mrsb_get_positions_async with a ring of its own: observe_kernel packs the rows into snapshot buffer n_obs & 1, which
+// the download stream finished copying out two reads ago, and the download stream copies them out once they are complete.
+int mrsb_get_observations_async(mrsb_handle h, double* out17) {
+  GUARD(h);
+  if (!out17) return fail(MRSB_ERR_INVALID, "null output");
+  if (!(h->ds.opts & STEP_OPT_IMU)) return fail(MRSB_ERR_STATE, "the IMU rows are switched off (mrsb_set_outputs)");
+  int rc = flush_params(h);  // the range rows read ground_z
+  if (!rc) rc = ensure_obs_pipeline(h);
+  if (rc) return rc;
+  const int     k = int(h->n_obs & 1);
+  const int64_t m = h->n_sub ? h->n_sub : h->ds.n;
+  if (h->n_obs >= 2) CU(cudaStreamWaitEvent(h->stream, h->ev_obs_down[k], 0));  // the snapshot buffer was downloaded two reads ago
+  h->n_launches += launch_observe(h->ds, 3, m, h->n_sub ? h->d_sub_idx.get() : nullptr, h->d_obs[k].get(), 17, h->stream);
+  CU(cudaEventRecord(h->ev_obs_snap[k], h->stream));
+  CU(cudaStreamWaitEvent(h->down_stream, h->ev_obs_snap[k], 0));
+  CU(cudaMemcpyAsync(out17, h->d_obs[k].get(), sizeof(double) * 17 * size_t(m), cudaMemcpyDeviceToHost, h->down_stream));
+  CU(cudaEventRecord(h->ev_obs_down[k], h->down_stream));
+  h->n_obs++;
+  CU(cudaGetLastError());
   return MRSB_OK;
 }
 

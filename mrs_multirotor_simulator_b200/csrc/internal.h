@@ -213,6 +213,10 @@ int launch_neighbours(const DevState& s, const DevGrid& t, double* pos, double* 
 int launch_publish_positions(const DevState& s, cudaStream_t stream);
 
 int launch_scatter_input(const DevState& s, int mode, int64_t n, const int32_t* idx_dev, const double* payload_dev, int stride, cudaStream_t stream);
+// row k (k < n <= INT32_MAX) sets UAV idx_dev[k] to mode modes_dev[k] with payload row k; of several rows for one UAV the last wins.
+// last_dev: one int32 per slot (s.ld), -1 before and after the call.
+int launch_input_rows(const DevState& s, int64_t n, const int32_t* idx_dev, const int32_t* modes_dev, const double* payload_dev, int stride,
+                      int32_t* last_dev, cudaStream_t stream);
 // payload[k][0..rows) <-> rows [row0, row0+rows) of a tiled array with `rows_total` components
 int launch_scatter_rows(double* dst, int rows_total, int row0, int rows, int64_t n, const int32_t* idx_dev, const double* payload_dev, int stride,
                         const int32_t* perm, cudaStream_t stream);

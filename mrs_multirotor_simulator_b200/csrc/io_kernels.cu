@@ -17,17 +17,11 @@ DEV int64_t at(const int32_t* perm, const int32_t* idx, int64_t k) {
 
 inline unsigned nblk(int64_t n, int t = 256) { return unsigned((n + t - 1) / t); }
 
-// UavSystem::setInput overloads (US:175-248): store the command, switch the mode.  cos/sin of the
-// commanded heading (used by CTL/acceleration_controller.hpp:50) are cached once per command
-// instead of being re-evaluated every step.
-__global__ void scatter_input_kernel(DevState s, int mode, int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ payload, int stride) {
-  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (k >= n) return;
-  const int64_t e = ext(idx, k);
-  if (e < 0 || e >= s.n) return;
-  const int64_t i = s.perm ? int64_t(s.perm[e]) : e;
-  const double* p    = payload + k * stride;
-  const int     rows = mode == MRSB_ACTUATOR_CMD ? MRSB_NM : (mode == MRSB_ATTITUDE_CMD ? 10 : (mode == MRSB_TILT_HDG_RATE_CMD ? 5 : 4));
+// UavSystem::setInput overloads (US:175-248) for the UAV in slot i: store the command row p[0 .. stride), switch the mode.  cos/sin
+// of the commanded heading (used by CTL/acceleration_controller.hpp:50) are cached once per command instead of being re-evaluated
+// every step.
+DEV void apply_input(const DevState& s, int mode, int64_t i, const double* __restrict__ p, int stride) {
+  const int rows = mode == MRSB_ACTUATOR_CMD ? MRSB_NM : (mode == MRSB_ATTITUDE_CMD ? 10 : (mode == MRSB_TILT_HDG_RATE_CMD ? 5 : 4));
   for (int r = 0; r < rows; r++) s.cmd[tix(CMD_ROWS, r, i)] = r < stride ? p[r] : 0.0;
   if (mode == MRSB_POSITION_CMD || mode == MRSB_VELOCITY_HDG_CMD || mode == MRSB_ACCELERATION_HDG_CMD) {
     double sn, cs;
@@ -37,6 +31,35 @@ __global__ void scatter_input_kernel(DevState s, int mode, int64_t n, const int3
   }
   s.mode[i] = uint8_t(mode);
   if (!(s.flags[i] & FLAG_HAD_INPUT)) s.flags[i] |= FLAG_HAD_INPUT;  // time_last_input_ > 0 from now on (ROSW:265)
+}
+
+__global__ void scatter_input_kernel(DevState s, int mode, int64_t n, const int32_t* __restrict__ idx, const double* __restrict__ payload, int stride) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int64_t e = ext(idx, k);
+  if (e < 0 || e >= s.n) return;
+  const int64_t i = s.perm ? int64_t(s.perm[e]) : e;
+  apply_input(s, mode, i, payload + k * stride, stride);
+}
+
+// Mixed-mode command rows (mrsb_set_input_rows_async): row k sets UAV idx[k] to mode modes[k], and of several rows for one UAV the
+// last one wins — without sorting.  last[slot] is a persistent word that holds -1 between calls.  The claim kernel leaves in it the
+// highest row number addressed to the slot; in the apply kernel that row alone applies itself and puts the -1 back.  A losing row
+// reads the winner's number or, once the winner is done, -1: either way not its own, so it skips.
+__global__ void input_rows_claim_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx, int32_t* __restrict__ last) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  atomicMax(&last[at(s.perm, idx, k)], int32_t(k));
+}
+
+__global__ void input_rows_apply_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx, const int32_t* __restrict__ modes,
+                                        const double* __restrict__ payload, int stride, int32_t* last) {
+  const int64_t k = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int64_t i = at(s.perm, idx, k);
+  if (last[i] != int32_t(k)) return;
+  apply_input(s, modes[k], i, payload + k * stride, stride);
+  last[i] = -1;
 }
 
 __global__ void set_mode_kernel(DevState s, int64_t n, const int32_t* __restrict__ idx, int mode) {
@@ -439,6 +462,13 @@ int launch_scatter_input(const DevState& s, int mode, int64_t n, const int32_t* 
   if (n <= 0) return 0;
   scatter_input_kernel<<<nblk(n), 256, 0, st>>>(s, mode, n, idx, payload, stride);
   return 1;
+}
+int launch_input_rows(const DevState& s, int64_t n, const int32_t* idx, const int32_t* modes, const double* payload, int stride, int32_t* last,
+                      cudaStream_t st) {
+  if (n <= 0) return 0;
+  input_rows_claim_kernel<<<nblk(n), 256, 0, st>>>(s, n, idx, last);
+  input_rows_apply_kernel<<<nblk(n), 256, 0, st>>>(s, n, idx, modes, payload, stride, last);
+  return 2;
 }
 int launch_set_mode(const DevState& s, int64_t n, const int32_t* idx, int mode, cudaStream_t st) {
   if (n <= 0) return 0;
