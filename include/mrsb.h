@@ -436,6 +436,10 @@ int mrsb_get_counters(mrsb_handle h, int64_t* out5);
  * CTAs, next tile fetched by TMA bulk copies into shared memory); [1] grid size; [2] motors per UAV the kernel was
  * specialised for (0 = per UAV); [3] INPUT_MODE it was specialised for (-1 = per UAV). */
 int mrsb_get_step_info(mrsb_handle h, int32_t* out4);
+/* Diagnostics: how many staged stepping launches of each airframe bucket swept with alternating direction (forward, backward,
+ * forward, ...; results do not depend on it).  Only a handle with a single bucket alternates, and only launches that stream more
+ * state than the L2 cache holds.  out[b] for the first min(cap, *n_buckets) buckets; synchronises the handle's stream. */
+int mrsb_get_sweep_launches(mrsb_handle h, int64_t* out, int32_t cap, int32_t* n_buckets);
 /* Diagnostics: device-clock stamps (nanoseconds, %globaltimer) the kernels of the last collision passes left when the handle was
  * created with the environment variable MRSB_TIMELINE=1: out[k][8] for the last min(n, max_passes, 4096) passes, oldest first —
  * [0] pass start, [1] peer hand-shake sent, [2] hand-shake complete, [3] halo refresh start, [4] list check start, [5] 1 if the pass

@@ -134,6 +134,7 @@ SIGNATURES = {
     "mrsb_set_pair_capacity": (C.c_int, [H, C.c_int64]),
     "mrsb_get_counters": (C.c_int, [H, C.c_void_p]),
     "mrsb_get_step_info": (C.c_int, [H, C.c_void_p]),
+    "mrsb_get_sweep_launches": (C.c_int, [H, C.c_void_p, C.c_int32, C.POINTER(C.c_int32)]),
     "mrsb_get_timeline": (C.c_int, [H, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
     "mrsb_get_collision_info": (C.c_int, [H, C.c_void_p]),
     "mrsb_forces_written": (C.c_int, [H]),

@@ -386,6 +386,13 @@ class UavBatch:
         return dict(variant={0: "none", 1: "direct", 2: "staged", 3: "staged+peer-stores"}[int(out[0])], grid=int(out[1]), n_motors=int(out[2]),
                     mode=int(out[3]))
 
+    def sweep_launches(self):
+        """Per airframe bucket: staged stepping launches that swept with alternating direction (diagnostics)."""
+        out = np.zeros(8, dtype=np.int64)
+        nb = C.c_int32()
+        check(self._L.mrsb_get_sweep_launches(self.h, _ptr(out), len(out), C.byref(nb)))
+        return out[: nb.value].tolist()
+
     def timeline(self, max_passes=4096):
         """Device-clock stamps of the last collision passes [k][8] (needs MRSB_TIMELINE=1 at creation); see mrsb_get_timeline."""
         out = np.zeros((max_passes, 8), dtype=np.uint64)

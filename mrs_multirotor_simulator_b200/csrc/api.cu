@@ -153,6 +153,7 @@ struct Bucket {
   int       nm    = 0;             // n_motors shared by its UAVs, or 0 if mixed (after per-UAV setParams)
   int       pset  = -1;            // parameter set shared by its UAVs, or -1 if mixed
   DevParams params{};              // host copy of that set (goes to the staged kernel by value)
+  uint32_t* sweep = nullptr;       // its staged launches' direction word (launch_step)
 };
 
 // Everything the launches of a collision pass, and of a tick of mrsb_run (stepping launch + pass), take by value.  Those launches
@@ -916,6 +917,9 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
   if (!rc) rc = dalloc(h, &s.flags, ld);
   if (!rc) rc = dalloc(h, &s.mode, ld);
   if (!rc) rc = dalloc(h, &s.gpos, 3 * size_t(s.n_global));
+  uint32_t* sweep = nullptr;
+  if (!rc) rc = dalloc(h, &sweep, h->buckets.size());
+  for (size_t i = 0; !rc && i < h->buckets.size(); i++) h->buckets[i].sweep = sweep + i;
   if (!rc) rc = dalloc(h, &h->d_pset, size_t(s.n_global));
   if (rc) return rc;
   s.pset = h->d_pset;
@@ -1382,7 +1386,8 @@ static void graph_args(const mrsb_sim* h, bool with_step, double dt, int k_subst
 
 // the stepping launch: one kernel per bucket, each on its own view of the tiled arrays
 static int launch_step_buckets(const GraphArgs& a, cudaStream_t stream, int* info) {
-  int own = 0;
+  int own = 0, filled = 0;
+  for (int i = 0; i < a.n_buckets; i++) filled += a.buckets[i].count > 0;
   for (int i = 0; i < a.n_buckets; i++) {
     const Bucket& b = a.buckets[i];
     if (b.count <= 0) continue;
@@ -1398,7 +1403,9 @@ static int launch_step_buckets(const GraphArgs& a, cudaStream_t stream, int* inf
       v.gbox = nullptr;  // its warps are not the external 32-UAV groups: publish_positions_kernel writes the boxes (below)
     }
     v.n = b.count;
-    own += launch_step(v, b.pset >= 0 ? &b.params : nullptr, a.dt, a.k_substeps, a.uniform_mode, b.nm, a.any_moment, stream, info);
+    // the sweep direction alternates only for a single bucket: with several, the other buckets' launches stream their own state
+    // through L2 between two launches of this one, and nothing of it is left to reuse
+    own += launch_step(v, b.pset >= 0 ? &b.params : nullptr, filled == 1 ? b.sweep : nullptr, a.dt, a.k_substeps, a.uniform_mode, b.nm, a.any_moment, stream, info);
   }
   if (a.publish) own += launch_publish_positions(a.s, stream);
   return own;
@@ -2318,6 +2325,18 @@ int mrsb_get_step_info(mrsb_handle h, int32_t* out4) {
   GUARD(h);
   if (!out4) return fail(MRSB_ERR_INVALID, "null output");
   for (int k = 0; k < 4; k++) out4[k] = h->step_info[k];
+  return MRSB_OK;
+}
+
+int mrsb_get_sweep_launches(mrsb_handle h, int64_t* out, int32_t cap, int32_t* n_buckets) {
+  GUARD(h);
+  const int32_t nb = int32_t(h->buckets.size());
+  if (n_buckets) *n_buckets = nb;
+  if (!out || cap <= 0) return MRSB_OK;
+  std::vector<uint32_t> words(size_t(nb), 0u);
+  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaMemcpy(words.data(), h->buckets[0].sweep, sizeof(uint32_t) * size_t(nb), cudaMemcpyDeviceToHost));
+  for (int32_t b = 0; b < std::min(cap, nb); b++) out[b] = int64_t(words[size_t(b)] >> 16);  // each alternating launch adds 2^16
   return MRSB_OK;
 }
 

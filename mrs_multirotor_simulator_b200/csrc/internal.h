@@ -192,9 +192,11 @@ struct DevGrid {
 
 // kernel launchers (step_kernel.cu / collide.cu / io_kernels.cu); all return the number of launches made
 // uniform_params: host copy of THE parameter set when every local UAV uses the same one, else nullptr
+// sweep: the launch's own device word, zero at first use, whose parity sets the direction of the staged kernel's sweep; nullptr:
+// always forward (the staged kernel also sweeps forward when its launch streams less than L2 holds)
 // info[4] (may be nullptr): [0] variant launched — 1 direct (one CTA per tile), 2 staged (persistent CTAs + TMA); [1] grid;
 // [2] NM_T and [3] MODE_T of the instantiation
-int launch_step(const DevState& s, const DevParams* uniform_params, double dt, int k_substeps, int uniform_mode, int uniform_nm, bool any_moment,
+int launch_step(const DevState& s, const DevParams* uniform_params, uint32_t* sweep, double dt, int k_substeps, int uniform_mode, int uniform_nm, bool any_moment,
                 cudaStream_t stream, int* info);
 // DevParams::filt = exp(dt * neg_inv_tau) for every parameter set of the table
 int launch_prep_params(DevParams* params, int n_sets, double dt, cudaStream_t stream);

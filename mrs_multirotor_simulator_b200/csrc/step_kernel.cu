@@ -6,9 +6,9 @@
 #include "internal.h"
 
 template <int NM_T>
-void launch_step_nm(const DevState& s, const DevParams* uniform_params, double dt, int k_substeps, int uniform_mode, bool any_moment, cudaStream_t stream, int* info);
+void launch_step_nm(const DevState& s, const DevParams* uniform_params, uint32_t* sweep, double dt, int k_substeps, int uniform_mode, bool any_moment, cudaStream_t stream, int* info);
 
-int launch_step(const DevState& s, const DevParams* uniform_params, double dt, int k_substeps, int uniform_mode, int uniform_nm, bool any_moment,
+int launch_step(const DevState& s, const DevParams* uniform_params, uint32_t* sweep, double dt, int k_substeps, int uniform_mode, int uniform_nm, bool any_moment,
                 cudaStream_t stream, int* info) {
   int scratch[4];
   if (!info) info = scratch;
@@ -16,16 +16,16 @@ int launch_step(const DevState& s, const DevParams* uniform_params, double dt, i
   if (s.n <= 0) return 0;
   switch (uniform_nm) {
     case 4:
-      launch_step_nm<4>(s, uniform_params, dt, k_substeps, uniform_mode, any_moment, stream, info);
+      launch_step_nm<4>(s, uniform_params, sweep, dt, k_substeps, uniform_mode, any_moment, stream, info);
       break;
     case 6:
-      launch_step_nm<6>(s, uniform_params, dt, k_substeps, uniform_mode, any_moment, stream, info);
+      launch_step_nm<6>(s, uniform_params, sweep, dt, k_substeps, uniform_mode, any_moment, stream, info);
       break;
     case 8:
-      launch_step_nm<8>(s, uniform_params, dt, k_substeps, uniform_mode, any_moment, stream, info);
+      launch_step_nm<8>(s, uniform_params, sweep, dt, k_substeps, uniform_mode, any_moment, stream, info);
       break;
     default:
-      launch_step_nm<0>(s, uniform_params, dt, k_substeps, uniform_mode, any_moment, stream, info);
+      launch_step_nm<0>(s, uniform_params, sweep, dt, k_substeps, uniform_mode, any_moment, stream, info);
       break;
   }
   return 1;

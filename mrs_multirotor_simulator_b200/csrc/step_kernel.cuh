@@ -889,16 +889,30 @@ DEV void stage_tile(const DevState& s, const DevParams& P, double* sm, uint64_t*
 
 template <int NM_T, int MODE_T, bool ONE>
 __global__ void __launch_bounds__(MRSB_STEP_THREADS, MRSB_STEP_MINB(ONE, MODE_T))
-    uav_step_staged_kernel(DevState s, const __grid_constant__ DevParams params, double dt, double inv_dt, int k_sub, int any_moment, int64_t n_tiles) {
+    uav_step_staged_kernel(DevState s, const __grid_constant__ DevParams params, double dt, double inv_dt, int k_sub, int any_moment, int64_t n_tiles,
+                           uint32_t* sweep) {
   // `params`: the one parameter set of the whole batch, passed BY VALUE: it lives in the constant
   // bank, so airframe constants and gains are instruction operands instead of ~80 loads per UAV
   using I = Img<NM_T, MODE_T>;
   extern __shared__ __align__(128) double sm[];  // I::ROWS x 128 doubles (tile image) [+ PID_ROWS x 128: PID parking, K > 1]
   __shared__ uint64_t bar;
-  if (threadIdx.x == 0) mbar_init(&bar, 1);
+  __shared__ uint32_t ticket;
+  if (threadIdx.x == 0) {
+    mbar_init(&bar, 1);
+    // `sweep` (nullptr: always forward): every other launch walks the tiles from the end, so that it starts on those the previous
+    // launch wrote last, while their lines are still in L2.  The word lives on the device because a captured tick graph replays the
+    // same launch.  Each launch adds exactly 2^16 to it (CTA 0 adds 2^16 - (gridDim.x - 1), every other CTA 1), so whatever value
+    // a CTA's add returns, its bit 16 is the parity of the launch — one atomic per CTA, nothing to wait for at the end.
+    ticket = sweep ? atomicAdd(sweep, blockIdx.x == 0 ? 65536u - (gridDim.x - 1u) : 1u) : 0u;
+  }
   __syncthreads();
-  int64_t tile = blockIdx.x;
-  if (threadIdx.x == 0 && tile < n_tiles) stage_tile<NM_T, MODE_T>(s, params, sm, &bar, tile);
+  // a CTA's k-th tile is blockIdx.x + k * gridDim.x, counted from the end on a backward sweep; tiles outside [0, n_tiles) end the
+  // sweep.  The step is re-read from shared memory where it is needed rather than kept in a register across step_uav, whose live
+  // set is what limits the register budget.
+  const auto stride   = [&] { return ((*reinterpret_cast<volatile uint32_t*>(&ticket) >> 16) & 1u) ? -int64_t(gridDim.x) : int64_t(gridDim.x); };
+  const auto in_range = [&](int64_t t) { return uint64_t(t) < uint64_t(n_tiles); };
+  int64_t    tile     = ((ticket >> 16) & 1u) ? n_tiles - 1 - blockIdx.x : int64_t(blockIdx.x);
+  if (threadIdx.x == 0 && in_range(tile)) stage_tile<NM_T, MODE_T>(s, params, sm, &bar, tile);
   TileIn in;
   in.st   = sm + I::ST * MRSB_TILE + threadIdx.x;
   in.rpm  = sm + I::RPM * MRSB_TILE + threadIdx.x;
@@ -908,19 +922,19 @@ __global__ void __launch_bounds__(MRSB_STEP_THREADS, MRSB_STEP_MINB(ONE, MODE_T)
   uint32_t phase = 0;
   // the per-UAV word that is not part of the tile image is prefetched one tile ahead
   int64_t  i0        = min(tile * MRSB_TILE + threadIdx.x, s.n - 1);
-  uint32_t flags_cur = tile < n_tiles ? s.flags[i0] : 0u;
+  uint32_t flags_cur = in_range(tile) ? s.flags[i0] : 0u;
   uint32_t disp_bits = 0u;
-  for (; tile < n_tiles; tile += gridDim.x) {
-    const int64_t next = tile + gridDim.x;
+  for (; in_range(tile); tile += stride()) {
+    const int64_t next       = tile + stride();
     uint32_t      flags_next = 0u;
-    if (next < n_tiles) flags_next = s.flags[min(next * MRSB_TILE + threadIdx.x, s.n - 1)];
+    if (in_range(next)) flags_next = s.flags[min(next * MRSB_TILE + threadIdx.x, s.n - 1)];
     mbar_wait(&bar, phase);
     phase ^= 1u;
     step_uav<NM_T, MODE_T, ONE>(
         s, in, tile, flags_cur, &params, 0, dt, inv_dt, k_sub, any_moment, disp_bits,
         [&] {
           __syncthreads();  // every lane has its inputs in registers: the image may be overwritten
-          if (threadIdx.x == 0 && next < n_tiles) stage_tile<NM_T, MODE_T>(s, params, sm, &bar, next);
+          if (threadIdx.x == 0 && in_range(next)) stage_tile<NM_T, MODE_T>(s, params, sm, &bar, next);
         },
         ONE ? nullptr : sm + I::ROWS * MRSB_TILE);
     flags_cur = flags_next;
@@ -948,8 +962,20 @@ int staged_grid(size_t smem) {
   return cached;
 }
 
+// L2 size of the current device, cached
+inline int64_t l2_bytes() {
+  static int64_t cached = -1;
+  if (cached < 0) {
+    int dev = 0, bytes = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&bytes, cudaDevAttrL2CacheSize, dev);
+    cached = bytes;
+  }
+  return cached;
+}
+
 template <int NM_T, int MODE_T>
-void launch_one(const DevState& s, const DevParams* uniform_params, double dt, int k, int any_moment, cudaStream_t st, int* info) {
+void launch_one(const DevState& s, const DevParams* uniform_params, uint32_t* sweep, double dt, int k, int any_moment, cudaStream_t st, int* info) {
   const int     threads = MRSB_STEP_THREADS;
   const int64_t n_tiles = (s.n + threads - 1) / threads;
   const double  inv_dt  = 1.0 / dt;
@@ -963,7 +989,10 @@ void launch_one(const DevState& s, const DevParams* uniform_params, double dt, i
       const size_t   smem = size_t(Img<NM_T, MODE_T>::ROWS + (kOne ? 0 : PID_ROWS)) * MRSB_TILE * sizeof(double);  // tile image (+ PID parking rows, K > 1)
       const int      grid = staged_grid<NM_T, MODE_T, kOne>(smem);
       if (grid <= 0 || n_tiles <= grid) return false;
-      uav_step_staged_kernel<NM_T, MODE_T, kOne><<<grid, threads, smem, st>>>(s, *uniform_params, dt, inv_dt, k, any_moment, n_tiles);
+      // alternating the direction pays only when the launch streams more than L2 holds: a smaller state stays resident either way
+      const int64_t streamed = n_tiles * int64_t(Img<NM_T, MODE_T>::ROWS) * MRSB_TILE * int64_t(sizeof(double));
+      uint32_t*     dir      = streamed > l2_bytes() ? sweep : nullptr;
+      uav_step_staged_kernel<NM_T, MODE_T, kOne><<<grid, threads, smem, st>>>(s, *uniform_params, dt, inv_dt, k, any_moment, n_tiles, dir);
       info[0] = 2;
       info[1] = grid;
       return true;
@@ -980,22 +1009,22 @@ void launch_one(const DevState& s, const DevParams* uniform_params, double dt, i
 }
 
 template <int NM_T>
-void launch_nm(const DevState& s, const DevParams* up, double dt, int k, int mode, int any_moment, cudaStream_t st, int* info) {
+void launch_nm(const DevState& s, const DevParams* up, uint32_t* sweep, double dt, int k, int mode, int any_moment, cudaStream_t st, int* info) {
   switch (mode) {
     case MRSB_ACTUATOR_CMD:
-      launch_one<NM_T, MRSB_ACTUATOR_CMD>(s, up, dt, k, any_moment, st, info);
+      launch_one<NM_T, MRSB_ACTUATOR_CMD>(s, up, sweep, dt, k, any_moment, st, info);
       break;
     case MRSB_VELOCITY_HDG_RATE_CMD:
-      launch_one<NM_T, MRSB_VELOCITY_HDG_RATE_CMD>(s, up, dt, k, any_moment, st, info);
+      launch_one<NM_T, MRSB_VELOCITY_HDG_RATE_CMD>(s, up, sweep, dt, k, any_moment, st, info);
       break;
     case MRSB_VELOCITY_HDG_CMD:
-      launch_one<NM_T, MRSB_VELOCITY_HDG_CMD>(s, up, dt, k, any_moment, st, info);
+      launch_one<NM_T, MRSB_VELOCITY_HDG_CMD>(s, up, sweep, dt, k, any_moment, st, info);
       break;
     case MRSB_POSITION_CMD:
-      launch_one<NM_T, MRSB_POSITION_CMD>(s, up, dt, k, any_moment, st, info);
+      launch_one<NM_T, MRSB_POSITION_CMD>(s, up, sweep, dt, k, any_moment, st, info);
       break;
     default:
-      launch_one<NM_T, -1>(s, up, dt, k, any_moment, st, info);
+      launch_one<NM_T, -1>(s, up, sweep, dt, k, any_moment, st, info);
       break;
   }
 }
@@ -1005,7 +1034,7 @@ void launch_nm(const DevState& s, const DevParams* up, double dt, int k, int mod
 // one translation unit per motor count (step_kernel_nm{0,4,6,8}.cu) instantiates this, so that the
 // ~40 kernel instantiations compile in parallel
 template <int NM_T>
-void launch_step_nm(const DevState& s, const DevParams* uniform_params, double dt, int k_substeps, int uniform_mode, bool any_moment, cudaStream_t stream,
-                    int* info) {
-  launch_nm<NM_T>(s, uniform_params, dt, k_substeps, uniform_mode, any_moment, stream, info);
+void launch_step_nm(const DevState& s, const DevParams* uniform_params, uint32_t* sweep, double dt, int k_substeps, int uniform_mode, bool any_moment,
+                    cudaStream_t stream, int* info) {
+  launch_nm<NM_T>(s, uniform_params, sweep, dt, k_substeps, uniform_mode, any_moment, stream, info);
 }
