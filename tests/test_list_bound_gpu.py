@@ -1,0 +1,530 @@
+"""The neighbour lists' rebuild decision pinned exactly, and results exact where the bound is tight.
+
+Every pass is predicted on the host (list_bound_ref.py) from the positions downloaded before and after every stepping launch,
+and the pass' rebuild flag must EQUAL the prediction: a bound looser than the kernels' arithmetic (lists kept too long) and a
+tighter one (padding slots or frozen UAVs adding displacement: rebuilds too often) both fail.  This is checked on the staged
+kernel at a size larger than L2 with both sweep directions and fused K = 10 launches, on the direct and the per-UAV-mode
+kernels, on bucketed and unbucketed mixed batches, with UAVs frozen by iterate_without_input, through mrsb_run's tick graph,
+across forced rebuilds and NaN UAVs, and at cell edges 3.5, 6 and 12 m.
+
+Then pairs of large UAVs (contact distance above sqrt(3), so nanoflann's ball binds) fly head-on from spawn separations that
+straddle the list radius, everybody else hovering, so that the pairs set the swarm's displacement bound and close at nearly
+2 D per pass: pairs, forces and crash flags equal the full pass every tick (MRSB_NO_NEIGHBOUR_LISTS=1), and the run is shown to
+have reached the edge of the bound."""
+import math
+import os
+import subprocess
+import sys
+
+import numpy as np
+import pytest
+
+import list_bound_ref as R
+from helpers import rand
+from oracle import binding as O
+from test_collisions_gpu import ENGINE, _row_hash, af, geometry, sorted_pairs
+
+pytestmark = pytest.mark.gpu
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+BIG = 4096 * 128 + 9  # as test_sweep_gpu.py: 4097 tiles (the last holds 9 UAVs), more tile images than L2 holds
+SQRT3 = math.sqrt(3.0)
+ENV = ("MRSB_NO_STAGING", "MRSB_NO_BUCKETS", "MRSB_COLLISION_CELL", "MRSB_TIMELINE", "MRSB_NO_NEIGHBOUR_LISTS")
+
+
+def make(types, spawn, tou=None, **env):
+    """A handle created under the given MRSB_* settings, which are read at creation (MRSB_NO_STAGING is also read per launch:
+    test_direct_kernel keeps it set while it steps)."""
+    from mrs_multirotor_simulator_b200 import UavBatch
+
+    old = {k: os.environ.pop(k, None) for k in ENV}
+    try:
+        for k, v in env.items():
+            os.environ[k] = str(v)
+        return UavBatch(types, type_of_uav=tou, spawn_xyz=spawn, n=len(spawn))
+    finally:
+        for k in ENV:
+            os.environ.pop(k, None)
+            if old[k] is not None:
+                os.environ[k] = old[k]
+
+
+def grid(n, pitch, z=20.0):
+    side = int(np.ceil(np.sqrt(n)))
+    i = np.arange(n)
+    return np.stack([pitch * (i % side), pitch * (i // side), np.full(n, z)], axis=1).astype(np.float64)
+
+
+def velocity_cmd(n, seed, speed=2.0):
+    return np.stack([rand(seed, 1, n, -speed, speed), rand(seed, 2, n, -speed, speed), rand(seed, 3, n, -0.5, 0.5), rand(seed, 4, n, -1, 1)], axis=1)
+
+
+def xof(b):
+    return b.get_state(fields=("x",))["x"]
+
+
+class Watch:
+    """A handle whose every collision pass is predicted by the host reference and checked against the rebuild count."""
+
+    def __init__(self, b):
+        self.b = b
+        info = b.collision_info()
+        assert info["neighbour_lists"], info
+        self.host = R.HostSide(info["skin"])
+        self.skin = info["skin"]
+        self.rebuilds = info["rebuilds"]
+        self.x = xof(b)
+        self.flags = []  # per pass: rebuilt
+        self.forced = []  # per pass: forced by the host
+        self.words = []  # per pass: the displacement word of its launch (0 without one)
+
+    def step(self, dt=0.01, k=1):
+        self.b.make_step(dt, k)
+        x = xof(self.b)
+        self.host.launch(R.disp_bits(self.x, x))
+        self.x = x
+
+    def set_state(self, idx, **kw):
+        self.b.set_state(idx=np.asarray(idx, dtype=np.int32), **kw)
+        if kw.get("x") is not None:
+            self.host.touch()
+        self.x = xof(self.b)
+
+    def collide(self):
+        self.forced.append(self.host.touched or self.host.launches != 1)
+        self.words.append(self.host.bits)
+        want = self.host.collide()
+        self.b.handle_collisions()
+        r = self.b.collision_info()["rebuilds"]
+        got, self.rebuilds = r - self.rebuilds, r
+        self.flags.append(bool(got))
+        assert got == int(want), f"pass {len(self.flags) - 1}: {'rebuilt' if got else 'kept the lists'}, the reference says otherwise " \
+                                 f"(D before the pass {self.host.bound.D!r}, skin {self.skin!r})"
+        return want
+
+    def tick(self, dt=0.01, k=1):
+        self.step(dt, k)
+        return self.collide()
+
+    def assert_both_ways(self, min_kept=1, min_rebuilt=1):
+        """Unforced passes must have gone both ways: lists kept, and rebuilt because the bound ran out."""
+        kept = sum(1 for f, r in zip(self.forced, self.flags) if not f and not r)
+        rebuilt = sum(1 for f, r in zip(self.forced, self.flags) if not f and r)
+        assert kept >= min_kept and rebuilt >= min_rebuilt, (kept, rebuilt)
+
+
+def flight(w, passes, cmd, k=1, flip_every=0):
+    """`passes` ticks from the commanded velocity (given through set_state(v=...), which forces no rebuild); with flip_every,
+    the commands change sign every flip_every ticks (paths that turn inside a launch)."""
+    w.b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd)
+    w.set_state(np.arange(len(cmd)), v=np.concatenate([cmd[:, :2], cmd[:, 2:3]], axis=1))
+    for t in range(passes):
+        if flip_every and t % flip_every == 0:
+            w.b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd * (-1.0 if (t // flip_every) % 2 else 1.0))
+        w.tick(0.01, k)
+
+
+# ---- the decision, exactly -----------------------------------------------------------------------------------------------------
+
+
+@pytest.mark.parametrize("k", [1, 10])
+def test_staged_kernel_larger_than_l2_both_sweep_directions(k):
+    """BIG x500 on the staged kernel: a partial last tile, a tile count that does not divide the persistent grid, the sweep
+    alternating every launch.  K = 10: the bound is measured from the start of the fused launch; commands flip sign every 3
+    ticks, so that many paths turn inside a launch (end minus start differs from the last substep's displacement)."""
+    n = BIG
+    b = make([af("x500")], grid(n, 4.0))
+    b.set_collisions(True, False, 100.0)
+    b.set_pair_capacity(4 * n)
+    cmd = velocity_cmd(n, 7, 3.0)
+    w = Watch(b)
+    flight(w, 40 if k == 1 else 24, cmd, k, flip_every=0 if k == 1 else 3)
+    info = b.step_info()
+    assert info["variant"] == "staged", info
+    assert b.sweep_launches() == [len(w.flags)]  # every launch alternated: both directions reported displacement
+    w.assert_both_ways(min_kept=5 if k == 1 else 2, min_rebuilt=2)
+    b.close()
+
+
+def test_direct_kernel():
+    n = 128 * 150 + 77
+    os.environ["MRSB_NO_STAGING"] = "1"
+    try:
+        b = make([af("x500")], grid(n, 3.0))
+        b.set_collisions(True, False, 100.0)
+        b.set_pair_capacity(4 * n)
+        w = Watch(b)
+        flight(w, 40, velocity_cmd(n, 9, 3.0))
+        assert b.step_info()["variant"] == "direct"
+    finally:
+        os.environ.pop("MRSB_NO_STAGING", None)
+    w.assert_both_ways(5, 2)
+
+
+def test_per_uav_mode_kernel():
+    """Half the UAVs on velocity commands, the other half on position commands: the kernel that reads each UAV's mode."""
+    n = 128 * 120 + 5
+    x0 = grid(n, 3.0)
+    b = make([af("x500")], x0)
+    b.set_collisions(True, False, 100.0)
+    b.set_pair_capacity(4 * n)
+    half = np.arange(0, n, 2, dtype=np.int32)
+    rest = np.arange(1, n, 2, dtype=np.int32)
+    vcmd = velocity_cmd(len(half), 10, 3.0)
+    b.set_input(O.VELOCITY_HDG_RATE_CMD, vcmd, idx=half)
+    b.set_input(O.POSITION_CMD, np.concatenate([x0[rest] + rand(11, 0, len(rest), -1.5, 1.5)[:, None], rand(11, 1, len(rest), -1, 1)[:, None]], axis=1),
+                idx=rest)
+    w = Watch(b)
+    w.set_state(half, v=vcmd[:, :3])
+    for _ in range(40):
+        w.tick()
+    assert b.step_info()["mode"] == -1, b.step_info()
+    w.assert_both_ways(5, 2)
+
+
+@pytest.mark.parametrize("bucketed", [True, False])
+def test_mixed_airframes(bucketed):
+    """x500 / f550 / naki interleaved.  Bucketed: one launch per bucket into one word, each bucket padded to whole tiles — padding
+    slots must not contribute.  Unbucketed (MRSB_NO_BUCKETS=1): one launch of the kernel that reads the motor count per UAV."""
+    n = 3 * 20001
+    tou = (np.arange(n) % 3).astype(np.int32)
+    frames = [af("x500"), af("f550"), af("naki")]
+    b = make(frames, grid(n, 3.0), tou, **({} if bucketed else {"MRSB_NO_BUCKETS": 1}))
+    b.set_collisions(True, False, 100.0)
+    b.set_pair_capacity(4 * n)
+    w = Watch(b)
+    flight(w, 40, velocity_cmd(n, 12, 3.0))
+    info = b.step_info()
+    assert len(b.sweep_launches()) == (3 if bucketed else 1)
+    assert (info["n_motors"] > 0) == bucketed, info  # per bucket: a motor count of its own; unbucketed: read per UAV
+    w.assert_both_ways(5, 2)
+
+
+def test_frozen_uavs_add_nothing():
+    """iterate_without_input(False): a third of the UAVs never get a command but are given 6 m/s through set_state(v=...) — they
+    would move if they were stepped.  The rest hover; with a 3.5 m cell the skin is 1.8 cm, so a few millimetres of spurious
+    displacement per pass (from the frozen UAVs or from the lanes past the last partial tile) changes the decisions."""
+    n = 128 * 40 + 9
+    b = make([af("x500")], grid(n, 5.0), MRSB_COLLISION_CELL=3.5)
+    b.set_collisions(True, False, 100.0)
+    b.set_iterate_without_input(False)
+    frozen = np.arange(0, n, 3, dtype=np.int32)
+    live = np.setdiff1d(np.arange(n), frozen).astype(np.int32)
+    w = Watch(b)
+    w.set_state(np.arange(n), v=np.tile([6.0, -3.0, 1.0], (n, 1)))  # velocity alone: no forced rebuild
+    x0 = xof(b)
+    for _ in range(30):  # nobody commanded: nothing moves, the bound stays exactly zero and the first lists live on
+        w.tick()
+    assert np.array_equal(xof(b), x0) and w.words == [0] * 30 and w.flags == [True] + [False] * 29
+    b.set_input(O.VELOCITY_HDG_RATE_CMD, np.zeros((len(live), 4)), idx=live)
+    x_frozen = xof(b)[frozen]
+    for _ in range(60):
+        w.tick()
+    assert np.array_equal(xof(b)[frozen], x_frozen)  # really frozen
+    assert not any(w.forced[1:])
+    assert sum(w.flags[31:]) >= 2
+    # and the commanded ones start to move: the bound must follow them, not the frozen ones
+    b.set_input(O.VELOCITY_HDG_RATE_CMD, np.tile([0.3, 0.0, 0.0, 0.0], (len(live), 1)), idx=live)
+    for _ in range(40):
+        w.tick()
+    assert np.array_equal(xof(b)[frozen], x_frozen)
+    w.assert_both_ways(20, 3)
+
+
+@pytest.mark.parametrize("calls", [(9, 14), (24,)])
+def test_tick_graph(calls):
+    """mrsb_run, several ticks per call (the tick captured as one graph with the pass' conditional rebuild): its per-pass flags
+    (timeline column 5) equal the prediction made from a twin driven tick by tick, whose positions equal the graph's."""
+    n = BIG
+    spawn = grid(n, 4.0)
+    cmd = velocity_cmd(n, 13, 3.0)
+    g = make([af("x500")], spawn, MRSB_TIMELINE=1)
+    t = make([af("x500")], spawn)
+    for b in (g, t):
+        b.set_collisions(True, False, 100.0)
+        b.set_pair_capacity(4 * n)
+        b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd)
+        b.set_state(v=cmd[:, :3])
+    g.make_step(0.01)
+    g.handle_collisions()
+    w = Watch(t)
+    w.tick()
+    for c in calls:
+        g.run(0.01, c, 1, True)
+        for _ in range(c):
+            w.tick()
+        assert np.array_equal(xof(g), w.x)
+    flags = [bool(r) for r in g.timeline()[:, 5]]
+    assert flags == w.flags, (flags, w.flags)
+    assert g.collision_info()["rebuilds"] == t.collision_info()["rebuilds"]
+    w.assert_both_ways(3, 1)
+    assert np.array_equal(g.get_collision_pairs(), t.get_collision_pairs())
+
+
+@pytest.mark.parametrize("cell", [3.5, 6.0, 12.0])
+def test_forced_rebuilds_nan_and_cell_sizes(cell):
+    """A crowd (12 m: many UAVs with more candidates than a list holds) at each cell edge, with every host-forced case: a pass
+    without a step, two launches per pass, set_state(x=...), set_state(v=...) alone (not forced), and a NaN UAV that rebuilds
+    every pass until set_state repairs it."""
+    n = 128 * 60 + 33
+    pitch = 1.5 if cell == 12.0 else 2.5
+    b = make([af("x500")], grid(n, pitch), MRSB_COLLISION_CELL=cell)
+    assert b.collision_info()["cell"] == cell
+    b.set_collisions(True, False, 100.0)
+    b.set_pair_capacity(40 * n)
+    cmd = velocity_cmd(n, 14, {3.5: 0.3, 6.0: 2.0, 12.0: 4.0}[cell])
+    b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd)
+    w = Watch(b)
+    w.set_state(np.arange(n), v=cmd[:, :3])
+    for _ in range(50 if cell == 12.0 else 30):
+        w.tick()
+    w.collide()  # no step
+    assert w.forced[-1] and w.flags[-1]
+    w.step()
+    w.step()
+    w.collide()  # two launches
+    assert w.forced[-1] and w.flags[-1]
+    for _ in range(5):
+        w.tick()
+    w.set_state([3, 4], v=np.array([[1.0, 0.0, 0.0], [0.0, -1.0, 0.0]]))
+    w.tick()
+    assert not w.forced[-1]
+    w.set_state([7], x=w.x[[7]] + 0.05)
+    w.collide()  # teleport, no step
+    w.set_state([8], x=w.x[[8]] - 0.05)
+    w.tick()  # teleport, then one step
+    assert w.forced[-2:] == [True, True] and w.flags[-2:] == [True, True]
+    for _ in range(5):
+        w.tick()
+    w.set_state([11], x=np.array([[math.nan, 0.0, 20.0]]))
+    for _ in range(4):
+        w.tick()
+    assert w.flags[-4:] == [True] * 4 and not any(w.forced[-3:])  # NaN displacement: every pass rebuilds
+    w.set_state([11], x=np.array([[-50.0, -50.0, 20.0]]))
+    for _ in range(40 if cell == 12.0 else 20):
+        w.tick()
+    assert not all(w.flags[-19:])  # repaired: lists live again
+    w.assert_both_ways(5, 1)
+    if cell == 12.0:
+        assert b.collision_info()["crowded_uavs"] > 100
+
+
+def skin_of_cell(cell):
+    """api.cu, set_collision_geometry, in the same double operations"""
+    r_list = (0.5 * cell) * (1.0 - 1e-6)
+    return (r_list - 1.7320508075688775) * (1.0 - 1e-6)
+
+
+def test_skin_between_the_round_up_and_the_round_down():
+    """The decision where the direction of every rounding shows: a first flight learns the displacement words; the cell edge of
+    a second, identical flight is then chosen (MRSB_COLLISION_CELL takes any double) so that 2 D of one pass lies one float32 ulp
+    of its word away from the skin — rounded up the pass must rebuild, rounded down it would keep the lists."""
+    n = 128 * 8 + 9
+    spawn = grid(n, 8.0)
+    cmd = velocity_cmd(n, 21, 2.0)
+
+    def fly(**env):
+        b = make([af("x500")], spawn, **env)
+        b.set_collisions(True, False, 100.0)
+        w = Watch(b)
+        flight(w, 30, cmd)
+        assert len(b.get_collision_pairs()) == 0  # no contact: the cell edge cannot change the flight
+        return w
+
+    first = fly()
+    assert first.flags[0] and not any(first.forced[1:])
+    end = first.flags.index(True, 1) if any(first.flags[1:]) else len(first.flags)  # the first lists' last pass + 1
+    words = first.words
+    target = None
+    for p in range(5, end):  # the first pass whose D is large enough for a cell edge of at least 3.5 m
+        d_up = d_down = 0.0
+        for q in range(1, p + 1):
+            d_up = R.add_ru(d_up, R.sqrt_ru(R.bits_f32(words[q])))
+            d_down = R.add_ru(d_down, R.sqrt_ru(R.bits_f32(words[q] - 1)))  # a word rounded down: one float32 ulp below
+        lo, hi = R.mul_ru(2.0, d_down), R.mul_ru(2.0, d_up)
+        if lo > skin_of_cell(3.5) and lo < hi:
+            target = (p, lo, hi)
+            break
+    assert target is not None
+    p, lo, hi = target
+    cell = 2.0 * (lo / (1.0 - 1e-6) + 1.7320508075688775) / (1.0 - 1e-6)
+    while skin_of_cell(cell) >= hi:
+        cell = math.nextafter(cell, 0.0)
+    while skin_of_cell(cell) < lo:
+        cell = math.nextafter(cell, math.inf)
+    assert lo <= skin_of_cell(cell) < hi
+    second = fly(MRSB_COLLISION_CELL=repr(cell))
+    assert second.skin == skin_of_cell(cell)
+    assert np.array_equal(second.x, first.x) and second.words == words
+    assert second.flags[:p + 1] == [True] + [False] * (p - 1) + [True], second.flags
+
+
+# ---- head-on approaches at the list radius ---------------------------------------------------------------------------------------
+
+
+def big_airframe():
+    return af("x500", arm_length=1.2, prop_radius=0.45)  # contact threshold ((1.2 + 0.45) + 1.2) + 0.45 = 3.3 > 3: sqrt(3) binds
+
+
+def head_on_layout(cell, n_buckets, r_list):
+    """Spawn positions, per-UAV velocity commands and the list of approaching pairs.  Pairs sit along x, 14 m apart in y, at
+    separations straddling r_list by ulps and millimetres; pairs further in (contact on a list-only pass); a pair with a crowd
+    around one UAV; pairs across a cell boundary and across the end of the bucket table."""
+    xyz, vel, pairs = [], [], []
+    speed = 0.5 if cell < 6.0 else 1.0  # per pass, well above what a hovering UAV still drifts
+
+    def pair(c, sep, axis_y=0.0):
+        a = len(xyz)
+        xyz.append([c[0] - sep / 2, c[1] + axis_y, c[2]])
+        xyz.append([xyz[-1][0] + sep, c[1] + axis_y, c[2]])
+        vel.extend([[speed, 0, 0, 0], [-speed, 0, 0, 0]])
+        pairs.append((a, a + 1))
+
+    ulp = math.ulp(r_list)
+    seps = [r_list + k * ulp for k in (-4, -1, 0, 1, 4)] + [r_list + mm * 1e-3 for mm in (-5, -2, -1, 1, 2, 3, 5, 8)]
+    # outside the lists at the first rebuild, inside them at the second, and in contact after closing more than half the skin
+    # since then (a pair that touched earlier would be thrown apart by the rebounce, outrunning the pairs that set the bound)
+    seps += [SQRT3 + f * (r_list - SQRT3) for f in (1.5, 1.6, 1.7, 1.8)]
+    row = 0
+    for s in seps:
+        pair((20.0, 14.0 * row + 7.0, 10.0), s)
+        row += 1
+    # one UAV of a pair crowded: 9 hovering UAVs on a ring 2.6 m around it, away from its partner (with the partner, more
+    # candidates than a list holds within a 3 m list radius)
+    for s in (r_list + 0.002, SQRT3 + 1.6 * (r_list - SQRT3)):
+        pair((20.0, 14.0 * row + 7.0, 10.0), s)
+        bx = list(xyz[-1])
+        for k in (0, 1, 2, 3, 4, 8, 9, 10, 11):
+            ang = math.pi * k / 6
+            xyz.append([bx[0] + 2.5 * math.cos(ang), bx[1] + 2.5 * math.sin(ang), bx[2] + (0.8 if k % 2 else -0.8)])
+            vel.append([0, 0, 0, 0])
+        row += 1
+    # across a cell boundary (x = 4 cells) at a few separations
+    for s in (r_list + 0.001, r_list - 0.001, SQRT3 + 1.6 * (r_list - SQRT3)):
+        pair((4 * cell, 14.0 * row + 7.0 + 0.3, 10.0), s)
+        row += 1
+    # across the end of the bucket table: cells cx, cx + 1 with buckets B - 1 and 0 (as test_collisions_gpu.py aims at it)
+    hits = []
+    for cy in range(-60, 0):
+        for cz in range(0, 3):
+            cx = (n_buckets - 1 - _row_hash(cy, cz)) % n_buckets
+            if cx < 400:
+                hits.append((cx, cy, cz))
+    assert len(hits) >= 3
+    for (cx, cy, cz), s in zip(hits[:3], (r_list + 0.001, r_list - 0.0005, SQRT3 + 1.7 * (r_list - SQRT3))):
+        pair((cell * (cx + 1), cell * cy + 0.5 * cell, cell * cz + 0.5 * cell), s)
+    return np.array(xyz), np.array(vel, dtype=np.float64), pairs
+
+
+@pytest.mark.parametrize("cell,crash", [(3.5, False), (6.0, False), (3.5, True), (6.0, True)])
+def test_head_on_pairs_at_the_list_radius(cell, crash):
+    settle = 150
+    t0 = big_airframe()
+    probe_n = 128
+    n_buckets = None
+    # the layout depends on the table size, which depends on n: fix n first with a throw-away layout, then read the table size
+    for _ in range(2):
+        probe = make([t0], np.zeros((probe_n, 3)) + np.arange(probe_n)[:, None] * 10.0, MRSB_COLLISION_CELL=cell)
+        info = probe.collision_info()
+        probe.close()
+        if n_buckets == info["n_buckets"]:
+            break
+        n_buckets = info["n_buckets"]
+        xyz, vel, pairs = head_on_layout(cell, n_buckets, info["list_radius"])
+        probe_n = len(xyz)
+    r_list, skin = info["list_radius"], info["skin"]
+    n = len(xyz)
+    tou = np.zeros(n, dtype=np.int32)
+    a = make([t0], xyz, MRSB_COLLISION_CELL=cell)
+    f = make([t0], xyz, MRSB_COLLISION_CELL=cell, MRSB_NO_NEIGHBOUR_LISTS=1)
+    assert a.collision_info()["n_buckets"] == n_buckets and a.collision_info()["list_radius"] == r_list
+    assert not f.collision_info()["neighbour_lists"]
+    for b in (a, f):
+        b.set_collisions(True, crash, 100.0)
+        b.set_pair_capacity(n * n)
+        b.set_input(O.VELOCITY_HDG_RATE_CMD, np.zeros((n, 4)))
+    arm, prop, mass = geometry([t0], tou)
+    w = Watch(a)
+    P = np.array(pairs)
+    passes = 200 if cell == 6.0 else 120
+    sep_hist, contact_hist = [], []
+    for t in range(-settle, passes):
+        if t == 0:
+            # everybody has settled into hover (a fresh UAV sags first, by more than the pairs will move per pass): put every UAV
+            # back on its spawn position — the next pass is a forced rebuild at the spawn separations — and start the approach
+            w.set_state(np.arange(n), x=xyz)
+            f.set_state(idx=np.arange(n, dtype=np.int32), x=xyz)
+            for b in (a, f):
+                b.set_input(O.VELOCITY_HDG_RATE_CMD, vel)
+        w.step()
+        f.make_step(0.01)
+        w.collide()
+        f.handle_collisions()
+        pa, pf = a.get_collision_pairs(), f.get_collision_pairs()
+        assert np.array_equal(pa, pf), f"pass {t}: pairs differ from the full pass"
+        assert np.array_equal(a.get_force(), f.get_force()), f"pass {t}: forces"
+        assert np.array_equal(a.has_crashed(), f.has_crashed()), f"pass {t}: crash flags"
+        x = w.x
+        assert np.array_equal(x, xof(f)), f"pass {t}: positions"
+        if t % 20 == 0 or t == -1:
+            ref_pairs, ref_forces, _ = O.collide_snapshot(x, arm, prop, mass, crash, 100.0, engine=ENGINE, cap=n * n)
+            assert np.array_equal(sorted_pairs(ref_pairs), pa), f"pass {t}: pairs differ from {ENGINE}"
+        if t < 0:
+            continue
+        if t == 0:
+            crowded = a.collision_info()["crowded_uavs"]
+        sep_hist.append(np.linalg.norm(x[P[:, 0]] - x[P[:, 1]], axis=1))
+        pset = set(map(tuple, pa.tolist()))
+        contact_hist.append(np.array([(i, j) in pset for i, j in pairs]))
+    sa, sf = a.get_full_state(), f.get_full_state()
+    for key in sa:
+        assert np.array_equal(sa[key], sf[key], equal_nan=True), key
+    # the edge was reached: (1) a pair entered contact on a list-only pass after closing at least half the skin since the last
+    # rebuild; (2) a pair outside every list at a rebuild came within 1.01 sqrt(3) before the next rebuild.  With a 6 m cell the
+    # UAVs' residual hover drift (a few mm per pass, in every direction) eats more than 1 % of sqrt(3) of a 1.27 m skin: there
+    # (2) asks for 90 % of the skin closed on list-only passes instead.
+    near = 1.01 * SQRT3 if cell < 6.0 else r_list - 0.9 * skin
+    flags = w.flags[settle:]
+    assert flags[0]
+    entered_late, entered_listed, crossed = 0, 0, 0
+    last = None
+    for t in range(passes):
+        if flags[t]:
+            if last is not None:
+                between = np.array(sep_hist[last + 1:t]) if t > last + 1 else np.zeros((0, len(pairs)))
+                if len(between):
+                    crossed += int(np.sum((sep_hist[last] > r_list) & (between.min(axis=0) < near)))
+            last = t
+            continue
+        if last is None:
+            continue
+        new = contact_hist[t] & ~contact_hist[t - 1]
+        closed = sep_hist[last] - sep_hist[t]
+        entered_late += int(np.sum(new & (closed >= skin / 2)))
+        entered_listed += int(np.sum(new))
+    rebuilt = sum(flags)
+    print(f"cell {cell} crash {crash}: {passes} passes, {rebuilt} rebuilds, {entered_listed} contacts begun on list-only passes, "
+          f"{entered_late} of them after closing half the skin, {crossed} crossings, skin {skin:.4f}")
+    # in crash mode the first contact crashes its pair, which then falls faster than anybody approaches: later contacts come on
+    # rebuild passes, so only "some contact began on a list-only pass" is asked there
+    assert crossed >= 1 and (entered_listed if crash else entered_late) >= 1, (entered_listed, entered_late, crossed, rebuilt)
+    assert 2 <= rebuilt < passes
+    if cell == 6.0:
+        assert crowded >= 2, crowded  # the rebuild at the spawn separations found the crowded UAVs
+    a.close()
+    f.close()
+
+
+# ---- sharded --------------------------------------------------------------------------------------------------------------------
+
+
+def test_sharded_bound_travels_through_the_hand_shake():
+    import torch
+
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    n = min(torch.cuda.device_count(), 4)
+    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={n}", "--master-addr", "127.0.0.1",
+                        "--master-port", "29547", os.path.join(ROOT, "tests", "list_bound_multi_gpu_check.py")], capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 0 and "LIST_BOUND_MULTI_GPU_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
