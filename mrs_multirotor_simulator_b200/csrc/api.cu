@@ -245,7 +245,6 @@ struct mrsb_sim {
   double*              gbuf[2]   = {nullptr, nullptr};
   uint32_t*            d_gbox[2] = {nullptr, nullptr};
   int64_t              pass_no   = 0;      // collision passes done so far (pull exchange)
-  bool                 wrote_since_pass = false;  // positions of buffer (pass_no + 1) & 1 are complete
   std::vector<int32_t> pending_geom[2];    // local indices whose geometry changed but is not yet in that buffer (-1 = all)
   PeerView             pv[2]{};            // what the kernels of a pass with parity k read
   PeerView             pv_local{};         // everything in this handle's own arrays
@@ -273,14 +272,20 @@ struct mrsb_sim {
   Graph pass[2], tick[2];
   bool  graph_failed = false;  // a capture failed (e.g. conditional nodes unavailable): no more graphs for this handle
 
+  // What the next collision pass may assume about the positions.  Written by stepped, positions_written and forces_written, reset
+  // by end_pass only.  The displacement word bounds them exactly when steps == 1 && !unbounded.
+  struct SincePass {
+    int  steps;      // stepping launches since the last pass
+    bool unbounded;  // something the word does not cover: host writes, forces, all-gather, no pass yet
+    bool written;    // the buffer being written holds current positions (pull exchange)
+  } since{0, true, false};
+
   // neighbour lists (single-shard handles)
   bool     lists_on            = false;
-  int      steps_since_pass    = 0;     // stepping launches since the last collision pass
-  bool     positions_touched   = true;  // positions were written by something else than ONE stepping launch
   int      rebuild_own         = 0;     // own kernels of one rebuild (for the launch counter)
   int64_t  list_passes         = 0;     // passes that went through decide_kernel (it counts them too: NlCtl::n_passes)
   int64_t  rebuilds_counted    = 0;
-  Mem<uint32_t, true> h_one;               // pinned constant 1 (source of the async "force rebuild" copy)
+  Mem<uint32_t, true> h_unbounded;         // pinned 0xFFFFFFFF: source of the async copy that raises NlCtl::disp_max_bits
   Mem<unsigned long long, true> h_until;   // pinned source of NlCtl::write_all_until (forces_written)
 
   // neighbour observations (mrsb_pack_neighbours_device): a table of its own, sized for n_local on the first call
@@ -631,6 +636,99 @@ static int repoint(mrsb_sim* h, int64_t n, const int32_t* idx, Edit edit, Key va
   return MRSB_OK;
 }
 
+// ---- the pass lifecycle: what the next collision pass may assume (mrsb_sim::since) ----------------------------------------
+// a stepping launch of k_substeps (on its own, or inside a tick graph)
+static void stepped(mrsb_sim* h, int32_t k_substeps) {
+  h->since.steps++;
+  h->since.written = true;
+  h->n_steps += k_substeps;
+}
+
+// Positions of local UAVs were written by something else than a stepping launch.  packed_current: the writer wrote the packed
+// positions too; if not, they are published here.  With the pull exchange they are published either way: the whole slice of the
+// buffer being written, and the per-group boxes the peers read.  device_signals: the writing kernel raised the displacement word
+// itself for the UAVs it moved (device masks: the host does not learn whom), so the next pass rebuilds only if it moved somebody.
+static int positions_written(mrsb_sim* h, bool packed_current, bool device_signals) {
+  if (!packed_current || h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);
+  h->since.written   = true;
+  h->since.unbounded = h->since.unbounded || !device_signals;
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
+// The next pass that goes through decide_kernel replaces every force it visits (SIM:356-358), not only the ones it knows to be
+// non-zero.  No host synchronisation: the copy reads the pinned word when it runs.  If a later call has raised the word by then,
+// more passes than needed write every force they visit, which writes the values they would have left in place.
+static int write_all_forces_next_pass(mrsb_sim* h) {
+  if (!h->grid.ctl) return MRSB_OK;
+  *h->h_until.get() = (unsigned long long)h->list_passes + 1ull;  // index of the next pass that goes through decide_kernel
+  CU(cudaMemcpyAsync(&h->grid.ctl->write_all_until, h->h_until.get(), sizeof(unsigned long long), cudaMemcpyHostToDevice, h->stream));
+  return MRSB_OK;
+}
+
+// forces were written by something else than the collision pass: the next pass must replace every UAV's force
+static int forces_written(mrsb_sim* h) {
+  int rc = write_all_forces_next_pass(h);
+  if (rc) return rc;
+  h->since.unbounded = true;  // that pass rebuilds: UAVs without candidates are only visited by a rebuild
+  return MRSB_OK;
+}
+
+// all-gather of the positions (sharded handles without the pull exchange)
+static int exchange_positions(mrsb_sim* h) {
+  if (h->n_ranks <= 1 || h->p2p) return MRSB_OK;  // pull exchange: nothing moves; the pass' first kernel hand-shakes
+  if (!h->comm) return fail(MRSB_ERR_STATE, "sharded handle (n_global > n_local) without a communicator: call mrsb_comm_init_nccl, or use mrsb_gather_buffer + mrsb_handle_collisions_gathered");
+  double* buf = h->ds.gpos;
+  if (h->equal_shards) {
+    NC(g_nccl.AllGather(buf + 3 * h->ds.shard_begin, buf, size_t(3 * h->ds.n), ncclDouble, h->comm, h->stream));
+  } else {
+    NC(g_nccl.GroupStart());
+    for (int r = 0; r < h->n_ranks; r++) {
+      double* p = buf + 3 * h->shard_begin_of[r];
+      NC(g_nccl.Broadcast(p, p, size_t(3 * h->shard_count_of[r]), ncclDouble, r, h->comm, h->stream));
+    }
+    NC(g_nccl.GroupEnd());
+  }
+  return positions_written(h, true, false);  // without the hand-shake there is no swarm-wide displacement bound for this pass
+}
+
+// Before every collision pass.  gathered: the caller put every shard's positions in place (mrsb_gather_buffer).  With neighbour
+// lists, a pass whose bound does not hold gets the displacement word raised to "unbounded": decide_kernel rebuilds (the word
+// decodes to NaN), and with the pull exchange the raised word reaches every peer through the hand-shake, so every rank rebuilds.
+static int begin_pass(mrsb_sim* h, bool gathered) {
+  int rc = flush_params(h);
+  if (rc) return rc;
+  if (!gathered) {
+    if (h->ds.n_global > h->ds.n && h->n_ranks <= 1) return fail(MRSB_ERR_STATE, "sharded handle without communicator");
+    rc = exchange_positions(h);
+    if (rc) return rc;
+  }
+  // nothing wrote positions since the last pass: the buffer this pass reads still holds the ones of two passes ago
+  if (h->p2p && !h->since.written) h->n_launches += launch_publish_positions(h->ds, h->stream);
+  if (!h->lists_on) return MRSB_OK;
+  if (h->since.unbounded || h->since.steps != 1)
+    CU(cudaMemcpyAsync(&h->grid.ctl->disp_max_bits, h->h_unbounded.get(), sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+  h->list_passes++;
+  return MRSB_OK;
+}
+
+// After every collision pass: the record starts afresh, and with the pull exchange the write buffer changes sides.
+static int end_pass(mrsb_sim* h) {
+  h->since = {0, false, false};
+  h->n_passes++;
+  if (h->p2p) {
+    h->pass_no++;
+    const int w = write_buf(h);
+    h->ds.gpos  = h->gbuf[w];
+    h->ds.gbox  = h->d_gbox[w];
+    h->ds.geom  = h->d_geom[w];
+    int rc      = apply_pending_geom(h, w);  // no peer reads this buffer any more (they have all started the pass that just ran)
+    if (rc) return rc;
+  }
+  CU(cudaGetLastError());
+  return MRSB_OK;
+}
+
 // Cell geometry of the spatial hash.  Handles that run the full pass every tick use the smallest cell
 // whose half covers the search radius sqrt(3) (4 m: fewest candidates).  Handles that keep neighbour
 // lists between rebuilds use a larger cell: the list radius is just under cell / 2, so a larger cell
@@ -645,8 +743,7 @@ static void set_collision_geometry(mrsb_sim* h, bool lists) {
   const double r_list = g.reach * (1.0 - 1e-6);
   g.list_r2  = r_list * r_list;
   g.skin     = (r_list - 1.7320508075688775) * (1.0 - 1e-6);
-  h->ds.disp_max       = lists ? &g.ctl->disp_max_bits : nullptr;
-  h->positions_touched = true;
+  h->ds.disp_max = lists ? &g.ctl->disp_max_bits : nullptr;
 }
 
 static void make_local_view(mrsb_sim* h) {
@@ -764,8 +861,8 @@ static int setup_p2p(mrsb_sim* h) {
   h->ds.gpos = h->gbuf[1];
   h->ds.gbox = h->d_gbox[1];
   h->ds.geom = h->d_geom[1];
-  h->n_launches += launch_publish_positions(h->ds, h->stream);
-  h->wrote_since_pass = true;
+  rc         = positions_written(h, false, false);
+  if (rc) return rc;
   // remote geometry is read from its owner from now on; the hand-shake also carries every rank's displacement bound, so
   // neighbour lists work across shards
   set_collision_geometry(h, h->grid.nl_count != nullptr);
@@ -1002,13 +1099,12 @@ int mrsb_create(const mrsb_create_info* info, mrsb_handle* out) {
     if (!rc && s.n_global > s.n) rc = dalloc(h, &g.halo_work, size_t(g.halo_cap / 32 + MRSB_MAX_RANKS + 1));
     if (!rc && getenv("MRSB_TIMELINE")) rc = dalloc(h, &g.tl, size_t(MRSB_TL_TICKS) * 8);
     if (!rc) rc = dalloc(h, &g.ctl, 1);
-    if (!rc) rc = h->h_one.alloc(2);
+    if (!rc) rc = h->h_unbounded.alloc(1);
     if (!rc) rc = h->h_until.alloc(1);
     if (rc) return rc;
     g.pairs       = h->pairs.get();
     g.halo_work_n = g.halo_n + 1;
-    h->h_one.get()[0] = 1u;
-    h->h_one.get()[1] = 0xFFFFFFFFu;  // "unbounded displacement"
+    *h->h_unbounded.get() = 0xFFFFFFFFu;
     // neighbour lists: single-shard handles now, sharded ones once the pull exchange is up (setup_p2p)
     if (s.n > 0 && !getenv("MRSB_NO_NEIGHBOUR_LISTS")) {
       g.nl_ld = s.ld;
@@ -1159,7 +1255,7 @@ int mrsb_get_positions_async(mrsb_handle h, double* out_xyz) {
   if (h->n_down >= 2) CU(cudaStreamWaitEvent(h->stream, h->ev_down[k], 0));  // the snapshot buffer was downloaded two reads ago
   if (!(h->ds.opts & STEP_OPT_GPOS)) return fail(MRSB_ERR_STATE, "packed positions are switched off (mrsb_set_outputs)");
   // pull exchange: the buffer being written holds the latest positions only once something wrote it since the last pass
-  const double* latest = (h->p2p && !h->wrote_since_pass) ? h->gbuf[h->pass_no & 1] : h->ds.gpos;
+  const double* latest = (h->p2p && !h->since.written) ? h->gbuf[h->pass_no & 1] : h->ds.gpos;
   if (h->n_sub) {
     h->n_launches += launch_gather_xyz(latest + 3 * h->ds.shard_begin, h->n_sub, h->d_sub_idx.get(), h->d_snap[k].get(), h->stream);
   } else {
@@ -1350,26 +1446,8 @@ int mrsb_clear_feedforward(mrsb_handle h, int64_t n, const int32_t* idx) {
 // ------------------------------------------------------------------------------------------
 // stepping
 // ------------------------------------------------------------------------------------------
-static int exchange_positions(mrsb_sim* h) {
-  if (h->n_ranks <= 1 || h->p2p) return MRSB_OK;  // pull exchange: nothing moves; the pass' first kernel hand-shakes
-  if (!h->comm) return fail(MRSB_ERR_STATE, "sharded handle (n_global > n_local) without a communicator: call mrsb_comm_init_nccl, or use mrsb_gather_buffer + mrsb_handle_collisions_gathered");
-  h->positions_touched = true;  // all-gather without the hand-shake: no swarm-wide displacement bound for this pass
-  double* buf = h->ds.gpos;
-  if (h->equal_shards) {
-    NC(g_nccl.AllGather(buf + 3 * h->ds.shard_begin, buf, size_t(3 * h->ds.n), ncclDouble, h->comm, h->stream));
-  } else {
-    NC(g_nccl.GroupStart());
-    for (int r = 0; r < h->n_ranks; r++) {
-      double* p = buf + 3 * h->shard_begin_of[r];
-      NC(g_nccl.Broadcast(p, p, size_t(3 * h->shard_count_of[r]), ncclDouble, r, h->comm, h->stream));
-    }
-    NC(g_nccl.GroupEnd());
-  }
-  return MRSB_OK;
-}
-
 // What the launches of the collision pass that comes next take (with_step: of a tick, its stepping launch first).  With the pull
-// exchange, h->ds already points at the buffers of that pass' parity (after_pass).
+// exchange, h->ds already points at the buffers of that pass' parity (end_pass).
 static void graph_args(const mrsb_sim* h, bool with_step, double dt, int k_substeps, GraphArgs* a) {
   std::memset(static_cast<void*>(a), 0, sizeof(*a));  // padding included
   std::memcpy(&a->s, &h->ds, sizeof(DevState));
@@ -1480,46 +1558,10 @@ static Graph build_pass_graph(mrsb_sim* h, const GraphArgs& a) {
   return g;
 }
 
-// host bookkeeping before a pass that goes through decide_kernel
-static int before_list_pass(mrsb_sim* h) {
-  // anything but exactly one stepping launch since the last pass: the displacement bound does not cover it
-  if (h->positions_touched || h->steps_since_pass != 1)
-    CU(cudaMemcpyAsync(&h->grid.ctl->force, h->h_one.get(), sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
-  h->positions_touched = false;
-  h->steps_since_pass  = 0;
-  h->list_passes++;
-  return MRSB_OK;
-}
-
-// host bookkeeping after any pass: with the pull exchange the write buffer changes sides
-static int after_pass(mrsb_sim* h) {
-  h->n_passes++;
-  if (h->p2p) {
-    h->pass_no++;
-    const int w         = write_buf(h);
-    h->ds.gpos          = h->gbuf[w];
-    h->ds.gbox          = h->d_gbox[w];
-    h->ds.geom          = h->d_geom[w];
-    h->wrote_since_pass = false;
-    int rc              = apply_pending_geom(h, w);  // no peer reads this buffer any more (they have all started the pass that just ran)
-    if (rc) return rc;
-  }
-  CU(cudaGetLastError());
-  return MRSB_OK;
-}
-
-static int collide_local(mrsb_sim* h) {
-  if (h->p2p && !h->wrote_since_pass) {
-    // nothing wrote positions since the last pass: the buffer this pass reads still holds the ones of two passes ago
-    h->n_launches += launch_publish_positions(h->ds, h->stream);
-    h->wrote_since_pass = true;
-  }
-  if (h->lists_on) {
-    int rc = before_list_pass(h);
-    if (rc) return rc;
-  } else {
-    h->steps_since_pass = 0;
-  }
+// One collision pass.  gathered: the caller put every shard's positions in place (mrsb_gather_buffer).
+static int collision_pass(mrsb_sim* h, bool gathered) {
+  int rc = begin_pass(h, gathered);
+  if (rc) return rc;
   GraphArgs a;
   graph_args(h, false, 0.0, 0, &a);
   Graph& g       = h->pass[write_buf(h)];
@@ -1540,7 +1582,7 @@ static int collide_local(mrsb_sim* h) {
   } else {
     h->n_launches += launch_collide(a.s, a.grid, a.pv, a.p2p, a.crash, a.rebounce, h->stream);
   }
-  return after_pass(h);
+  return end_pass(h);
 }
 
 static int before_step(mrsb_sim* h, double dt, int32_t k_substeps) {
@@ -1553,47 +1595,31 @@ static int before_step(mrsb_sim* h, double dt, int32_t k_substeps) {
   return MRSB_OK;
 }
 
-int mrsb_make_step(mrsb_handle h, double dt, int32_t k_substeps) {
-  GUARD(h);
-  int rc = before_step(h, dt, k_substeps);
-  if (rc) return rc;
+static int make_step(mrsb_sim* h, double dt, int32_t k_substeps) {
   GraphArgs a;
   graph_args(h, true, dt, k_substeps, &a);
   h->n_launches += launch_step_buckets(a, h->stream, h->step_info);
-  h->wrote_since_pass = true;
-  h->n_steps += k_substeps;
-  h->steps_since_pass++;
+  stepped(h, k_substeps);
   CU(cudaGetLastError());
   return MRSB_OK;
 }
 
-static int before_collisions(mrsb_sim* h) {
-  int rc = flush_params(h);
-  if (rc) return rc;
-  if (h->ds.n_global > h->ds.n && h->n_ranks <= 1) return fail(MRSB_ERR_STATE, "sharded handle without communicator");
-  if (h->lists_on && (h->positions_touched || h->steps_since_pass != 1))
-    // anything but exactly one stepping launch since the last pass: this rank's displacement is unbounded —
-    // said through the displacement word, so that every peer rebuilds as well
-    CU(cudaMemcpyAsync(&h->grid.ctl->disp_max_bits, h->h_one.get() + 1, sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
-  return MRSB_OK;
+int mrsb_make_step(mrsb_handle h, double dt, int32_t k_substeps) {
+  GUARD(h);
+  int rc = before_step(h, dt, k_substeps);
+  return rc ? rc : make_step(h, dt, k_substeps);
 }
 
 int mrsb_handle_collisions(mrsb_handle h) {
   GUARD(h);
   if (!(h->coll_crash || h->coll_enabled)) return MRSB_OK;  // SIM:299-301
-  int rc = before_collisions(h);
-  if (rc) return rc;
-  rc = exchange_positions(h);
-  if (rc) return rc;
-  return collide_local(h);
+  return collision_pass(h, false);
 }
 
 int mrsb_handle_collisions_gathered(mrsb_handle h) {
   GUARD(h);
   if (!(h->coll_crash || h->coll_enabled)) return MRSB_OK;
-  int rc = flush_params(h);
-  if (rc) return rc;
-  return collide_local(h);
+  return collision_pass(h, true);
 }
 
 // One tick = stepping launch + collision pass.  With neighbour lists the two are ONE graph (per buffer parity): a single
@@ -1602,7 +1628,8 @@ int mrsb_handle_collisions_gathered(mrsb_handle h) {
 static int run_tick_graph(mrsb_sim* h, double dt, int32_t k_substeps, bool* done) {
   *done = false;
   if (!h->lists_on || h->graph_failed || getenv("MRSB_NO_GRAPH")) return MRSB_OK;
-  if (h->positions_touched || h->steps_since_pass != 0) return MRSB_OK;  // let the ordinary path sort that out first
+  // the graph's pass assumes its own stepping launch and nothing else since the last pass: otherwise the ordinary path goes first
+  if (h->since.unbounded || h->since.steps != 0) return MRSB_OK;
   GraphArgs a;
   graph_args(h, true, dt, k_substeps, &a);
   Graph& g = h->tick[write_buf(h)];
@@ -1617,34 +1644,26 @@ static int run_tick_graph(mrsb_sim* h, double dt, int32_t k_substeps, bool* done
       return MRSB_OK;
     }
   }
-  // bookkeeping of make_step + before_collisions + collide_local for "exactly one stepping launch, then the pass"
-  h->wrote_since_pass = true;
-  h->n_steps += k_substeps;
-  h->list_passes++;
+  stepped(h, k_substeps);
+  int rc = begin_pass(h, false);
+  if (rc) return rc;
   CU(cudaGraphLaunch(g.exec, h->stream));
   h->n_launches += g.own;
   *done = true;
-  return after_pass(h);
+  return end_pass(h);
 }
 
 int mrsb_run(mrsb_handle h, double dt, int32_t k_substeps, int32_t n_ticks, int32_t with_collisions) {
   GUARD(h);
   const bool collide = with_collisions && (h->coll_crash || h->coll_enabled);
   for (int t = 0; t < n_ticks; t++) {
-    if (collide) {
-      int rc = before_step(h, dt, k_substeps);
-      if (rc) return rc;
-      bool done = false;
-      rc        = run_tick_graph(h, dt, k_substeps, &done);
-      if (rc) return rc;
-      if (done) continue;
-    }
-    int rc = mrsb_make_step(h, dt, k_substeps);
+    int rc = before_step(h, dt, k_substeps);
     if (rc) return rc;
-    if (collide) {
-      rc = mrsb_handle_collisions(h);
-      if (rc) return rc;
-    }
+    bool done = false;
+    if (collide) rc = run_tick_graph(h, dt, k_substeps, &done);
+    if (!rc && !done) rc = make_step(h, dt, k_substeps);
+    if (!rc && !done && collide) rc = collision_pass(h, false);
+    if (rc) return rc;
   }
   return MRSB_OK;
 }
@@ -1691,11 +1710,7 @@ int mrsb_set_state(mrsb_handle h, int64_t n, const int32_t* idx, const double* x
   if (R && !rc) rc = put_rows(h, h->ds.st, ST_ROWS, 6, 9, n, idx, R, 9, 0);
   if (omega && !rc) rc = put_rows(h, h->ds.st, ST_ROWS, 15, 3, n, idx, omega, 3, 0);
   if (motor_rpm && !rc) rc = put_rows(h, h->ds.rpm, MRSB_NM, 0, MRSB_NM, n, idx, motor_rpm, MRSB_NM, 0);
-  if (x && !rc) {
-    h->n_launches += launch_publish_positions(h->ds, h->stream);
-    h->wrote_since_pass  = true;
-    h->positions_touched = true;
-  }
+  if (x && !rc) rc = positions_written(h, false, false);
   return rc;
 }
 
@@ -1706,37 +1721,7 @@ int mrsb_set_state_pos(mrsb_handle h, int64_t n, const int32_t* idx, const doubl
   int            rc    = upload(h, n, idx, {{xyz, 3}, {heading, 1}}, &d_idx, d);
   if (rc || n == 0) return rc;
   h->n_launches += launch_set_state_pos(h->ds, n, d_idx, d[0], d[1], h->stream);
-  if (h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);  // the whole slice of the buffer being written, and its group boxes
-  h->wrote_since_pass  = true;
-  h->positions_touched = true;
-  CU(cudaGetLastError());
-  return MRSB_OK;
-}
-
-// The next pass that goes through decide_kernel replaces every force it visits (SIM:356-358), not only the ones it knows to be
-// non-zero.  No host synchronisation: the copy reads the pinned word when it runs.  If a later call has raised the word by then,
-// more passes than needed write every force they visit, which writes the values they would have left in place.
-static int write_all_forces_next_pass(mrsb_sim* h) {
-  if (!h->grid.ctl) return MRSB_OK;
-  *h->h_until.get() = (unsigned long long)h->list_passes + 1ull;  // index of the next pass that goes through decide_kernel
-  CU(cudaMemcpyAsync(&h->grid.ctl->write_all_until, h->h_until.get(), sizeof(unsigned long long), cudaMemcpyHostToDevice, h->stream));
-  return MRSB_OK;
-}
-
-// forces were written by something else than the collision pass: the next pass must replace every UAV's force
-static int forces_written(mrsb_sim* h) {
-  int rc = write_all_forces_next_pass(h);
-  if (rc) return rc;
-  h->positions_touched = true;  // that pass rebuilds: UAVs without candidates are only visited by a rebuild
-  return MRSB_OK;
-}
-
-// after a respawn: the buffer peers read has to show the new positions, and their per-group boxes (pull exchange)
-static int respawned(mrsb_sim* h) {
-  if (h->p2p) h->n_launches += launch_publish_positions(h->ds, h->stream);
-  h->wrote_since_pass = true;
-  CU(cudaGetLastError());
-  return MRSB_OK;
+  return positions_written(h, true, false);
 }
 
 int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz, const double* heading) {
@@ -1748,9 +1733,8 @@ int mrsb_respawn(mrsb_handle h, int64_t n, const int32_t* idx, const double* xyz
   rc = flush_params(h);  // the kernel reads the take-off flag of every UAV's parameter set
   if (rc) return rc;
   h->n_launches += launch_respawn(h->ds, h->d_takeoff0.get(), n, d_idx, d[0], d[1], h->stream);
-  h->positions_touched = true;
   note_mode(h, MRSB_INPUT_UNKNOWN, n, idx == nullptr);
-  return respawned(h);
+  return positions_written(h, true, false);
 }
 
 int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const double* xyz_dev, const double* heading_dev) {
@@ -1762,7 +1746,7 @@ int mrsb_respawn_masked_device(mrsb_handle h, const uint8_t* mask_dev, const dou
   // the batch can no longer be assumed to share one input mode unless it is already INPUT_UNKNOWN
   h->n_launches += launch_respawn_masked(h->ds, h->d_takeoff0.get(), mask_dev, xyz_dev, heading_dev, h->stream);
   note_mode(h, MRSB_INPUT_UNKNOWN, 1, false);
-  return respawned(h);
+  return positions_written(h, true, true);
 }
 
 // ---- snapshots ------------------------------------------------------------------------------
@@ -1834,11 +1818,10 @@ int mrsb_snapshot_save(mrsb_handle h, int32_t id) {
   return MRSB_OK;
 }
 
-// host bookkeeping after a restore.  all_own: every UAV took its own record.
-static int restored(mrsb_sim* h, const mrsb_sim::Snapshot& s, bool all_own) {
+// the host's input hints after a restore.  all_own: every UAV took its own record.
+static void restored(mrsb_sim* h, const mrsb_sim::Snapshot& s, bool all_own) {
   h->any_moment   = h->any_moment || s.any_moment;
   h->uniform_mode = (all_own || h->uniform_mode == s.uniform_mode) ? s.uniform_mode : -1;
-  return respawned(h);
 }
 
 int mrsb_snapshot_restore(mrsb_handle h, int32_t id, int64_t n, const int32_t* idx, const int32_t* src) {
@@ -1863,8 +1846,8 @@ int mrsb_snapshot_restore(mrsb_handle h, int32_t id, int64_t n, const int32_t* i
   if (rc) return rc;
   const SnapshotParts p = parts_of(h, *s);
   h->n_launches += launch_snapshot_restore(h->ds, p.rows, p.flags, p.mode, n, d_idx, d_src, h->stream);
-  h->positions_touched = true;
-  return restored(h, *s, !idx && !src && n == h->ds.n);
+  restored(h, *s, !idx && !src && n == h->ds.n);
+  return positions_written(h, true, false);
 }
 
 int mrsb_snapshot_restore_device(mrsb_handle h, int32_t id, const int32_t* src_dev) {
@@ -1879,7 +1862,8 @@ int mrsb_snapshot_restore_device(mrsb_handle h, int32_t id, const int32_t* src_d
   if (rc) return rc;
   const SnapshotParts p = parts_of(h, *s);
   h->n_launches += launch_snapshot_restore_masked(h->ds, p.rows, p.flags, p.mode, src_dev, h->stream);
-  return restored(h, *s, src_dev == nullptr);
+  restored(h, *s, src_dev == nullptr);
+  return positions_written(h, true, true);
 }
 
 int mrsb_snapshot_image_size(mrsb_handle h, size_t* bytes) {
@@ -2233,12 +2217,7 @@ static int refresh_opts(mrsb_sim* h) {
   if (opts == h->ds.opts) return MRSB_OK;
   const bool pos_back = (opts & STEP_OPT_GPOS) && !(h->ds.opts & STEP_OPT_GPOS);
   h->ds.opts          = opts;
-  if (pos_back) {  // the packed positions were not kept up to date meanwhile
-    h->n_launches += launch_publish_positions(h->ds, h->stream);
-    h->wrote_since_pass  = true;
-    h->positions_touched = true;
-    CU(cudaGetLastError());
-  }
+  if (pos_back) return positions_written(h, false, false);  // the packed positions were not kept up to date meanwhile
   return MRSB_OK;
 }
 
@@ -2444,11 +2423,7 @@ int mrsb_gather_buffer(mrsb_handle h, void** device_ptr, size_t* bytes) {
 
 int mrsb_publish_positions(mrsb_handle h) {
   GUARD(h);
-  h->wrote_since_pass  = true;
-  h->positions_touched = true;
-  h->n_launches += launch_publish_positions(h->ds, h->stream);
-  CU(cudaGetLastError());
-  return MRSB_OK;
+  return positions_written(h, false, false);
 }
 
 int mrsb_get_device_view(mrsb_handle h, mrsb_device_view* out) {

@@ -46,7 +46,7 @@
 // condition `decide_kernel` sets on the device, so no host round trip is involved.  Results are the
 // same bits either way: the lists only choose which pairs are tested.  Anything that moves UAVs
 // other than one stepping launch (set_state, publish_positions, several launches between passes)
-// forces a rebuild.  A UAV with more than NL_CAP candidates keeps no list: it remembers where its
+// forces a rebuild: the host raises the displacement word to "unbounded" before that pass.  A UAV with more than NL_CAP candidates keeps no list: it remembers where its
 // record sits in the (now ageing) table and, every pass, walks the stencil of its build-time cell —
 // the records there are a superset of its possible neighbours for as long as the lists are valid —
 // testing each candidate's CURRENT position (`check_crowded`).  Only the crowded UAVs pay for that.  Sharded handles use the lists when the peer
@@ -941,7 +941,7 @@ __global__ void __launch_bounds__(32) decide_kernel(NlCtl* __restrict__ c, unsig
   // every load first (they are independent: one round trip), then the decision, then the stores
   uint32_t                 bits  = c->disp_max_bits;  // largest squared displacement of the stepping launch since the last pass (float, rounded up)
   const double             D_old = c->D_total;
-  const uint32_t           force = c->force, valid = c->valid;
+  const uint32_t           valid = c->valid;
   const unsigned long long n_rebuilds = c->n_rebuilds, n_passes = c->n_passes;
   if (p.n_ranks > 1) {
     const unsigned long long epoch = c->epoch + 1ull;
@@ -973,15 +973,14 @@ __global__ void __launch_bounds__(32) decide_kernel(NlCtl* __restrict__ c, unsig
   }
   if (lane != 0) return;
   if (row) row[2] = now_ns();
-  const double d       = __dsqrt_ru(double(__uint_as_float(bits)));  // NaN stays NaN
+  const double d       = __dsqrt_ru(double(__uint_as_float(bits)));  // NaN stays NaN: an unbounded word rebuilds
   double       D       = __dadd_ru(D_old, d);
-  const bool   rebuild = always || force || !valid || !(__dmul_ru(2.0, D) <= skin);
+  const bool   rebuild = always || !valid || !(__dmul_ru(2.0, D) <= skin);
   if (has_handle) cudaGraphSetConditional(handle, rebuild ? 1u : 0u);
   *pair_counter    = 0ull;  // pairs found by this pass
   c->disp_max_bits = 0u;
   if (rebuild) {
     D            = 0.0;
-    c->force     = 0u;
     c->valid     = 1u;
     c->n_crowded = 0u;  // build_lists_kernel counts them again
     c->n_active  = 0u;  // ... and compact_kernel the UAVs with work

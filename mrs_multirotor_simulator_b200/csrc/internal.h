@@ -142,8 +142,8 @@ struct P2PCtl {
 #define MRSB_NL_CAP 8
 #define MRSB_TL_TICKS 4096
 struct NlCtl {
-  uint32_t disp_max_bits;  // written by the stepping kernel (DevState::disp_max points here)
-  uint32_t force;          // host: positions changed behind the stepping kernel's back -> rebuild
+  uint32_t disp_max_bits;  // written by the stepping kernel (DevState::disp_max points here); 0xFFFFFFFF (a NaN: "unbounded")
+                           // makes the pass rebuild: the host raises it before a pass whose bound does not hold (api.cu, begin_pass)
   uint32_t valid;          // lists exist
   uint32_t n_active;       // entries of DevGrid::nl_active (UAVs with something to check on list-only passes)
   uint32_t n_crowded;      // UAVs with more than MRSB_NL_CAP candidates at the last rebuild (they walk the table instead)

@@ -3,7 +3,7 @@
 Every stepping launch publishes the float bits of the largest squared displacement |x_end - x_start|^2 of any UAV it stepped,
 rounded up, through atomicMax.  The first kernel of every collision pass turns that word into d = sqrt_ru(float(bits)), adds it
 into D = add_ru(D, d) and keeps the lists while mul_ru(2, D) <= skin; a rebuild resets D to 0.  The host forces a rebuild
-(api.cu, before_collisions / before_list_pass) before the first pass and after anything but exactly one stepping launch.
+(api.cu, begin_pass) before the first pass and after anything but exactly one stepping launch.
 
 The directed roundings are computed exactly with fractions.Fraction (CPython's float(Fraction) rounds correctly), so this is
 the decision bit for bit, not an approximation of it."""
@@ -152,7 +152,7 @@ class ListBound:
 class HostSide:
     """api.cu's bookkeeping around the word: a pass after anything but exactly one stepping launch since the last pass (or after
     positions were written otherwise: set_state(x=...), respawn, the first pass) is forced — the host writes UNBOUNDED into the
-    word and raises the force flag."""
+    word, which decodes to NaN and fails the bound."""
 
     def __init__(self, skin):
         self.bound = ListBound(skin)

@@ -5,7 +5,8 @@ and the pass' rebuild flag must EQUAL the prediction: a bound looser than the ke
 tighter one (padding slots or frozen UAVs adding displacement: rebuilds too often) both fail.  This is checked on the staged
 kernel at a size larger than L2 with both sweep directions and fused K = 10 launches, on the direct and the per-UAV-mode
 kernels, on bucketed and unbucketed mixed batches, with UAVs frozen by iterate_without_input, through mrsb_run's tick graph,
-across forced rebuilds and NaN UAVs, and at cell edges 3.5, 6 and 12 m.
+across forced rebuilds and NaN UAVs, and at cell edges 3.5, 6 and 12 m.  The pass after every call that writes positions or
+forces otherwise, and the passes of handle_collisions_gathered, are pinned the same way.
 
 Then pairs of large UAVs (contact distance above sqrt(3), so nanoflann's ball binds) fly head-on from spawn separations that
 straddle the list radius, everybody else hovering, so that the pairs set the swarm's displacement bound and close at nearly
@@ -90,11 +91,12 @@ class Watch:
             self.host.touch()
         self.x = xof(self.b)
 
-    def collide(self):
+    def collide(self, do_pass=None):
+        """One pass, through handle_collisions or `do_pass`."""
         self.forced.append(self.host.touched or self.host.launches != 1)
         self.words.append(self.host.bits)
         want = self.host.collide()
-        self.b.handle_collisions()
+        (do_pass or self.b.handle_collisions)()
         r = self.b.collision_info()["rebuilds"]
         got, self.rebuilds = r - self.rebuilds, r
         self.flags.append(bool(got))
@@ -105,6 +107,15 @@ class Watch:
     def tick(self, dt=0.01, k=1):
         self.step(dt, k)
         return self.collide()
+
+    def run_tick(self, dt=0.01):
+        """One tick through mrsb_run: its stepping launch and its pass, one graph once the tick graph is captured.  The word is
+        learnt from the positions after the tick (a pass moves nobody), so the pass is checked after it ran."""
+        self.b.run(dt, 1)
+        x = xof(self.b)
+        self.host.launch(R.disp_bits(self.x, x))
+        self.x = x
+        return self.collide(lambda: None)
 
     def assert_both_ways(self, min_kept=1, min_rebuilt=1):
         """Unforced passes must have gone both ways: lists kept, and rebuilt because the bound ran out."""
@@ -307,6 +318,151 @@ def test_forced_rebuilds_nan_and_cell_sizes(cell):
     w.assert_both_ways(5, 1)
     if cell == 12.0:
         assert b.collision_info()["crowded_uavs"] > 100
+
+
+# ---- every position writer, and the pass after it ------------------------------------------------------------------------------
+
+# calls between two passes after which the displacement word no longer bounds the positions (the next pass rebuilds) ...
+FORCING = ("set_state_x", "set_state_pos", "respawn", "snapshot_restore", "publish_positions", "positions_back_on", "apply_force",
+           "forces_written", "respawn_masked_one")
+# ... and calls that leave the bound intact
+BOUNDED = ("set_state_v", "set_external_moment", "respawn_masked_zero", "snapshot_restore_device_nobody")
+
+
+def write(b, writer, snap, step):
+    """`writer` on handle b; `step`: a stepping launch of b.  Everything is derived from b's state, so twins get the same call."""
+    import torch
+
+    n = b.n
+    idx = np.array([3, 40, n - 2], dtype=np.int32)
+    x = xof(b)
+    if writer == "set_state_x":
+        b.set_state(idx=idx, x=x[idx] + 0.05)
+    elif writer == "set_state_v":
+        b.set_state(idx=idx, v=np.tile([0.5, -0.5, 0.2], (len(idx), 1)))
+    elif writer == "set_state_pos":
+        b.set_state_pos(x[idx] - 0.05, np.full(len(idx), 0.3), idx=idx)
+    elif writer == "respawn":
+        b.respawn(x[idx] + [0.1, 0.0, 0.0], 0.2, idx=idx)
+    elif writer == "snapshot_restore":
+        snap.restore(idx=idx)
+    elif writer == "publish_positions":
+        b.publish_positions()
+    elif writer == "positions_back_on":
+        # the packed positions are not kept while nothing needs them; switching collisions back on republishes them
+        b.set_collisions(False, False, 100.0)
+        b.set_outputs(positions=False)
+        step()
+        step()
+        b.set_collisions(True, False, 100.0)
+    elif writer == "apply_force":
+        b.apply_force(np.tile([3.0, 0.0, -1.0], (len(idx), 1)), idx=idx)
+    elif writer == "forces_written":
+        b.forces_written()
+    elif writer == "set_external_moment":
+        b.set_external_moment(np.tile([0.0, 0.0, 0.01], (len(idx), 1)), idx=idx)
+    elif writer.startswith("respawn_masked"):
+        mask = torch.zeros(n, dtype=torch.bool, device="cuda:0")
+        if writer == "respawn_masked_one":
+            mask[17] = True
+        xyz = torch.as_tensor(x + [0.0, 0.1, 0.0], dtype=torch.float64, device="cuda:0")
+        heading = torch.zeros(n, dtype=torch.float64, device="cuda:0")
+        torch.cuda.synchronize()
+        b.respawn_masked_device(mask.data_ptr(), xyz.data_ptr(), heading.data_ptr())
+        b.sync()  # before the tensors go
+    elif writer == "snapshot_restore_device_nobody":
+        src = torch.full((n,), -1, dtype=torch.int32, device="cuda:0")
+        torch.cuda.synchronize()
+        snap.restore_device(src.data_ptr())
+        b.sync()
+    else:
+        raise AssertionError(writer)
+
+
+@pytest.mark.parametrize("via", ["handle_collisions", "run"])
+@pytest.mark.parametrize("writer", FORCING + BOUNDED)
+def test_every_position_writer_and_the_next_pass(writer, via):
+    """Every call that writes positions (or forces) other than a stepping launch, between two ticks of a swarm in contact: the
+    pass after it rebuilds exactly as the reference predicts — always after a FORCING call, never after a BOUNDED one — and it,
+    and the passes after it, find the pairs and forces of the full pass (MRSB_NO_NEIGHBOUR_LISTS=1).  Ticks go through
+    handle_collisions, or through mrsb_run (whose tick graph is captured by then)."""
+    n = 128 * 4 + 9
+    spawn = grid(n, 0.85)  # neighbours in contact (x500: below sqrt(0.8) m)
+    cmd = velocity_cmd(n, 31, 1.0)
+    a = make([af("x500")], spawn)
+    f = make([af("x500")], spawn, MRSB_NO_NEIGHBOUR_LISTS=1)
+    snaps = []
+    for b in (a, f):
+        b.set_collisions(True, False, 100.0)
+        b.set_pair_capacity(40 * n)
+        b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd)
+        snaps.append(b.snapshot())
+        snaps[-1].save()
+    w = Watch(a)
+
+    def tick():
+        if via == "run":
+            w.run_tick()
+            f.run(0.01, 1)
+        else:
+            w.tick()
+            f.make_step(0.01)
+            f.handle_collisions()
+        p = a.get_collision_pairs()
+        assert len(p) and np.array_equal(p, f.get_collision_pairs()), f"pass {len(w.flags) - 1}: pairs"
+        assert np.array_equal(a.get_force(), f.get_force()), f"pass {len(w.flags) - 1}: forces"
+
+    for _ in range(4):
+        tick()
+    write(a, writer, snaps[0], w.step)
+    write(f, writer, snaps[1], lambda: f.make_step(0.01))
+    if writer in FORCING:
+        w.host.touch()
+    w.x = xof(a)
+    tick()
+    assert w.flags[-1] == w.forced[-1] == (writer in FORCING), (w.flags, w.forced)
+    for _ in range(2):
+        tick()
+    assert w.flags[-2:] == [False, False]
+    assert np.array_equal(w.x, xof(f))
+    a.close()
+    f.close()
+
+
+def test_gathered_pass_decides_like_handle_collisions():
+    """mrsb_handle_collisions_gathered on a single-shard handle with neighbour lists (the packed positions are complete without a
+    gather): every pass rebuilds as a twin's through handle_collisions and as the reference predicts, forced passes included (a
+    pass without a step, two launches, set_state(x=...), apply_force), with the same pairs and forces."""
+    n = 128 * 8 + 9
+    spawn = grid(n, 0.85)
+    cmd = velocity_cmd(n, 33, 1.0)
+    g = make([af("x500")], spawn, MRSB_COLLISION_CELL=4.0)  # skin 0.27 m: the bound runs out within the run
+    t = make([af("x500")], spawn, MRSB_COLLISION_CELL=4.0)
+    for b in (g, t):
+        b.set_collisions(True, False, 100.0)
+        b.set_pair_capacity(40 * n)
+        b.set_input(O.VELOCITY_HDG_RATE_CMD, cmd)
+    wg, wt = Watch(g), Watch(t)
+    found = 0
+    for p in range(60):
+        for w, do_pass in ((wg, g.handle_collisions_gathered), (wt, None)):
+            if p == 12:
+                w.step()  # two launches before this pass
+            if p == 20:
+                w.set_state([5], x=w.x[[5]] + 0.05)
+            if p == 28:
+                w.b.apply_force(np.array([[2.0, 0.0, 0.0]]), idx=np.array([9], dtype=np.int32))
+                w.host.touch()
+            if p != 16:  # a pass without a step
+                w.step()
+            w.collide(do_pass)
+        pairs = g.get_collision_pairs()
+        assert np.array_equal(pairs, t.get_collision_pairs()), f"pass {p}: pairs"
+        found += len(pairs)
+        assert np.array_equal(g.get_force(), t.get_force()), f"pass {p}: forces"
+    assert wg.flags == wt.flags and wg.forced == wt.forced
+    assert found and [p for p in range(60) if wg.forced[p]] == [0, 12, 16, 20, 28], (found, wg.forced)
+    wg.assert_both_ways(5, 1)
 
 
 def skin_of_cell(cell):
